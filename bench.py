@@ -3,6 +3,7 @@
 particle-microsteps/sec with contact resolution).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload arm_table] [--particles P] [--impl reference]
+                    [--dump-outputs DIR]
 
 A "step" is ONE ForwardSimulateRobots call (simple_particle_contact_simulator.hpp:788) over one batch of
 synthetic particles: 25 controller steps x their microsteps x contact resolution per particle.  Default
@@ -15,10 +16,14 @@ e2e     = the same metric with HOST buffers (pinned) through the C ABI: H2D of s
           result records inside the timed region; at N > 1 the records of ALL ranks are gathered (ncclAllGather) and
           read back on every rank inside it.
 config5 = BASELINE config 5 in the same line: 1,048,576 arm particles IN TOTAL split over the N GPUs (strong scaling),
-          all-gather of the end states included, device-timed.
+          all-gather of the end states included, device-timed.  A fixed-size leg: one warm-up call and two timed calls
+          whatever --steps and --warmup say (--config5-particles 0 skips it).
+--steps K sets the number of timed steps of value and of e2e; --warmup W the untimed steps before them.
 roofline= the simulate kernel against the unit ncu shows binding for the workload.
 --impl reference times the CPU restatement of the reference (oracle/, all host threads) on a bounded sample; that arm
 never loads libfksgpu.so.
+--dump-outputs DIR writes the end-state records of the last device-timed step (all ranks' records at N > 1) to
+DIR/<field>.npy as float64, so that two builds can be compared output for output on the same seeded inputs.
 """
 import argparse
 import json
@@ -50,7 +55,14 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--config5-particles", type=int, default=1048576, help="total particles of the strong-scaling leg (0 = skip it)")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="CPU work budget of the cpu_baseline sample")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the end-state records of the last timed step to DIR/<field>.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm (the reference arm sizes its sample by timing)")
+    return args
 
 
 def host_threads():
@@ -118,6 +130,25 @@ def algorithmic_work(stats, P, D, J):
     flops = (fk + 39 * P) * M + (3 * fk + P * (36 + 12 * D + 21 + 30) + 36 * P + 39 * P) * I + (40 + 6 * D * D) * K
     gathers = P * M + 8 * P * I
     return nbytes, flops, gathers
+
+
+DUMP_LIMIT_BYTES = 64_000_000  # all files of one dump together, .npy headers included
+NPY_HEADER_BYTES = 1024  # bound on one .npy header (numpy pads it to a multiple of 64 bytes: 128 for these arrays)
+
+
+def dump_outputs(path, records):
+    """One float64 .npy per field of the end-state records, plus particle_id.npy.  A batch whose dump would exceed
+    DUMP_LIMIT_BYTES is represented by a fixed, seeded sample of its particles (the ids are in particle_id.npy)."""
+    os.makedirs(path, exist_ok=True)
+    n = len(records)
+    per_particle = 8 * (1 + sum(int(np.prod(records.dtype[f].shape)) for f in records.dtype.names))
+    budget = DUMP_LIMIT_BYTES - (1 + len(records.dtype.names)) * NPY_HEADER_BYTES
+    ids = np.arange(n)
+    if n * per_particle > budget:
+        ids = np.sort(np.random.default_rng(0).choice(n, budget // per_particle, replace=False))
+    np.save(os.path.join(path, "particle_id.npy"), ids.astype(np.float64))
+    for f in records.dtype.names:
+        np.save(os.path.join(path, f + ".npy"), records[f][ids].astype(np.float64))
 
 
 def oracle_simulator(w, threads):
@@ -250,6 +281,8 @@ def main():
         ev[i][1].record(stream)
         kernel_ms.append(sim.kernel_times_ms())  # waits for this step's kernels; the events above are on the stream
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, (d_gather if world > 1 else d_results).cpu().numpy().view(sim.dtype))
     step_ms = sum(a.elapsed_time(b) for a, b in ev)
     stats = sim.get_statistics()
     launches = sim.launch_count - launches0

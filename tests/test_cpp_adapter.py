@@ -16,32 +16,32 @@ PROGRAMS = {
 }
 
 
-def build(name):
-    exe = "/tmp/fksgpu_example_" + name
+def build(name, directory):
+    exe = str(directory / ("fksgpu_example_" + name))
     subprocess.check_call(["/usr/bin/g++", "-std=c++11", "-Wall", "-Werror", "-I" + os.path.join(ROOT, "include"), PROGRAMS[name],
                            "-L" + LIB, "-lfksgpu", "-Wl,-rpath," + LIB, "-o", exe])
     return exe
 
 
 @pytest.mark.parametrize("name", ["se2", "linked_se3"])
-def test_adapter_compiles_and_fails_loudly_without_a_gpu(name):
+def test_adapter_compiles_and_fails_loudly_without_a_gpu(name, tmp_path):
     import torch
 
-    r = subprocess.run([build(name)], capture_output=True, text=True)
+    r = subprocess.run([build(name, tmp_path)], capture_output=True, text=True)
     if torch.cuda.is_available():
         assert r.returncode == 0, r.stdout
     else:
         assert r.returncode == 3 and "no CUDA device" in r.stdout
 
 
-def test_glue_templates_against_mock_reference_types():
-    r = subprocess.run([build("glue_mock")], capture_output=True, text=True)
+def test_glue_templates_against_mock_reference_types(tmp_path):
+    r = subprocess.run([build("glue_mock", tmp_path)], capture_output=True, text=True)
     assert r.returncode == 0 and "ok" in r.stdout, r.stdout + r.stderr
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", ["se2", "linked_se3"])
-def test_adapter_on_gpu(name):
-    r = subprocess.run([build(name)], capture_output=True, text=True)
+def test_adapter_on_gpu(name, tmp_path):
+    r = subprocess.run([build(name, tmp_path)], capture_output=True, text=True)
     print(r.stdout)
     assert r.returncode == 0 and "ok" in r.stdout and "FAILED" not in r.stdout, r.stdout + r.stderr
