@@ -46,12 +46,15 @@ EXPORTS = (
     "fks_forward_simulate_async",
     "fks_sim_synchronize",
     "fks_forward_simulate_device",
+    "fks_forward_simulate_sequence",
+    "fks_forward_simulate_sequence_device",
     "fks_multi_sim_create",
     "fks_multi_sim_destroy",
     "fks_multi_sim_device_count",
     "fks_multi_sim_result_stride",
     "fks_multi_forward_simulate",
     "fks_multi_forward_simulate_device",
+    "fks_multi_forward_simulate_sequence",
     "fks_multi_get_statistics",
     "fks_multi_reset_statistics",
     "fks_check_config_collision",
@@ -100,6 +103,14 @@ lib.fks_forward_simulate.argtypes = _sim_args
 lib.fks_reverse_simulate.argtypes = _sim_args
 lib.fks_forward_simulate_async.argtypes = _sim_args
 lib.fks_sim_synchronize.argtypes = [C.c_void_p]
+_seq_args = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_int, P(NoiseTape), C.c_uint64,
+             C.c_void_p]
+lib.fks_forward_simulate_sequence.argtypes = _seq_args
+lib.fks_multi_forward_simulate_sequence.argtypes = _seq_args
+lib.fks_forward_simulate_sequence_device.argtypes = [
+    C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
+    C.c_uint64, C.c_void_p, C.c_void_p,
+]
 lib.fks_multi_sim_create.argtypes = [P(C.c_int32), C.c_int32, P(EnvDesc), P(RobotDesc), P(SolverParams), C.c_double, C.c_uint64, C.c_int32,
                                      P(C.c_void_p)]
 lib.fks_multi_sim_destroy.argtypes = [C.c_void_p]

@@ -688,8 +688,9 @@ size_t fks_sim_result_stride(const fks_sim* sim) {
     return sim ? (size_t)sim->robot->stride * 8 + sizeof(fks_result_tail) : 0;
 }
 
-static int simulate_on_stream(fks_sim* s, const double* d_starts, const double* d_targets, size_t n, size_t n_targets,
-                              int allow_contacts, int noise_mode, const double* d_tape, const uint64_t* d_tape_off,
+// n_legs consecutive legs per particle (1: a single ForwardSimulateRobots call); d_targets and d_results are leg-major
+static int simulate_on_stream(fks_sim* s, const double* d_starts, const double* d_targets, size_t n, size_t n_targets, size_t n_legs,
+                              uint64_t leg_id_stride, int allow_contacts, int noise_mode, const double* d_tape, const uint64_t* d_tape_off,
                               const uint64_t* d_dec, const uint64_t* d_dec_off,
                               uint64_t first_particle_id, void* d_results, cudaStream_t stream) {
     if (n == 0) return FKS_OK;
@@ -715,6 +716,8 @@ static int simulate_on_stream(fks_sim* s, const double* d_starts, const double* 
     a.n_targets = n_targets;
     a.seed = s->seed;
     a.first_id = first_particle_id;
+    a.leg_id_stride = leg_id_stride;
+    a.n_legs = (int)n_legs;
     a.allow_contacts = allow_contacts ? 1 : 0;
     a.noise_mode = noise_mode;
     a.cfg_stride = s->robot->stride;
@@ -762,21 +765,34 @@ static int check_batch(const fks_sim* sim, const void* starts, const void* targe
     return FKS_OK;
 }
 
-int fks_forward_simulate_async(fks_sim* s, const double* starts, const double* targets, size_t n, size_t n_targets,
-                         int allow_contacts, int noise_mode, const fks_noise_tape* tape, uint64_t first_particle_id,
-                         void* results) {
-    int rc = check_batch(s, starts, targets, n, n_targets, noise_mode, tape ? tape->draws : nullptr, tape ? tape->offsets : nullptr, results);
-    if (rc != FKS_OK || n == 0) return rc;
+}  // extern "C"
+
+int fks_host::check_sequence(const char* fn, const void* targets, size_t n, size_t n_legs, uint64_t first_particle_id) {
+    if (n_legs == 0 || !targets) return fail(FKS_ERR_INVALID_ARGUMENT, std::string(fn) + ": need at least one leg and its targets");
+    // the kernel counts legs in 31 bits (the top bit of WarpVars::leg marks a pending leg)
+    if (n_legs > 0x7FFFFFFFull) return fail(FKS_ERR_INVALID_ARGUMENT, std::string(fn) + ": more than 2^31 - 1 legs");
+    if (n != 0 && (n_legs > UINT64_MAX / n || (uint64_t)(n_legs * n) > UINT64_MAX - first_particle_id))
+        return fail(FKS_ERR_INVALID_ARGUMENT, std::string(fn) + ": first_particle_id + n_legs * n_particles overflows 64 bits");
+    return FKS_OK;
+}
+
+// (fks_internal.h) the pitches let one device's shard of a multi-GPU call read and write its slices of the caller's arrays in place
+int fks_host::simulate_host_async(fks_sim* s, const double* starts, const double* targets, size_t targets_pitch, size_t n,
+                                  size_t n_targets, size_t n_legs, uint64_t leg_id_stride, int allow_contacts, int noise_mode,
+                                  const fks_noise_tape* tape, uint64_t first_particle_id, void* results, size_t results_pitch) {
+    if (n == 0) return FKS_OK;
+    int rc = FKS_OK;
     NvtxRange range("fks_forward_simulate");
     DeviceGuard guard(s->device);
     if (!guard.ok) return fail(FKS_ERR_CUDA, "fks_forward_simulate: cudaSetDevice failed");
     const size_t stride = (size_t)s->robot->stride;
     const size_t rec = fks_sim_result_stride(s);
+    const size_t leg_targets = n_targets * stride;  // doubles of one leg's targets on the device
     size_t n_draws = 0;
     if (noise_mode == FKS_NOISE_INJECTED) n_draws = (size_t)tape->offsets[n];
     if ((rc = ensure(&s->d_starts, &s->cap_starts, n * stride)) != FKS_OK) return rc;
-    if ((rc = ensure(&s->d_targets, &s->cap_targets, n_targets * stride)) != FKS_OK) return rc;
-    if ((rc = ensure(&s->d_results, &s->cap_results, n * rec)) != FKS_OK) return rc;
+    if ((rc = ensure(&s->d_targets, &s->cap_targets, n_legs * leg_targets)) != FKS_OK) return rc;
+    if ((rc = ensure(&s->d_results, &s->cap_results, n_legs * n * rec)) != FKS_OK) return rc;
     const bool with_decisions = noise_mode == FKS_NOISE_INJECTED && tape->decisions && tape->decision_offsets;
     size_t n_dec_words = 0;
     if (noise_mode == FKS_NOISE_INJECTED) {
@@ -791,7 +807,11 @@ int fks_forward_simulate_async(fks_sim* s, const double* starts, const double* t
     {
         NvtxRange h2d("fks: H2D starts / targets / tape");
         FKS_CUDA(cudaMemcpyAsync(s->d_starts, starts, n * stride * 8, cudaMemcpyHostToDevice, s->stream));
-        FKS_CUDA(cudaMemcpyAsync(s->d_targets, targets, n_targets * stride * 8, cudaMemcpyHostToDevice, s->stream));
+        if (n_legs == 1 || targets_pitch == leg_targets)
+            FKS_CUDA(cudaMemcpyAsync(s->d_targets, targets, n_legs * leg_targets * 8, cudaMemcpyHostToDevice, s->stream));
+        else
+            FKS_CUDA(cudaMemcpy2DAsync(s->d_targets, leg_targets * 8, targets, targets_pitch * 8, leg_targets * 8, n_legs,
+                                       cudaMemcpyHostToDevice, s->stream));
         if (noise_mode == FKS_NOISE_INJECTED) {
             if (n_draws) FKS_CUDA(cudaMemcpyAsync(s->d_tape, tape->draws, n_draws * 8, cudaMemcpyHostToDevice, s->stream));
             FKS_CUDA(cudaMemcpyAsync(s->d_tape_off, tape->offsets, (n + 1) * 8, cudaMemcpyHostToDevice, s->stream));
@@ -803,14 +823,41 @@ int fks_forward_simulate_async(fks_sim* s, const double* starts, const double* t
     }
     {
         NvtxRange launch("fks: simulate kernel");
-        rc = simulate_on_stream(s, s->d_starts, s->d_targets, n, n_targets, allow_contacts, noise_mode, s->d_tape,
+        rc = simulate_on_stream(s, s->d_starts, s->d_targets, n, n_targets, n_legs, leg_id_stride, allow_contacts, noise_mode, s->d_tape,
                                 (const uint64_t*)s->d_tape_off, with_decisions ? (const uint64_t*)s->d_dec : nullptr,
                                 with_decisions ? (const uint64_t*)s->d_dec_off : nullptr, first_particle_id, s->d_results, s->stream);
     }
     if (rc != FKS_OK) return rc;
     NvtxRange d2h("fks: D2H records");
-    FKS_CUDA(cudaMemcpyAsync(results, s->d_results, n * rec, cudaMemcpyDeviceToHost, s->stream));
+    if (n_legs == 1 || results_pitch == n * rec)
+        FKS_CUDA(cudaMemcpyAsync(results, s->d_results, n_legs * n * rec, cudaMemcpyDeviceToHost, s->stream));
+    else
+        FKS_CUDA(cudaMemcpy2DAsync(results, results_pitch, s->d_results, n * rec, n * rec, n_legs, cudaMemcpyDeviceToHost, s->stream));
     return FKS_OK;
+}
+
+extern "C" {
+
+int fks_forward_simulate_async(fks_sim* s, const double* starts, const double* targets, size_t n, size_t n_targets,
+                         int allow_contacts, int noise_mode, const fks_noise_tape* tape, uint64_t first_particle_id,
+                         void* results) {
+    const int rc = check_batch(s, starts, targets, n, n_targets, noise_mode, tape ? tape->draws : nullptr, tape ? tape->offsets : nullptr, results);
+    if (rc != FKS_OK || n == 0) return rc;
+    return fks_host::simulate_host_async(s, starts, targets, n_targets * (size_t)s->robot->stride, n, n_targets, 1, n, allow_contacts,
+                                         noise_mode, tape, first_particle_id, results, n * fks_sim_result_stride(s));
+}
+
+int fks_forward_simulate_sequence(fks_sim* s, const double* starts, const double* targets, size_t n, size_t n_targets, size_t n_legs,
+                                  int allow_contacts, int noise_mode, const fks_noise_tape* tape, uint64_t first_particle_id,
+                                  void* results) {
+    int rc = fks_host::check_sequence("fks_forward_simulate_sequence", targets, n, n_legs, first_particle_id);
+    if (rc == FKS_OK)
+        rc = check_batch(s, starts, targets, n, n_targets, noise_mode, tape ? tape->draws : nullptr, tape ? tape->offsets : nullptr, results);
+    if (rc != FKS_OK || n == 0) return rc;
+    rc = fks_host::simulate_host_async(s, starts, targets, n_targets * (size_t)s->robot->stride, n, n_targets, n_legs, n, allow_contacts,
+                                       noise_mode, tape, first_particle_id, results, n * fks_sim_result_stride(s));
+    if (rc != FKS_OK) return rc;
+    return fks_sim_synchronize(s);
 }
 
 int fks_sim_synchronize(fks_sim* s) {
@@ -885,7 +932,19 @@ int fks_forward_simulate_device(fks_sim* s, const double* d_starts, const double
     if (rc != FKS_OK || n == 0) return rc;
     DeviceGuard guard(s->device);
     if (!guard.ok) return fail(FKS_ERR_CUDA, "fks_forward_simulate_device: cudaSetDevice failed");
-    return simulate_on_stream(s, d_starts, d_targets, n, n_targets, allow_contacts, noise_mode, d_tape_draws, d_tape_offsets,
+    return simulate_on_stream(s, d_starts, d_targets, n, n_targets, 1, n, allow_contacts, noise_mode, d_tape_draws, d_tape_offsets,
+                              nullptr, nullptr, first_particle_id, d_results, (cudaStream_t)cuda_stream);
+}
+
+int fks_forward_simulate_sequence_device(fks_sim* s, const double* d_starts, const double* d_targets, size_t n, size_t n_targets,
+                                         size_t n_legs, int allow_contacts, int noise_mode, const double* d_tape_draws,
+                                         const uint64_t* d_tape_offsets, uint64_t first_particle_id, void* d_results, void* cuda_stream) {
+    int rc = fks_host::check_sequence("fks_forward_simulate_sequence_device", d_targets, n, n_legs, first_particle_id);
+    if (rc == FKS_OK) rc = check_batch(s, d_starts, d_targets, n, n_targets, noise_mode, d_tape_draws, d_tape_offsets, d_results);
+    if (rc != FKS_OK || n == 0) return rc;
+    DeviceGuard guard(s->device);
+    if (!guard.ok) return fail(FKS_ERR_CUDA, "fks_forward_simulate_sequence_device: cudaSetDevice failed");
+    return simulate_on_stream(s, d_starts, d_targets, n, n_targets, n_legs, n, allow_contacts, noise_mode, d_tape_draws, d_tape_offsets,
                               nullptr, nullptr, first_particle_id, d_results, (cudaStream_t)cuda_stream);
 }
 

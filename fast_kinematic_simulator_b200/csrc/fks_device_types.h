@@ -113,6 +113,9 @@ struct WarpVars {
     // the current / previous kinematic state, the last collision bits, and whether the next thing it needs is a contact solve
     int after, op, op_in, op_out, op_u, op_tn, op_derive, measure, cur, prev, want_solve;
     unsigned cc;
+    // leg of a sequence call the particle is in, top bit: the next leg is due (used by the sequence kernel only).  Here,
+    // behind the fields above: inserted among them it shifts their offsets, and the single-call kernel's spill code with them
+    unsigned leg;
     int ctx;        // index of this context in the CTA's pool (fixed: its slot of the global context store)
 };
 constexpr int kWarpVarsDoubles = (int)((sizeof(WarpVars) + 7) / 8);
@@ -144,7 +147,7 @@ struct WarpLayout {
     int tn;       // noise_batch * S: truncated-normal draws of the next noise_batch microsteps
     int qr;       // S doubles: the actuated twist of the SE(3) robot (apply_control)
     int cand;     // 32 doubles = 32 candidate records of collect_corrections
-    int vars;     // WarpVars (kWarpVarsDoubles) + 2 * S doubles of PID state
+    int vars;     // WarpVars (kWarpVarsDoubles) + 2 * S doubles of PID state (inside [target, save2_end): parked with the context)
     int flags;    // 1 (u32 FKS_FLAG_* bits raised by any lane)
     int save2_end;  // a particle's context = [cfg, T + 2 L12) + [G, G + L12) + [target, save2_end): what has to survive between phases
     int stats;    // FKS_NUM_STATS u64 counters of this WARP (not part of a context)
@@ -273,6 +276,10 @@ struct LaunchArgs {
     char* ctx_store;
     int pool, ctx_stride;
     unsigned long long n_particles, n_targets, seed, first_id;
+    // sequence calls (fks_forward_simulate_sequence): every particle runs n_legs consecutive legs; leg k of particle i draws
+    // Philox noise as particle first_id + k * leg_id_stride + i (leg_id_stride = the whole batch, also for one device's shard)
+    unsigned long long leg_id_stride;
+    int n_legs;
     int allow_contacts, noise_mode, cfg_stride, rec_stride;
     int P, warps_per_block;
     int pts_off, warps_off;          // byte offsets of the point arrays / the warp blocks in dynamic shared memory

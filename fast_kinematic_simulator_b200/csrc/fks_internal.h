@@ -21,6 +21,18 @@ struct GridGeometry {
 };
 // Returns FKS_OK or FKS_ERR_INVALID_ARGUMENT (message set).  Used by the host and the device builder.
 int compute_grid_geometry(const fks_obstacle* obstacles, size_t n_obstacles, double resolution, GridGeometry* out);
+
+// what a sequence call asks beyond a single call's checks, before anything is allocated or copied: 1 .. 2^31 - 1 legs, their
+// targets, and first_particle_id + n_legs * n computed without overflowing 64 bits (so the last id used is at most 2^64 - 2)
+// -- FKS_OK or FKS_ERR_INVALID_ARGUMENT, message prefixed by `fn`
+int check_sequence(const char* fn, const void* targets, size_t n, size_t n_legs, uint64_t first_particle_id);
+// The host-buffer batch behind fks_forward_simulate_async / fks_forward_simulate_sequence and each device's shard of the
+// multi-GPU calls: copies in, n_legs legs per particle (Philox ids first_particle_id + k * leg_id_stride + i), copies out,
+// asynchronous on the simulator's stream.  Leg k's targets are read at targets + k * targets_pitch (doubles) and its
+// records written at results + k * results_pitch (bytes).  Arguments are checked by the caller.
+int simulate_host_async(fks_sim* s, const double* starts, const double* targets, size_t targets_pitch, size_t n, size_t n_targets,
+                        size_t n_legs, uint64_t leg_id_stride, int allow_contacts, int noise_mode, const fks_noise_tape* tape,
+                        uint64_t first_particle_id, void* results, size_t results_pitch);
 }  // namespace fks_host
 
 // Device environment (fks_env_create / fks_env_build_device).

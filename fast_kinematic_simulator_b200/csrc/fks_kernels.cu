@@ -1786,7 +1786,8 @@ __device__ __forceinline__ void colpiv_qr_solve(int wb, double* A, int ld, int r
     else colpiv_qr_lanes<2>(wb, A, ld, rows, cols, x_off);
 }
 
-// actuator noise of the next `count` microsteps, one truncated-normal draw per axis in axis order (SURVEY A.6)
+// actuator noise of the next `count` microsteps, one truncated-normal draw per axis in axis order (SURVEY A.6); `pid` is the
+// Philox particle id relative to first_id (leg * leg_id_stride + particle in a sequence call)
 __device__ __noinline__ void fill_noise(int wb, unsigned long long pid, unsigned step, unsigned micro0, int count,
                                         unsigned long long tape_pos, unsigned long long tape_end) {
     const Frame& fr = frame();
@@ -1869,6 +1870,10 @@ enum {
     AF_DONE             // no particles left
 };
 enum { NEED_EMPTY = 0, NEED_ROUND = 1, NEED_SOLVE = 2, NEED_DEAD = 3 };  // what a context of the pool waits for
+// WarpVars::leg of a sequence call: set when a leg has ended and the next one is due (AF_FETCH then continues the particle
+// instead of claiming a new one).  A flag rather than an `after` state of its own: an extra case of the state machine's switch
+// changes the single-call kernel's code even where it is never taken.
+constexpr unsigned kLegPending = 0x80000000u;
 
 #ifndef FKS_COPY_UNROLL
 #define FKS_COPY_UNROLL 4
@@ -1895,8 +1900,9 @@ __device__ __forceinline__ void context_copy(double* ws, double* g, const WarpLa
 }  // namespace
 
 // TRACE = true is the single-particle instantiation that records the step trace (fks_forward_simulate_traced); the batch
-// kernel carries none of it.
-template <int KIND, bool TRACE = false>
+// kernel carries none of it.  SEQ = true is the instantiation of sequence calls (n_legs > 1, fks_forward_simulate_sequence):
+// every particle runs n_legs legs; the single-call kernel has no leg logic at all (leg is 0 there).
+template <int KIND, bool TRACE = false, bool SEQ = false>
 __global__ void __launch_bounds__(kThreadsPerBlock, FKS_MIN_BLOCKS) simulate_kernel(const __grid_constant__ LaunchArgs args) {
     // ---- stage parameters, robot and points into shared memory, once per CTA ---------------------
     {
@@ -1973,6 +1979,7 @@ __global__ void __launch_bounds__(kThreadsPerBlock, FKS_MIN_BLOCKS) simulate_ker
         wv->cur = wv->prev = 0;
         wv->m_result = 0.0;
         wv->ctx = warp;
+        if (SEQ) wv->leg = 0u;
     }
     __syncwarp();
 
@@ -2067,6 +2074,7 @@ __global__ void __launch_bounds__(kThreadsPerBlock, FKS_MIN_BLOCKS) simulate_ker
                         wv->cur = wv->prev = 0;
                         wv->m_result = 0.0;
                         wv->ctx = got;
+                        if (SEQ) wv->leg = 0u;
                     }
                     __syncwarp();
                 } else {
@@ -2123,37 +2131,48 @@ __global__ void __launch_bounds__(kThreadsPerBlock, FKS_MIN_BLOCKS) simulate_ker
             if (ev == 0) {
                 switch (after) {
                     case AF_FETCH: {
-                        unsigned long long next_id = 0ull;
-                        if (lane == 0) next_id = (unsigned long long)atomicAdd(a.counter, 1u);
-                        next_id = __shfl_sync(FKS_FULL, next_id, 0);
-                        wv->pid = next_id;  // every lane stores the same value
-                        if (next_id >= a.n_particles) {
-                            after = AF_DONE;
-                            break;
+                        // ForwardSimulateRobot (spcs:824-829): clone + ResetPosition(start).  The start of a fresh particle is
+                        // its entry of `starts`; a later leg of a sequence call starts where the previous leg left the
+                        // particle, as the next call of a chain of single calls would, and its tape positions run on.
+                        const bool next_leg = SEQ && (wv->leg & kLegPending) != 0u;
+                        const unsigned leg = next_leg ? wv->leg & ~kLegPending : 0u;
+                        const double* start = ws + wl.cfg + cur * S;
+                        if (!next_leg) {
+                            unsigned long long next_id = 0ull;
+                            if (lane == 0) next_id = (unsigned long long)atomicAdd(a.counter, 1u);
+                            next_id = __shfl_sync(FKS_FULL, next_id, 0);
+                            wv->pid = next_id;  // every lane stores the same value
+                            if (next_id >= a.n_particles) {
+                                after = AF_DONE;
+                                break;
+                            }
+                            start = a.starts + (size_t)wv->pid * stride;
                         }
-                        // ForwardSimulateRobot (spcs:824-829): clone + ResetPosition(start)
                         cur = 0;
-                        const double* start = a.starts + (size_t)wv->pid * stride;
                         const double* tgt = a.targets + (a.n_targets == a.n_particles ? (size_t)wv->pid * stride : 0);
+                        if (SEQ) tgt += (size_t)leg * a.n_targets * stride;  // targets are leg-major
                         if (lane < stride) {
                             ws[wl.cfg + lane] = start[lane];
                             ws[wl.target + lane] = tgt[lane];
                         }
                         if (lane == 0) *reinterpret_cast<unsigned*>(ws + wl.flags) = 0u;
                         __syncwarp();
+                        if (SEQ) wv->leg = leg;  // every lane has read the pending flag above
                         if (lane < S) {  // pid:98-102 zeroed
                             pid_state[lane] = 0.0;
                             pid_state[S + lane] = 0.0;
                         }
-                        wv->tape_pos = wv->tape_end = 0ull;
-                        if (a.noise_mode == FKS_NOISE_INJECTED) {
-                            wv->tape_pos = a.tape_off[wv->pid];
-                            wv->tape_end = a.tape_off[wv->pid + 1];
-                        }
-                        wv->dec_pos = wv->dec_end = 0ull;
-                        if (a.dec_tape != nullptr) {
-                            wv->dec_pos = a.dec_off[wv->pid];
-                            wv->dec_end = a.dec_off[wv->pid + 1];
+                        if (!next_leg) {
+                            wv->tape_pos = wv->tape_end = 0ull;
+                            if (a.noise_mode == FKS_NOISE_INJECTED) {
+                                wv->tape_pos = a.tape_off[wv->pid];
+                                wv->tape_end = a.tape_off[wv->pid + 1];
+                            }
+                            wv->dec_pos = wv->dec_end = 0ull;
+                            if (a.dec_tape != nullptr) {
+                                wv->dec_pos = a.dec_off[wv->pid];
+                                wv->dec_end = a.dec_off[wv->pid + 1];
+                            }
                         }
                         wv->collided = wv->any_resolve_failed = false;
                         wv->flags = wv->n_micro_total = wv->n_iter_total = wv->n_steps = 0u;
@@ -2337,7 +2356,8 @@ __global__ void __launch_bounds__(kThreadsPerBlock, FKS_MIN_BLOCKS) simulate_ker
                 const int slot = (int)(wv->micro % (unsigned)nb);
                 if (slot == 0) {
                     const unsigned left = wv->number_microsteps - wv->micro;
-                    fill_noise(wb, wv->pid, wv->step, wv->micro, left < (unsigned)nb ? (int)left : nb, wv->tape_pos, wv->tape_end);
+                    const unsigned long long noise_id = SEQ ? wv->pid + (unsigned long long)wv->leg * a.leg_id_stride : wv->pid;
+                    fill_noise(wb, noise_id, wv->step, wv->micro, left < (unsigned)nb ? (int)left : nb, wv->tape_pos, wv->tape_end);
                 }
                 if (a.noise_mode == FKS_NOISE_INJECTED && wv->tape_pos + (unsigned long long)D > wv->tape_end) wv->flags |= FKS_FLAG_TAPE_EXHAUSTED;
                 wv_add(&wv->tape_pos, (unsigned long long)D);
@@ -2386,12 +2406,13 @@ __global__ void __launch_bounds__(kThreadsPerBlock, FKS_MIN_BLOCKS) simulate_ker
                     after = AF_NOCONTACT_KIN;
                 }
             } else {
-                // ---- end of particle: result record = cfg_stride doubles + fks_result_tail -------------------
+                // ---- end of particle (of its leg): result record = cfg_stride doubles + fks_result_tail, leg-major --------
                 ev = 0;
                 if (wv->collided) wv->flags |= FKS_FLAG_DID_CONTACT;
                 __syncwarp();
                 wv->flags |= *reinterpret_cast<const unsigned*>(ws + wl.flags);
                 char* rec = a.results + (size_t)wv->pid * a.rec_stride;
+                if (SEQ) rec += (size_t)wv->leg * a.n_particles * a.rec_stride;  // records are leg-major
                 if (lane < stride) reinterpret_cast<double*>(rec)[lane] = ws[wl.cfg + cur * S + lane];
                 if (lane == 0) {
                     unsigned* tail = reinterpret_cast<unsigned*>(rec + (size_t)stride * 8);
@@ -2404,6 +2425,7 @@ __global__ void __launch_bounds__(kThreadsPerBlock, FKS_MIN_BLOCKS) simulate_ker
                 }
                 __syncwarp();
                 after = AF_FETCH;
+                if (SEQ && wv->leg + 1u < (unsigned)a.n_legs) wv_add(&wv->leg, 1u | kLegPending);  // the next fetch continues it
             }
         }
         }  // end of phase T
@@ -2734,11 +2756,16 @@ size_t simulate_smem_plan(LaunchArgs* args, int L, int J, int D, int P, int stri
     return off;
 }
 
-static const void* kernel_ptr(int kind, bool trace = false) {
+template <int KIND>
+static const void* kernel_ptr_of(bool trace, bool seq) {
+    if (trace) return (const void*)simulate_kernel<KIND, true>;
+    return seq ? (const void*)simulate_kernel<KIND, false, true> : (const void*)simulate_kernel<KIND>;
+}
+static const void* kernel_ptr(int kind, bool trace = false, bool seq = false) {
     switch (kind) {
-        case FKS_ROBOT_SE2: return trace ? (const void*)simulate_kernel<FKS_ROBOT_SE2, true> : (const void*)simulate_kernel<FKS_ROBOT_SE2>;
-        case FKS_ROBOT_SE3: return trace ? (const void*)simulate_kernel<FKS_ROBOT_SE3, true> : (const void*)simulate_kernel<FKS_ROBOT_SE3>;
-        case FKS_ROBOT_LINKED: return trace ? (const void*)simulate_kernel<FKS_ROBOT_LINKED, true> : (const void*)simulate_kernel<FKS_ROBOT_LINKED>;
+        case FKS_ROBOT_SE2: return kernel_ptr_of<FKS_ROBOT_SE2>(trace, seq);
+        case FKS_ROBOT_SE3: return kernel_ptr_of<FKS_ROBOT_SE3>(trace, seq);
+        case FKS_ROBOT_LINKED: return kernel_ptr_of<FKS_ROBOT_LINKED>(trace, seq);
     }
     return nullptr;
 }
@@ -2767,7 +2794,7 @@ int simulate_kernel_info(int kind, size_t dyn_smem, int warps_per_block, KernelI
 int launch_simulate(int kind, const LaunchArgs& args, int grid, size_t dyn_smem, void* stream,
                     const void* l2_window_base, size_t l2_window_bytes) {
     const int block_threads = 32 * args.warps_per_block;
-    const void* fn = kernel_ptr(kind, args.trace != nullptr);
+    const void* fn = kernel_ptr(kind, args.trace != nullptr, args.n_legs > 1);
     if (!fn) return (int)cudaErrorInvalidValue;
     {
         // the attribute is per function and per device, and simulators of the same robot kind share the function: set it for

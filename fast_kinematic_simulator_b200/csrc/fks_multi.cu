@@ -135,13 +135,18 @@ static void shard_of(size_t n, size_t G, size_t d, size_t* lo, size_t* hi) {
     *hi = *lo + base + (d < extra ? 1 : 0);
 }
 
-int fks_multi_forward_simulate(fks_multi_sim* m, const double* starts, const double* targets, size_t n, size_t n_targets,
-                               int allow_contacts, int noise_mode, const fks_noise_tape* tape, uint64_t first_particle_id,
-                               void* results) {
+// n_legs consecutive legs per particle (fks_multi_forward_simulate_sequence; 1 = fks_multi_forward_simulate): every shard keys
+// its Philox ids by the whole batch (leg_id_stride = n) and writes its [n_legs][shard] records into the caller's [n_legs][n] array
+static int multi_simulate(fks_multi_sim* m, const double* starts, const double* targets, size_t n, size_t n_targets, size_t n_legs,
+                          int allow_contacts, int noise_mode, const fks_noise_tape* tape, uint64_t first_particle_id, void* results) {
     if (!m) return mfail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_forward_simulate: null simulator");
     if (n == 0) return FKS_OK;
     if (!starts || !targets || !results || !(n_targets == 1 || n_targets == n))
         return mfail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_forward_simulate: need buffers and 1 target or one per start");
+    if (noise_mode != FKS_NOISE_PHILOX && noise_mode != FKS_NOISE_INJECTED && noise_mode != FKS_NOISE_NONE)
+        return mfail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_forward_simulate: unknown noise mode");
+    if (noise_mode == FKS_NOISE_INJECTED && (!tape || !tape->draws || !tape->offsets))
+        return mfail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_forward_simulate: injected noise needs a tape");
     const size_t G = m->devices.size();
     const size_t stride = (size_t)m->cfg_stride;
     int rc = FKS_OK;
@@ -170,15 +175,29 @@ int fks_multi_forward_simulate(fks_multi_sim* m, const double* starts, const dou
             }
             t = &tapes[d];
         }
-        rc = fks_forward_simulate_async(m->sims[d], starts + lo * stride, n_targets == n ? targets + lo * stride : targets, hi - lo,
-                                        n_targets == n ? hi - lo : 1, allow_contacts, noise_mode, t, first_particle_id + lo,
-                                        (char*)results + lo * m->rec_stride);
+        rc = fks_host::simulate_host_async(m->sims[d], starts + lo * stride, n_targets == n ? targets + lo * stride : targets,
+                                           n_targets * stride, hi - lo, n_targets == n ? hi - lo : 1, n_legs, n, allow_contacts, noise_mode,
+                                           t, first_particle_id + lo, (char*)results + lo * m->rec_stride, n * m->rec_stride);
     }
     for (size_t d = 0; d < G; d++) {
         const int rs = fks_sim_synchronize(m->sims[d]);
         if (rc == FKS_OK) rc = rs;
     }
     return rc;
+}
+
+int fks_multi_forward_simulate(fks_multi_sim* m, const double* starts, const double* targets, size_t n, size_t n_targets,
+                               int allow_contacts, int noise_mode, const fks_noise_tape* tape, uint64_t first_particle_id,
+                               void* results) {
+    return multi_simulate(m, starts, targets, n, n_targets, 1, allow_contacts, noise_mode, tape, first_particle_id, results);
+}
+
+int fks_multi_forward_simulate_sequence(fks_multi_sim* m, const double* starts, const double* targets, size_t n, size_t n_targets,
+                                        size_t n_legs, int allow_contacts, int noise_mode, const fks_noise_tape* tape,
+                                        uint64_t first_particle_id, void* results) {
+    const int rc = fks_host::check_sequence("fks_multi_forward_simulate_sequence", targets, n, n_legs, first_particle_id);
+    if (rc != FKS_OK) return rc;
+    return multi_simulate(m, starts, targets, n, n_targets, n_legs, allow_contacts, noise_mode, tape, first_particle_id, results);
 }
 
 int fks_multi_forward_simulate_device(fks_multi_sim* m, const double* const* d_starts, const double* const* d_targets, size_t n,

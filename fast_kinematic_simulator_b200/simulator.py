@@ -9,6 +9,9 @@ Names follow the reference:
 * ``GpuParticleContactSimulator.forward_simulate_robots`` <- SimpleParticleContactSimulator::
   ForwardSimulateRobots (simple_particle_contact_simulator.hpp:788-804); ``reverse_simulate_robots``
   (:806-822); ``get_statistics`` / ``reset_statistics`` (:488-512).
+* ``forward_simulate_sequence`` runs every particle through several consecutive ForwardSimulateRobot legs in one call
+  (fks_forward_simulate_sequence): the records equal those of chained ``forward_simulate_robots`` calls whose
+  ``first_particle_id`` advances by n per call.
 
 Everything computes in libfksgpu.so; this module only marshals numpy arrays across the C ABI.
 """
@@ -211,6 +214,18 @@ def make_tape(draws, offsets, decisions=None, decision_offsets=None):
     return t, keep
 
 
+def sequence_inputs(starts, targets, stride):
+    """Checked arrays of a sequence call: starts (n, stride); targets (M, n_targets, stride), (M, stride) meaning one
+    target per leg."""
+    starts = _as_f64(starts).reshape(-1, stride)
+    targets = _as_f64(targets)
+    if targets.ndim == 2:
+        targets = targets.reshape(targets.shape[0], 1, targets.shape[1])
+    if targets.ndim != 3 or targets.shape[2] != stride:
+        raise ValueError("sequence targets must have shape (legs, n_targets, %d) or (legs, %d), not %s" % (stride, stride, targets.shape))
+    return starts, np.ascontiguousarray(targets)
+
+
 def _dev_ptr(x):
     if x is None:
         return None
@@ -254,7 +269,32 @@ class GpuParticleContactSimulator:
                                 first_particle_id=0, out=None):
         return self._simulate(lib.fks_reverse_simulate, starts, targets, allow_contacts, noise_mode, tape, first_particle_id, out)
 
+    def forward_simulate_sequence(self, starts, targets, allow_contacts=True, noise_mode=capi.NOISE_PHILOX, tape=None,
+                                  first_particle_id=0, out=None):
+        """Every particle through M consecutive legs in one kernel launch (fks_forward_simulate_sequence): leg k drives it from
+        where leg k-1 left it to targets[k].  targets: (M, n_targets, stride) or (M, stride).  Returns SimulationResults over
+        records of shape (M, n), equal to M chained forward_simulate_robots calls with first_particle_id + k * n.  An injected
+        tape holds one span per particle covering all its legs."""
+        starts, targets = sequence_inputs(starts, targets, self.config_stride)
+        n, (m, n_targets) = starts.shape[0], targets.shape[:2]
+        if out is None:
+            out = np.empty((m, n), dtype=self.dtype)
+        ctape, keep = (None, None)
+        if tape is not None:
+            ctape, keep = make_tape(*tape)
+        check(lib.fks_forward_simulate_sequence(self._h, starts.ctypes.data, targets.ctypes.data, n, n_targets, m, int(bool(allow_contacts)),
+                                                int(noise_mode), C.byref(ctape) if ctape is not None else None, int(first_particle_id),
+                                                out.ctypes.data))
+        return SimulationResults(out)
+
     # -- device-resident variant (torch tensors or raw pointers), asynchronous on `stream` --------
+    def forward_simulate_sequence_device(self, d_starts, d_targets, n, n_targets, n_legs, d_results, allow_contacts=True,
+                                         noise_mode=capi.NOISE_PHILOX, d_tape=None, d_tape_offsets=None, first_particle_id=0, stream=0):
+        """forward_simulate_sequence on device buffers: d_targets [n_legs][n_targets][stride], d_results [n_legs][n] records."""
+        check(lib.fks_forward_simulate_sequence_device(self._h, _dev_ptr(d_starts), _dev_ptr(d_targets), int(n), int(n_targets), int(n_legs),
+                                                       int(bool(allow_contacts)), int(noise_mode), _dev_ptr(d_tape), _dev_ptr(d_tape_offsets),
+                                                       int(first_particle_id), _dev_ptr(d_results), int(stream) if stream else None))
+
     def forward_simulate_device(self, d_starts, d_targets, n, n_targets, d_results, allow_contacts=True,
                                 noise_mode=capi.NOISE_PHILOX, d_tape=None, d_tape_offsets=None, first_particle_id=0, stream=0):
         def ptr(x):
@@ -429,6 +469,22 @@ class MultiGpuParticleContactSimulator:
         check(lib.fks_multi_forward_simulate(self._h, starts.ctypes.data, targets.ctypes.data, n, targets.shape[0],
                                              int(bool(allow_contacts)), int(noise_mode), C.byref(ctape) if ctape is not None else None,
                                              int(first_particle_id), out.ctypes.data))
+        return SimulationResults(out)
+
+    def forward_simulate_sequence(self, starts, targets, allow_contacts=True, noise_mode=capi.NOISE_PHILOX, tape=None,
+                                  first_particle_id=0, out=None):
+        """GpuParticleContactSimulator.forward_simulate_sequence over the devices (fks_multi_forward_simulate_sequence)."""
+        starts, targets = sequence_inputs(starts, targets, self.config_stride)
+        n, (m, n_targets) = starts.shape[0], targets.shape[:2]
+        if out is None:
+            out = np.empty((m, n), dtype=self.dtype)
+        ctape, keep = (None, None)
+        if tape is not None:
+            ctape, keep = make_tape(*tape)
+        check(lib.fks_multi_forward_simulate_sequence(self._h, starts.ctypes.data, targets.ctypes.data, n, n_targets, m,
+                                                      int(bool(allow_contacts)), int(noise_mode),
+                                                      C.byref(ctape) if ctape is not None else None, int(first_particle_id),
+                                                      out.ctypes.data))
         return SimulationResults(out)
 
     def forward_simulate_device(self, d_starts, d_targets, n, n_targets, d_results, allow_contacts=True, first_particle_id=0):

@@ -285,6 +285,41 @@ int fks_forward_simulate_device(fks_sim* sim, const double* d_starts, const doub
                                 const uint64_t* d_tape_offsets, uint64_t first_particle_id,
                                 void* d_results, void* cuda_stream);
 
+/* Sequence call: every particle runs n_legs consecutive legs in ONE kernel launch; leg k is exactly one ForwardSimulateRobot
+ * (spcs.hpp:824-829) from where leg k-1 left the particle towards leg k's target.  The records equal, byte for byte, those of
+ * the chain of single calls
+ *     for k in 0 .. n_legs-1:
+ *         fks_forward_simulate(sim, starts_k, targets + k * n_targets * cfg_stride, n, n_targets, allow_contacts, noise_mode,
+ *                              tape_k, first_particle_id + k * n, results + k * n * fks_sim_result_stride(sim))
+ *         starts_{k+1} = the configurations of those records
+ * in every noise mode, and so do the statistics (fks_get_statistics afterwards = the chain's sum).
+ *  - noise: leg k of particle i draws Philox noise as particle first_particle_id + k * n_particles + i, controller steps counted
+ *    from 0 inside the leg -- the ids a caller that advances first_particle_id by n_particles per call uses;
+ *  - each leg restarts like ForwardSimulateRobot: PID state zeroed (ResetPosition), flags and counters cleared.  A leg that
+ *    ended by a failed resolve, the shortcut distance or a stop with allow_contacts == 0 still hands its end state on;
+ *  - targets: leg-major, [n_legs][n_targets][cfg_stride]; n_targets is 1 or n_particles, the same for every leg;
+ *  - results: leg-major, [n_legs][n_particles] records of fks_sim_result_stride() bytes: leg k's records are a batch result
+ *    of their own (fks_end_states_* take them at d_results + k * n_particles * stride);
+ *  - injected tapes: ONE span per particle (offsets / decision_offsets have n_particles + 1 entries) holding the particle's
+ *    per-leg spans of the chain's tapes one after the other.  The tape positions are not reset between legs, so the equality
+ *    with the chain holds when every leg consumes exactly its own span -- as when the tapes record the same trajectories.
+ *    A leg that consumes fewer draws or decision records than its span (e.g. a particle that desynchronised from the recorded
+ *    run) shifts every later leg's draws, and one that consumes more reads the next leg's draws instead of raising
+ *    FKS_FLAG_TAPE_EXHAUSTED (only the particle's last leg can run out);
+ *  - n_legs == 1 is fks_forward_simulate.
+ * n_legs == 0 or above 2^31 - 1, a null `targets` or first_particle_id + n_legs * n_particles beyond 64 bits (the sum itself must
+ * not wrap) is FKS_ERR_INVALID_ARGUMENT;
+ * n_particles == 0 launches nothing.  The _device flavour takes device buffers and runs asynchronously on `cuda_stream` like
+ * fks_forward_simulate_device; the _multi flavour shards the particles over the devices like fks_multi_forward_simulate
+ * (records do not depend on the device count). */
+int fks_forward_simulate_sequence(fks_sim* sim, const double* starts, const double* targets, size_t n_particles,
+                                  size_t n_targets, size_t n_legs, int allow_contacts, int noise_mode,
+                                  const fks_noise_tape* tape, uint64_t first_particle_id, void* results);
+int fks_forward_simulate_sequence_device(fks_sim* sim, const double* d_starts, const double* d_targets, size_t n_particles,
+                                         size_t n_targets, size_t n_legs, int allow_contacts, int noise_mode,
+                                         const double* d_tape_draws, const uint64_t* d_tape_offsets,
+                                         uint64_t first_particle_id, void* d_results, void* cuda_stream);
+
 /* CheckConfigCollision (spcs.hpp:1398-1416), batched: out_collides[i] = 1 when configuration i collides with the
  * environment inflated by inflation_ratio cells (CheckEnvironmentCollision, spcs.hpp:921-981 with threshold
  * inflation_ratio * resolution) or with itself (CheckSelfCollisions, spcs.hpp:1324-1396, cells of
@@ -357,6 +392,10 @@ size_t fks_multi_sim_result_stride(const fks_multi_sim* sim);
 int fks_multi_forward_simulate(fks_multi_sim* sim, const double* starts, const double* targets, size_t n_particles,
                                size_t n_targets, int allow_contacts, int noise_mode, const fks_noise_tape* tape,
                                uint64_t first_particle_id, void* results);
+/* fks_forward_simulate_sequence over the devices: host buffers, same layouts, tapes sharded like fks_multi_forward_simulate */
+int fks_multi_forward_simulate_sequence(fks_multi_sim* sim, const double* starts, const double* targets, size_t n_particles,
+                                        size_t n_targets, size_t n_legs, int allow_contacts, int noise_mode,
+                                        const fks_noise_tape* tape, uint64_t first_particle_id, void* results);
 int fks_multi_forward_simulate_device(fks_multi_sim* sim, const double* const* d_starts, const double* const* d_targets,
                                       size_t n_particles, size_t n_targets, int allow_contacts, uint64_t first_particle_id,
                                       void* const* d_results);

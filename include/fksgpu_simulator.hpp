@@ -163,6 +163,25 @@ struct NoiseTape {
     }
 };
 
+// flattens the inputs of a sequence call (starts [n][stride], targets [leg][n_targets][stride]) and returns n_targets; throws
+// std::invalid_argument when there is no leg or the legs' target counts differ or are not 1 / n
+template <typename Configuration>
+size_t FlattenSequence(const std::vector<Configuration>& starts, const std::vector<std::vector<Configuration>>& targets_per_leg, int stride,
+                       std::vector<double>* hs, std::vector<double>* ht) {
+    const size_t n = starts.size(), s = (size_t)stride;
+    if (targets_per_leg.empty()) throw std::invalid_argument("fksgpu: a sequence needs at least one leg");
+    const size_t n_targets = targets_per_leg[0].size();
+    for (const auto& leg : targets_per_leg)
+        if (leg.size() != n_targets || !(n_targets == 1 || n_targets == n))
+            throw std::invalid_argument("fksgpu: every leg needs the same number of targets, 1 or one per start");
+    hs->resize(n * s);
+    ht->resize(targets_per_leg.size() * n_targets * s);
+    for (size_t i = 0; i < n; i++) ConfigTraits<Configuration>::Flatten(starts[i], hs->data() + i * s, stride);
+    for (size_t k = 0; k < targets_per_leg.size(); k++)
+        for (size_t i = 0; i < n_targets; i++) ConfigTraits<Configuration>::Flatten(targets_per_leg[k][i], ht->data() + (k * n_targets + i) * s, stride);
+    return n_targets;
+}
+
 template <typename Configuration>
 class GpuParticleContactSimulator : public SimulatorInterface<Configuration> {
 public:
@@ -259,6 +278,34 @@ public:
             }
         }
         return Unpack(result.data(), target);
+    }
+
+    // M consecutive ForwardSimulateRobot legs per particle in one call (fks_forward_simulate_sequence): leg k drives every
+    // particle from where leg k-1 left it to targets_per_leg[k] (1 target or one per start, the same count for every leg).
+    // Returns [leg][particle]; equal to M consecutive ForwardSimulateRobots calls (the particle id advances by n * M).
+    std::vector<std::vector<Result>> ForwardSimulateRobotsSequence(const std::vector<Configuration>& start_positions,
+                                                                   const std::vector<std::vector<Configuration>>& targets_per_leg,
+                                                                   bool allow_contacts) {
+        const size_t n = start_positions.size(), m = targets_per_leg.size();
+        std::vector<double> hs, ht;
+        const size_t n_targets = FlattenSequence(start_positions, targets_per_leg, stride_, &hs, &ht);
+        std::vector<unsigned char> rec(m * n * record_);
+        fks_noise_tape view;
+        const fks_noise_tape* tape = nullptr;
+        if (noise_mode_ == FKS_NOISE_INJECTED) {
+            if (!tape_ || tape_->offsets.size() != n + 1) throw std::invalid_argument("fksgpu: the noise tape does not match the batch");
+            view = tape_->View();
+            tape = &view;
+        }
+        Check(fks_forward_simulate_sequence(sim_, hs.data(), ht.data(), n, n_targets, m, allow_contacts ? 1 : 0, noise_mode_, tape,
+                                            next_particle_id_, rec.data()));
+        next_particle_id_ += n * m;
+        if (noise_mode_ == FKS_NOISE_INJECTED) SetNoiseMode(FKS_NOISE_PHILOX);  // a tape describes one call
+        std::vector<std::vector<Result>> out(m, std::vector<Result>(n));
+        for (size_t k = 0; k < m; k++)
+            for (size_t i = 0; i < n; i++)
+                out[k][i] = Unpack(rec.data() + (k * n + i) * record_, n_targets == 1 ? targets_per_leg[k][0] : targets_per_leg[k][i]);
+        return out;
     }
 
     // spcs.hpp:1398: planner-side static query (environment inflated by inflation_ratio cells, self collisions)
@@ -411,19 +458,24 @@ public:
                                          next_particle_id_, rec.data()));
         next_particle_id_ += n;
         std::vector<Result> out(n);
-        for (size_t i = 0; i < n; i++) {
-            const unsigned char* r = rec.data() + i * record_;
-            fks_result_tail tail;
-            std::memcpy(&tail, r + sizeof(double) * (size_t)stride_, sizeof(tail));
-            out[i].result_config = ConfigTraits<Configuration>::Unflatten(reinterpret_cast<const double*>(r), stride_);
-            out[i].actual_target = targets.size() == 1 ? targets[0] : targets[i];
-            out[i].did_contact = (tail.flags & FKS_FLAG_DID_CONTACT) != 0;
-            out[i].outcome_is_nominal = true;
-            out[i].flags = tail.flags;
-            out[i].n_microsteps = tail.n_microsteps;
-            out[i].n_resolver_iterations = tail.n_resolver_iters;
-            out[i].n_steps = tail.n_steps;
-        }
+        for (size_t i = 0; i < n; i++) out[i] = Unpack(rec.data() + i * record_, targets.size() == 1 ? targets[0] : targets[i]);
+        return out;
+    }
+    // GpuParticleContactSimulator::ForwardSimulateRobotsSequence over all devices
+    std::vector<std::vector<Result>> ForwardSimulateRobotsSequence(const std::vector<Configuration>& starts,
+                                                                   const std::vector<std::vector<Configuration>>& targets_per_leg,
+                                                                   bool allow_contacts) {
+        const size_t n = starts.size(), m = targets_per_leg.size();
+        std::vector<double> hs, ht;
+        const size_t n_targets = FlattenSequence(starts, targets_per_leg, stride_, &hs, &ht);
+        std::vector<unsigned char> rec(m * n * record_);
+        Check(fks_multi_forward_simulate_sequence(sim_, hs.data(), ht.data(), n, n_targets, m, allow_contacts ? 1 : 0, FKS_NOISE_PHILOX,
+                                                  nullptr, next_particle_id_, rec.data()));
+        next_particle_id_ += n * m;
+        std::vector<std::vector<Result>> out(m, std::vector<Result>(n));
+        for (size_t k = 0; k < m; k++)
+            for (size_t i = 0; i < n; i++)
+                out[k][i] = Unpack(rec.data() + (k * n + i) * record_, n_targets == 1 ? targets_per_leg[k][0] : targets_per_leg[k][i]);
         return out;
     }
     std::vector<uint64_t> GetStatisticCounters() {
@@ -435,6 +487,21 @@ public:
     void SetNextParticleId(uint64_t id) { next_particle_id_ = id; }
 
 private:
+    Result Unpack(const unsigned char* r, const Configuration& target) const {
+        Result out;
+        fks_result_tail tail;
+        std::memcpy(&tail, r + sizeof(double) * (size_t)stride_, sizeof(tail));
+        out.result_config = ConfigTraits<Configuration>::Unflatten(reinterpret_cast<const double*>(r), stride_);
+        out.actual_target = target;
+        out.did_contact = (tail.flags & FKS_FLAG_DID_CONTACT) != 0;
+        out.outcome_is_nominal = true;
+        out.flags = tail.flags;
+        out.n_microsteps = tail.n_microsteps;
+        out.n_resolver_iterations = tail.n_resolver_iters;
+        out.n_steps = tail.n_steps;
+        return out;
+    }
+
     fks_multi_sim* sim_;
     int stride_ = 0;
     size_t record_ = 0;
