@@ -7,6 +7,7 @@ OK, ERR_INVALID_ARGUMENT, ERR_CUDA, ERR_NO_DEVICE, ERR_UNSUPPORTED, ERR_OUT_OF_M
 ROBOT_SE2, ROBOT_SE3, ROBOT_LINKED = 0, 1, 2
 JOINT_PRISMATIC, JOINT_REVOLUTE, JOINT_CONTINUOUS, JOINT_FIXED = 0, 1, 2, 3
 NOISE_PHILOX, NOISE_INJECTED, NOISE_NONE = 0, 1, 2
+LINKAGE_SINGLE, LINKAGE_COMPLETE = 0, 1
 FLAG_DID_CONTACT = 1 << 0
 FLAG_RESOLVE_FAILED = 1 << 1
 FLAG_ENDED_BY_FAILURE = 1 << 2

@@ -75,6 +75,7 @@ EXPORTS = (
     "fks_env_download",
     "fks_end_states_partition",
     "fks_end_states_pairwise_distance",
+    "fks_end_states_cluster",
     "fks_debug_qr_solve",
     "fks_measure_fp64_peak",
     "fks_measure_gather_rate",
@@ -152,6 +153,8 @@ lib.fks_env_build_timings.argtypes = [C.c_void_p, P(C.c_double), C.c_int]
 lib.fks_env_download.argtypes = [C.c_void_p, P(C.c_void_p)]
 lib.fks_end_states_partition.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, P(C.c_uint64), C.c_void_p]
 lib.fks_end_states_pairwise_distance.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]
+lib.fks_end_states_cluster.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, P(C.c_uint64), C.c_size_t, C.c_int, C.c_double, C.c_int,
+                                       C.c_void_p, P(C.c_uint64), C.c_void_p]
 lib.fks_debug_qr_solve.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_size_t, C.c_void_p, C.c_void_p]
 lib.fks_measure_fp64_peak.argtypes = [C.c_int, P(C.c_double)]
 lib.fks_measure_gather_rate.argtypes = [C.c_int, C.c_size_t, P(C.c_double)]

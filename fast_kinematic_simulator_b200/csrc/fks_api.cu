@@ -118,6 +118,11 @@ struct fks_sim {
     size_t cap_starts, cap_targets, cap_tape, cap_tape_off, cap_results, cap_dec, cap_dec_off;
     unsigned int* d_part = nullptr;  // fks_end_states_partition: totals + per-block counts
     size_t cap_part = 0;
+    // fks_end_states_cluster: [offsets | totals | counts, segment lists] and the distance matrices of the large segments
+    unsigned long long* d_clu = nullptr;
+    size_t cap_clu = 0;
+    double* d_clu_mat = nullptr;
+    size_t cap_clu_mat = 0;
     unsigned long long* d_trace_buf = nullptr;  // fks_forward_simulate_traced: [counter word | records], grown on demand
     size_t cap_trace_buf = 0;
     size_t smem_limit;
@@ -675,6 +680,8 @@ void fks_sim_destroy(fks_sim* s) {
     cudaFree(s->d_dec_off);
     cudaFree(s->d_trace_buf);
     cudaFree(s->d_part);
+    cudaFree(s->d_clu);
+    cudaFree(s->d_clu_mat);
     cudaFree(s->d_ctx_store);
     cudaFree(s->d_results);
     if (s->last_done) cudaEventDestroy(s->last_done);
@@ -1093,6 +1100,94 @@ int fks_end_states_pairwise_distance(fks_sim* s, const void* d_results, const ui
                                             s->robot->stride, d_subset, (unsigned)m, d_out, cuda_stream);
     if (rc != 0) return cuda_fail((cudaError_t)rc, "fks_end_states_pairwise_distance: launch");
     s->launches += 1;
+    return FKS_OK;
+}
+
+int fks_end_states_cluster(fks_sim* s, const void* d_results, const uint32_t* d_order, const uint64_t* segment_offsets, size_t n_segments,
+                           int linkage, double max_cluster_distance, int separate_contact, uint32_t* d_labels, uint64_t* cluster_counts,
+                           void* cuda_stream) {
+    if (!s) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_cluster: null simulator");
+    if (std::isnan(max_cluster_distance)) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_cluster: max_cluster_distance is NaN");
+    if (linkage != FKS_LINKAGE_SINGLE && linkage != FKS_LINKAGE_COMPLETE) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_cluster: unknown linkage");
+    if (n_segments == 0) return FKS_OK;
+    if (!segment_offsets || !cluster_counts) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_cluster: null segment offsets or counts");
+    if (n_segments > 0xffffffffull) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_cluster: more than 2^32 - 1 segments");
+    if (segment_offsets[0] != 0) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_cluster: segment_offsets[0] must be 0");
+    std::vector<uint32_t> small_segs, large_segs;
+    unsigned small_cap = 0, large_cap = 0;
+    for (size_t i = 0; i < n_segments; i++) {
+        if (segment_offsets[i + 1] < segment_offsets[i]) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_cluster: segment_offsets decrease");
+        const uint64_t len = segment_offsets[i + 1] - segment_offsets[i];
+        if (len > kClusterMaxSegment)
+            return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_cluster: a segment is longer than " + std::to_string(kClusterMaxSegment) + " positions");
+        if (len == 0) continue;
+        if (len <= kClusterSmallMax) {
+            small_segs.push_back((uint32_t)i);
+            small_cap = std::max(small_cap, (unsigned)len);
+        } else {
+            large_segs.push_back((uint32_t)i);
+            large_cap = std::max(large_cap, (unsigned)len);
+        }
+    }
+    const uint64_t m = segment_offsets[n_segments];
+    if (m > 0xffffffffull) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_cluster: 2^32 or more positions");
+    std::fill(cluster_counts, cluster_counts + n_segments, (uint64_t)0);
+    if (m == 0) return FKS_OK;
+    if (!d_results || !d_labels) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_cluster: null records or labels");
+    NvtxRange range("fks_end_states_cluster");
+    DeviceGuard guard(s->device);
+    if (!guard.ok) return fail(FKS_ERR_CUDA, "fks_end_states_cluster: cudaSetDevice failed");
+    cudaStream_t stream = (cudaStream_t)cuda_stream;
+
+    // one upload: [offsets (n + 1) | totals (2) | counts (n, zero), small segments, large segments as u32]
+    const size_t n_u32 = n_segments + small_segs.size() + large_segs.size();
+    std::vector<unsigned long long> meta(n_segments + 3 + (n_u32 + 1) / 2, 0ull);
+    std::memcpy(meta.data(), segment_offsets, (n_segments + 1) * sizeof(uint64_t));
+    uint32_t* meta32 = reinterpret_cast<uint32_t*>(meta.data() + n_segments + 3);
+    std::copy(small_segs.begin(), small_segs.end(), meta32 + n_segments);
+    std::copy(large_segs.begin(), large_segs.end(), meta32 + n_segments + small_segs.size());
+    int rc;
+    if ((rc = ensure(&s->d_clu, &s->cap_clu, meta.size())) != FKS_OK) return rc;
+    // large segments: one matrix slot per CTA, as many CTAs as SMs, segments and a 1 GiB workspace allow (at least one)
+    int large_slots = 0;
+    if (!large_segs.empty()) {
+        const size_t slot = (size_t)large_cap * large_cap;
+        large_slots = (int)std::max<size_t>(1, std::min<size_t>({large_segs.size(), (size_t)s->num_sms, ((size_t)1 << 30) / (slot * sizeof(double))}));
+        if ((rc = ensure(&s->d_clu_mat, &s->cap_clu_mat, slot * large_slots)) != FKS_OK) return rc;
+    }
+    FKS_CUDA(cudaMemcpyAsync(s->d_clu, meta.data(), meta.size() * sizeof(unsigned long long), cudaMemcpyHostToDevice, stream));
+    unsigned* d32 = reinterpret_cast<unsigned*>(s->d_clu + n_segments + 3);
+    ClusterLaunch c;
+    c.robot = s->robot->d_robot;
+    c.results = (const char*)d_results;
+    c.rec_stride = fks_sim_result_stride(s);
+    c.cfg_stride = s->robot->stride;
+    c.complete = linkage == FKS_LINKAGE_COMPLETE;
+    c.separate_contact = separate_contact != 0;
+    c.threshold = max_cluster_distance;
+    c.order = d_order;
+    c.offsets = s->d_clu;
+    c.n_segments = (unsigned)n_segments;
+    c.small_segs = d32 + n_segments;
+    c.n_small = (unsigned)small_segs.size();
+    c.small_cap = small_cap;
+    c.large_segs = d32 + n_segments + small_segs.size();
+    c.n_large = (unsigned)large_segs.size();
+    c.large_cap = large_cap;
+    c.work = s->d_clu_mat;
+    c.large_slots = large_slots;
+    c.labels = d_labels;
+    c.counts = d32;
+    c.totals = s->d_clu + n_segments + 1;
+    rc = launch_cluster(s->robot->host.kind, c, stream);
+    if (rc != 0) return cuda_fail((cudaError_t)rc, "fks_end_states_cluster: launch");
+    s->launches += 2 + (small_segs.empty() ? 0 : 1) + (large_segs.empty() ? 0 : 1);
+    std::vector<unsigned> base(n_segments);
+    unsigned long long total = 0;
+    FKS_CUDA(cudaMemcpyAsync(base.data(), d32, n_segments * sizeof(unsigned), cudaMemcpyDeviceToHost, stream));
+    FKS_CUDA(cudaMemcpyAsync(&total, c.totals + 1, sizeof(total), cudaMemcpyDeviceToHost, stream));
+    FKS_CUDA(cudaStreamSynchronize(stream));
+    for (size_t i = 0; i < n_segments; i++) cluster_counts[i] = (i + 1 < n_segments ? base[i + 1] : total) - base[i];
     return FKS_OK;
 }
 

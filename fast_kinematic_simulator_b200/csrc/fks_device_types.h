@@ -324,6 +324,33 @@ int launch_partition(const char* results, size_t rec_stride, int cfg_stride, siz
                      unsigned* order, void* stream);
 int launch_pairwise_distance(int kind, const DevRobot* robot, const char* results, size_t rec_stride, int cfg_stride, const unsigned* subset,
                              unsigned m, double* out, void* stream);
+// fks_end_states_cluster: segments of up to kClusterSmallMax positions keep their distance matrix in shared memory (160^2
+// doubles = 200 KiB of the 227 KiB a CTA can have), longer ones in a global slot of large_cap^2 doubles per CTA; the
+// per-position state of a segment (20 bytes each) stays in shared memory, which bounds a segment at kClusterMaxSegment.
+constexpr unsigned kClusterSmallMax = 160;
+constexpr unsigned kClusterMaxSegment = 8192;
+struct ClusterLaunch {
+    const DevRobot* robot;
+    const char* results;
+    size_t rec_stride;
+    int cfg_stride;
+    int complete, separate_contact;
+    double threshold;
+    const unsigned* order;              // device, or null
+    const unsigned long long* offsets;  // device [n_segments + 1]
+    unsigned n_segments;
+    const unsigned* small_segs;         // device: the non-empty segments of at most kClusterSmallMax positions
+    unsigned n_small, small_cap;        // their number and the longest one
+    const unsigned* large_segs;         // device: the longer segments
+    unsigned n_large, large_cap;
+    double* work;                       // large_slots * large_cap^2 doubles
+    int large_slots;
+    unsigned* labels;                   // [m]
+    unsigned* counts;                   // device [n_segments], zeroed: clusters per segment, then their exclusive scan
+    unsigned long long* totals;         // device [2]: totals[1] = all clusters
+};
+// the launches of one call: the two clustering kernels (those with segments), the scan of the counts and the relabel pass
+int launch_cluster(int kind, const ClusterLaunch& c, void* stream);
 int launch_dbg_copy(unsigned long long* out, void* stream);  // developer counters of the FKS_PHASE_TIMERS build
 int launch_fp64_peak(double* out, int grid, int iters, void* stream);
 int launch_gather(const float* data, unsigned long long n_mask, float* out, int grid, int iters, void* stream);

@@ -2969,6 +2969,317 @@ int launch_pairwise_distance(int kind, const DevRobot* robot, const char* result
     return (int)cudaGetLastError();
 }
 
+// ---------------------------------------------------------------------------------------------
+// fks_end_states_cluster: flat agglomerative clustering (single / complete linkage, distance cutoff) of every segment of a
+// position range, one CTA per segment.  A segment's distances form the upper triangle of an n x n matrix D (row pitch n):
+// D[p][q], p < q, is the pairwise kernel's entry [p][q] for the same records, +inf where that is NaN or the contact flags
+// differ under separate_contact.  Small segments keep D in shared memory, large ones in a global slot of the CTA.
+//
+// Merge loop.  A cluster is named by its smallest position (its representative); only representatives' rows and columns of D
+// are finite, the others are +inf.  nn[i] / nnd[i] cache the smallest (D[i][j], j) over j > i, so the smallest
+// (nnd[i], i, nn[i]) over i is the smallest merge key (L, min rep, max rep).  Merging a < b writes op(D[a][k], D[b][k]) into
+// a's row and column (op = min for single, max for complete linkage: the Lance-Williams update of the two, exact), sets b's
+// to +inf, and repairs the cache: row a is rescanned, so is every row whose neighbour was a or b (b is gone; under complete
+// linkage a's distances grew), and a row i < a with another neighbour only compares its cache with the new D[i][a] -- under
+// single linkage it can only have shrunk, under complete linkage it grew from a value that already lost.
+// ---------------------------------------------------------------------------------------------
+constexpr int kClusterSmallBlock = 256;
+constexpr int kClusterLargeBlock = 1024;
+
+struct ClusterArgs {
+    const DevRobot* robot;
+    const char* results;
+    size_t rec_stride;
+    int cfg_stride;
+    int complete;
+    int separate_contact;
+    double threshold;
+    const unsigned* order;                // position -> record id, or null (identity)
+    const unsigned long long* offsets;    // [n_segments + 1]
+    const unsigned* segs;                 // segment ids this launch clusters
+    unsigned n_segs;
+    unsigned n_cap;                       // largest segment of this launch
+    double* work;                         // large path: one n_cap x n_cap slot per CTA
+    unsigned* labels;                     // [m]: segment-local cluster ids (the relabel kernel adds the segment's base)
+    unsigned* counts;                     // [n_segments]: clusters per segment
+};
+
+// per-segment state in shared memory behind the matrix (small path) or at the start of it (large path)
+struct ClusterSmem {
+    unsigned* rep;   // [n_cap] representative of each position
+    unsigned* nn;    // [n_cap] cached nearest j > i (n = none), reused for the ranks of the representatives at the end
+    double* nnd;     // [n_cap] D[i][nn[i]]
+    unsigned* list;  // [n_cap] rows to rescan
+};
+__host__ __device__ inline size_t cluster_state_bytes(unsigned n_cap) { return (size_t)n_cap * (8 + 4 + 4 + 4); }
+
+struct ClusterShared {
+    double wd[32];
+    unsigned wi[32];
+    unsigned a, b, go, n_list, carry;
+};
+
+__device__ __forceinline__ bool cluster_key_less(double d, unsigned i, double e, unsigned j) { return d < e || (d == e && i < j); }
+
+// (d, i) of the warp's smallest key, in every lane
+__device__ __forceinline__ void cluster_warp_min(double& d, unsigned& i) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const double od = __shfl_xor_sync(FKS_FULL, d, o);
+        const unsigned oi = __shfl_xor_sync(FKS_FULL, i, o);
+        if (cluster_key_less(od, oi, d, i)) {
+            d = od;
+            i = oi;
+        }
+    }
+}
+
+// one warp: nn[i] / nnd[i] = smallest (D[i][j], j) over j > i (none: n / +inf)
+__device__ __forceinline__ void cluster_rescan_row(const double* D, unsigned n, unsigned i, ClusterSmem& st) {
+    const int lane = threadIdx.x & 31;
+    const double* row = D + (size_t)i * n;
+    double bd = INFINITY;
+    unsigned bj = n;
+    for (unsigned j = i + 1 + lane; j < n; j += 32) {
+        const double d = row[j];
+        if (d < bd) {
+            bd = d;
+            bj = j;
+        }
+    }
+    cluster_warp_min(bd, bj);
+    if (lane == 0) {
+        st.nn[i] = bj;
+        st.nnd[i] = bd;
+    }
+}
+
+template <int KIND>
+__device__ void cluster_segment(const ClusterArgs& a, unsigned s, double* D, ClusterSmem& st, ClusterShared& sh) {
+    const unsigned begin = (unsigned)a.offsets[s], n = (unsigned)(a.offsets[s + 1] - a.offsets[s]);
+    const unsigned tid = threadIdx.x, nt = blockDim.x, lane = tid & 31, warp = tid >> 5, n_warps = nt >> 5;
+    // distances, upper triangle, one warp per row: the operands and the inlined config_distance of pairwise_distance_kernel,
+    // so the same bits
+    for (unsigned p = warp; p < n; p += n_warps) {
+        const size_t ip = a.order ? a.order[begin + p] : begin + p;
+        const double* from = reinterpret_cast<const double*>(a.results + ip * a.rec_stride);
+        const bool from_contact = record_in_contact(a.results, a.rec_stride, a.cfg_stride, ip);
+        for (unsigned q = p + 1 + lane; q < n; q += 32) {
+            const size_t iq = a.order ? a.order[begin + q] : begin + q;
+            double d = config_distance<KIND>(*a.robot, from, reinterpret_cast<const double*>(a.results + iq * a.rec_stride));
+            if (isnan(d) || (a.separate_contact && record_in_contact(a.results, a.rec_stride, a.cfg_stride, iq) != from_contact)) d = INFINITY;
+            D[(size_t)p * n + q] = d;
+        }
+    }
+    for (unsigned p = tid; p < n; p += nt) st.rep[p] = p;
+    __syncthreads();
+    for (unsigned i = warp; i < n; i += n_warps) cluster_rescan_row(D, n, i, st);
+    __syncthreads();
+
+    unsigned merges = 0;
+    for (;;) {
+        // smallest (nnd[i], i)
+        double bd = INFINITY;
+        unsigned bi = n;
+        for (unsigned i = tid; i < n; i += nt) {
+            const double d = st.nnd[i];
+            if (d < bd) {
+                bd = d;
+                bi = i;
+            }
+        }
+        cluster_warp_min(bd, bi);
+        if (lane == 0) {
+            sh.wd[warp] = bd;
+            sh.wi[warp] = bi;
+        }
+        __syncthreads();
+        if (warp == 0) {
+            bd = lane < n_warps ? sh.wd[lane] : INFINITY;
+            bi = lane < n_warps ? sh.wi[lane] : n;
+            cluster_warp_min(bd, bi);
+            if (lane == 0) {
+                sh.go = bd < INFINITY && bd <= a.threshold;
+                sh.a = bi;
+                sh.b = sh.go ? st.nn[bi] : 0u;
+                sh.n_list = 0;
+            }
+        }
+        __syncthreads();
+        if (!sh.go) break;
+        const unsigned ca = sh.a, cb = sh.b;
+        merges++;
+        // row / column a <- op(a, b); b -> +inf; b's members join a
+        for (unsigned k = tid; k < n; k += nt) {
+            if (st.rep[k] == cb) st.rep[k] = ca;
+            if (k == ca) continue;
+            const size_t bk = k < cb ? (size_t)k * n + cb : (size_t)cb * n + k;
+            if (k == cb) {
+                D[(size_t)ca * n + cb] = INFINITY;
+                continue;
+            }
+            const size_t ak = k < ca ? (size_t)k * n + ca : (size_t)ca * n + k;
+            const double x = D[ak], y = D[bk];
+            D[ak] = a.complete ? fmax(x, y) : fmin(x, y);
+            D[bk] = INFINITY;
+        }
+        __syncthreads();
+        // cache repair (rows of merged-away positions are all +inf and stay out of the argmin through nnd = +inf)
+        for (unsigned i = tid; i < n; i += nt) {
+            if (i == cb) {
+                st.nnd[i] = INFINITY;
+                st.nn[i] = n;
+                continue;
+            }
+            if (st.rep[i] != i) continue;
+            const unsigned j = st.nn[i];
+            bool rescan = i == ca || j == cb;
+            if (i < ca && !rescan) {
+                if (j == ca) {
+                    rescan = true;
+                } else {
+                    const double d = D[(size_t)i * n + ca];
+                    if (cluster_key_less(d, ca, st.nnd[i], j)) {
+                        st.nnd[i] = d;
+                        st.nn[i] = ca;
+                    }
+                }
+            }
+            if (rescan) st.list[atomicAdd(&sh.n_list, 1u)] = i;
+        }
+        __syncthreads();
+        for (unsigned r = warp; r < sh.n_list; r += n_warps) cluster_rescan_row(D, n, st.list[r], st);
+        __syncthreads();
+    }
+
+    // dense ids in representative order: exclusive count of representatives below each position
+    if (tid == 0) sh.carry = 0;
+    __syncthreads();
+    for (unsigned base = 0; base < n; base += nt) {
+        const unsigned p = base + tid;
+        const bool is_rep = p < n && st.rep[p] == p;
+        const unsigned ballot = __ballot_sync(FKS_FULL, is_rep);
+        if (lane == 0) sh.wi[warp] = (unsigned)__popc(ballot);
+        __syncthreads();
+        unsigned before = sh.carry + (unsigned)__popc(ballot & ((1u << lane) - 1u));
+        for (unsigned w = 0; w < warp; w++) before += sh.wi[w];
+        if (p < n) st.nn[p] = before;
+        __syncthreads();
+        if (tid == 0)
+            for (unsigned w = 0; w < n_warps; w++) sh.carry += sh.wi[w];
+        __syncthreads();
+    }
+    for (unsigned p = tid; p < n; p += nt) a.labels[begin + p] = st.nn[st.rep[p]];
+    if (tid == 0) a.counts[s] = n - merges;
+    __syncthreads();  // the next segment reuses the shared state
+}
+
+// segments of at most kClusterSmallMax positions: D, then the per-position state, in dynamic shared memory
+template <int KIND>
+__global__ void __launch_bounds__(kClusterSmallBlock) cluster_small_kernel(ClusterArgs a) {
+    extern __shared__ __align__(16) unsigned char cluster_smem[];
+    __shared__ ClusterShared sh;
+    double* D = reinterpret_cast<double*>(cluster_smem);
+    const unsigned n_cap = a.n_cap;
+    ClusterSmem st;
+    st.nnd = D + (size_t)n_cap * n_cap;
+    st.rep = reinterpret_cast<unsigned*>(st.nnd + n_cap);
+    st.nn = st.rep + n_cap;
+    st.list = st.nn + n_cap;
+    for (unsigned t = blockIdx.x; t < a.n_segs; t += gridDim.x) cluster_segment<KIND>(a, a.segs[t], D, st, sh);
+}
+
+// larger segments: D in the CTA's slot of the global workspace, the per-position state in dynamic shared memory
+template <int KIND>
+__global__ void __launch_bounds__(kClusterLargeBlock) cluster_large_kernel(ClusterArgs a) {
+    extern __shared__ __align__(16) unsigned char cluster_smem[];
+    __shared__ ClusterShared sh;
+    const unsigned n_cap = a.n_cap;
+    double* D = a.work + (size_t)blockIdx.x * n_cap * n_cap;
+    ClusterSmem st;
+    st.nnd = reinterpret_cast<double*>(cluster_smem);
+    st.rep = reinterpret_cast<unsigned*>(st.nnd + n_cap);
+    st.nn = st.rep + n_cap;
+    st.list = st.nn + n_cap;
+    for (unsigned t = blockIdx.x; t < a.n_segs; t += gridDim.x) cluster_segment<KIND>(a, a.segs[t], D, st, sh);
+}
+
+// labels of segment s += the clusters of the segments before it (exclusive scan of the counts)
+__global__ void __launch_bounds__(256) cluster_relabel_kernel(const unsigned long long* offsets, unsigned n_segments, const unsigned* base,
+                                                              unsigned* labels) {
+    for (unsigned s = blockIdx.x; s < n_segments; s += gridDim.x) {
+        const unsigned add = base[s];
+        for (unsigned long long p = offsets[s] + threadIdx.x; p < offsets[s + 1]; p += blockDim.x) labels[p] += add;
+    }
+}
+
+size_t cluster_small_smem(unsigned n_cap) { return (size_t)n_cap * n_cap * 8 + cluster_state_bytes(n_cap); }
+
+template <typename Kernel>
+static int cluster_launch(Kernel k, const ClusterArgs& a, int block, size_t smem, int max_grid, void* stream) {
+    if (a.n_segs == 0) return 0;
+    cudaError_t err = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (err != cudaSuccess) return (int)err;
+    int per_sm = 0;
+    err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, block, smem);
+    if (err != cudaSuccess) return (int)err;
+    int dev = 0, sms = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    long long grid = (long long)(per_sm > 0 ? per_sm : 1) * sms;
+    if (grid > (long long)a.n_segs) grid = a.n_segs;
+    if (max_grid > 0 && grid > max_grid) grid = max_grid;
+    k<<<(unsigned)grid, block, smem, (cudaStream_t)stream>>>(a);
+    return (int)cudaGetLastError();
+}
+
+int launch_cluster(int kind, const ClusterLaunch& c, void* stream) {
+    ClusterArgs a;
+    a.robot = c.robot;
+    a.results = c.results;
+    a.rec_stride = c.rec_stride;
+    a.cfg_stride = c.cfg_stride;
+    a.complete = c.complete;
+    a.separate_contact = c.separate_contact;
+    a.threshold = c.threshold;
+    a.order = c.order;
+    a.offsets = c.offsets;
+    a.labels = c.labels;
+    a.counts = c.counts;
+    cudaStream_t st = (cudaStream_t)stream;
+    int rc = 0;
+    ClusterArgs sm = a, lg = a;
+    sm.segs = c.small_segs;
+    sm.n_segs = c.n_small;
+    sm.n_cap = c.small_cap;
+    sm.work = nullptr;
+    lg.segs = c.large_segs;
+    lg.n_segs = c.n_large;
+    lg.n_cap = c.large_cap;
+    lg.work = c.work;
+    const size_t small_smem = cluster_small_smem(c.small_cap), large_smem = cluster_state_bytes(c.large_cap);
+    switch (kind) {
+        case FKS_ROBOT_SE2:
+            if ((rc = cluster_launch(cluster_small_kernel<FKS_ROBOT_SE2>, sm, kClusterSmallBlock, small_smem, 0, stream)) != 0) return rc;
+            if ((rc = cluster_launch(cluster_large_kernel<FKS_ROBOT_SE2>, lg, kClusterLargeBlock, large_smem, c.large_slots, stream)) != 0) return rc;
+            break;
+        case FKS_ROBOT_SE3:
+            if ((rc = cluster_launch(cluster_small_kernel<FKS_ROBOT_SE3>, sm, kClusterSmallBlock, small_smem, 0, stream)) != 0) return rc;
+            if ((rc = cluster_launch(cluster_large_kernel<FKS_ROBOT_SE3>, lg, kClusterLargeBlock, large_smem, c.large_slots, stream)) != 0) return rc;
+            break;
+        case FKS_ROBOT_LINKED:
+            if ((rc = cluster_launch(cluster_small_kernel<FKS_ROBOT_LINKED>, sm, kClusterSmallBlock, small_smem, 0, stream)) != 0) return rc;
+            if ((rc = cluster_launch(cluster_large_kernel<FKS_ROBOT_LINKED>, lg, kClusterLargeBlock, large_smem, c.large_slots, stream)) != 0) return rc;
+            break;
+        default: return (int)cudaErrorInvalidValue;
+    }
+    // base of every segment's ids: partition's exclusive scan, in place over the counts (totals[1] = all clusters)
+    partition_scan_kernel<<<1, kPartitionBlock, 0, st>>>(c.counts, c.n_segments, 0, c.totals);
+    const unsigned relabel_grid = c.n_segments < 65535u ? c.n_segments : 65535u;
+    cluster_relabel_kernel<<<relabel_grid, 256, 0, st>>>(c.offsets, c.n_segments, c.counts, c.labels);
+    return (int)cudaGetLastError();
+}
+
 #ifdef FKS_PHASE_TIMERS
 __global__ void dbg_copy_kernel(unsigned long long* out) {
     if (threadIdx.x < 64) {

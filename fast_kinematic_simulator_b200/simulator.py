@@ -319,6 +319,20 @@ class GpuParticleContactSimulator:
         check(lib.fks_end_states_pairwise_distance(self._h, _dev_ptr(d_results), _dev_ptr(d_subset), int(m), _dev_ptr(d_out),
                                                    int(stream) if stream else None))
 
+    def end_states_cluster(self, d_results, segment_offsets, d_labels, max_cluster_distance, linkage=capi.LINKAGE_COMPLETE, d_order=None,
+                           separate_contact=False, stream=0):
+        """Flat single / complete-linkage clustering under max_cluster_distance inside every segment [offsets[s], offsets[s+1])
+        of the positions (record d_order[p], or p), on the device (fks_end_states_cluster).  d_labels (m x uint32 on the device)
+        receives global cluster ids, segment by segment in increasing order of each cluster's smallest position; returns the
+        clusters per segment (numpy uint64)."""
+        offsets = np.ascontiguousarray(segment_offsets, dtype=np.uint64)
+        n_segments = max(len(offsets) - 1, 0)
+        counts = np.zeros(max(n_segments, 1), np.uint64)
+        check(lib.fks_end_states_cluster(self._h, _dev_ptr(d_results), _dev_ptr(d_order), offsets.ctypes.data_as(C.POINTER(C.c_uint64)),
+                                         n_segments, int(linkage), float(max_cluster_distance), int(bool(separate_contact)),
+                                         _dev_ptr(d_labels), counts.ctypes.data_as(C.POINTER(C.c_uint64)), int(stream) if stream else None))
+        return counts[:n_segments]
+
     def trace_dtype(self):
         width = (lib.fks_sim_trace_stride(self._h) - 16) // 8
         return np.dtype([("kind", np.uint32), ("step", np.uint32), ("microstep", np.uint32), ("iteration", np.uint32),

@@ -458,6 +458,29 @@ int fks_end_states_partition(fks_sim* sim, const void* d_results, size_t n_parti
 int fks_end_states_pairwise_distance(fks_sim* sim, const void* d_results, const uint32_t* d_subset, size_t m, double* d_out,
                                      void* cuda_stream);
 
+/* fks_end_states_cluster: the grouping step itself -- flat agglomerative clustering under a distance cutoff, per segment.
+ * Positions 0 .. m-1 name records d_order[p] (d_order == NULL: record p); segment s covers positions
+ * [segment_offsets[s], segment_offsets[s+1]) of the HOST array segment_offsets (n_segments + 1 entries, [0] = 0,
+ * non-decreasing, last = m; empty segments are allowed).  Typical segments: {0, n_free, n} over the order of
+ * fks_end_states_partition, or one per leg of a sequence result (ids k * n + i from the base pointer).
+ *  - distance of positions p < q of one segment: d(p, q) = entry [p][q] of fks_end_states_pairwise_distance over the same ids
+ *    (same direction, same bits); +inf where that is NaN, and with separate_contact != 0 where the two records'
+ *    FKS_FLAG_DID_CONTACT differ;
+ *  - every segment starts from singletons; a cluster is named by its smallest position (its representative); the linkage of
+ *    clusters A, B is the minimum (FKS_LINKAGE_SINGLE) or maximum (FKS_LINKAGE_COMPLETE) of d over their pairs; while some
+ *    pair has a finite linkage <= max_cluster_distance, the pair with the smallest (linkage, smaller rep, larger rep) merges.
+ *    Clusters never cross segments and a pair at +inf never merges.  (scipy: linkage + fcluster(t, "distance") up to ties);
+ *  - d_labels[p] (device, m entries) = global cluster id: segment s's clusters are base_s .. base_s + cluster_counts[s] - 1
+ *    in increasing order of representative, base_s = the sum of the earlier segments' counts; cluster_counts is a HOST
+ *    array of n_segments entries.  The call returns after the stream has finished.
+ * Segments of up to 160 positions are clustered in shared memory, longer ones (up to 8192 positions) in a device workspace
+ * the simulator keeps.  FKS_ERR_INVALID_ARGUMENT: NaN max_cluster_distance, unknown linkage, null buffers when m > 0,
+ * malformed offsets, m >= 2^32, or a segment longer than 8192 positions.  m == 0 or n_segments == 0 launches nothing. */
+enum { FKS_LINKAGE_SINGLE = 0, FKS_LINKAGE_COMPLETE = 1 };
+int fks_end_states_cluster(fks_sim* sim, const void* d_results, const uint32_t* d_order, const uint64_t* segment_offsets,
+                           size_t n_segments, int linkage, double max_cluster_distance, int separate_contact, uint32_t* d_labels,
+                           uint64_t* cluster_counts, void* cuda_stream);
+
 /* -------------------------------------------------------------------------------------------
  * Test entry: the device's stacked-Jacobian solver (ComputeResolverCorrectionStepStackedJacobian, spcs.hpp:1990-1998 =
  * J.colPivHouseholderQr().solve(c)) on caller-provided systems, one warp each.  System i has rows[i] rows and `cols`
