@@ -614,6 +614,7 @@ int fks_sim_create(const fks_env* env, const fks_robot* robot, const fks_solver_
     int rc = 0;
     for (;; wpb = (wpb > 4) ? wpb - 4 : wpb - 1) {
         s->dyn_smem = simulate_smem_plan(&s->plan, h.L, h.J, h.D, h.P, robot->stride, wpb, s->smem_limit);
+        if (s->dyn_smem == 0) break;
         s->kinfo.max_blocks_per_sm = 0;
         rc = simulate_kernel_info(h.kind, s->dyn_smem, wpb, &s->kinfo);
         if ((rc == 0 && s->kinfo.max_blocks_per_sm >= 1) || wpb <= 1) break;
@@ -625,6 +626,7 @@ int fks_sim_create(const fks_env* env, const fks_robot* robot, const fks_solver_
     s->plan.trace_capacity = 0;
     s->plan.trace_width = 0;
     if (const char* ev = std::getenv("FKS_CULL")) s->plan.cull_mode = std::atoi(ev);  // developer knob
+    if (s->dyn_smem == 0) { delete s; return fail(FKS_ERR_UNSUPPORTED, "fks_sim_create: warp block layout not 16-byte aligned for bulk copies"); }
     if (rc != 0) { delete s; return cuda_fail((cudaError_t)rc, "fks_sim_create: kernel attributes"); }
     if (s->kinfo.max_blocks_per_sm < 1) { delete s; return fail(FKS_ERR_UNSUPPORTED, "fks_sim_create: robot does not fit one CTA's shared memory"); }
     cudaDeviceProp prop;

@@ -150,6 +150,7 @@ struct WarpLayout {
     int vars;     // WarpVars (kWarpVarsDoubles) + 2 * S doubles of PID state (inside [target, save2_end): parked with the context)
     int flags;    // 1 (u32 FKS_FLAG_* bits raised by any lane)
     int save2_end;  // a particle's context = [cfg, T + 2 L12) + [G, G + L12) + [target, save2_end): what has to survive between phases
+                    // (parked as whole 16-byte units: the third range also carries qr[0], which is dead between phases)
     int stats;    // FKS_NUM_STATS u64 counters of this WARP (not part of a context)
     int total;
     int noise_batch;
@@ -172,9 +173,10 @@ inline __host__ __device__ WarpLayout make_warp_layout(int L, int J, int D, int 
     // (D + 1) columns of ld doubles.  The solver's lane 4 g + i reads rows = i (mod 4) of column g: a leading dimension
     // = 4 (mod 16) puts the 16 lanes of a half warp on 16 different bank pairs; take it when it costs at most a quarter
     // of the rows
+    // Even in any case: columns are moved between shared and global memory as bulk copies, which start on 16 bytes
     auto pick_ld = [](int doubles, int columns) {
         const int cap = doubles / columns;
-        int ld = cap;
+        int ld = cap & ~1;
         const int pref = cap - ((cap - 4) & 15);
         if (cap >= 20 && pref >= 20 && pref * 4 >= cap * 3) ld = pref;
         return ld < 0 ? 0 : ld;
@@ -313,9 +315,13 @@ int launch_simulate(int kind, const LaunchArgs& args, int grid, size_t dyn_smem,
                     const void* l2_window_base, size_t l2_window_bytes);
 // bytes of one particle context in the global context store for this layout
 size_t context_bytes(const WarpLayout& wl);
-// bytes of CTA-level scheduling state behind the warp blocks in dynamic shared memory
+// bytes of CTA-level scheduling state behind the warp blocks in dynamic shared memory: a flag word (16), what every context
+// waits for (kMaxPool), which context each warp holds (kMaxPool), then one mbarrier per warp for its bulk loads
 constexpr size_t kSyncBytes = 16 + 2 * kMaxPool + 4 * kMaxPool;
-// fills args.wl / pts_off / warps_off / warps_per_block and returns the dynamic shared memory size
+constexpr size_t kSyncBarOff = 16 + 2 * kMaxPool;
+static_assert(kSyncBarOff % 8 == 0 && kSyncBarOff + 8 * kWarpsPerBlock <= kSyncBytes, "one mbarrier per warp in the sync area");
+// fills args.wl / pts_off / warps_off / warps_per_block and returns the dynamic shared memory size, or 0 when a range that the
+// kernel moves with bulk copies does not sit on 16-byte boundaries
 size_t simulate_smem_plan(LaunchArgs* args, int L, int J, int D, int P, int stride, int warps_per_block, size_t smem_limit);
 int launch_check_config(int kind, const LaunchArgs& args, int grid, size_t dyn_smem, void* stream, double inflation_ratio, unsigned char* out);
 int launch_qr_solve(double* work, const unsigned long long* offsets, const int* rows, int cols, int n, double* x_out, unsigned* flags_out,

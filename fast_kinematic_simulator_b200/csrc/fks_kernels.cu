@@ -68,6 +68,55 @@ __device__ __forceinline__ T wv_add(T* field, T inc) {
     *field = v;
     return v;
 }
+
+// ---- bulk copies (cp.async.bulk, 1-D TMA) between a warp's shared block and global memory -------------------------------
+// Lane 0 issues them with uniform operands; the bytes move in the async proxy and occupy no registers.  Addresses and sizes
+// are multiples of 16 bytes (simulate_smem_plan checks the layout).  The ordering rules they rely on, from the memory
+// consistency model of the PTX ISA:
+//  (a) Accesses of one location through the generic proxy (the lanes' loads and stores) and through the async proxy (bulk
+//      copies) are ordered only by a proxy fence.  Every lane that touched the shared data runs fence.proxy.async.shared::cta
+//      (and .global for global data it wrote), then __syncwarp orders those lanes before lane 0, which issues the bulk copy.
+//      A global slot last written by a bulk store of another warp is visible to lane 0's generic proxy after the barrier
+//      of simulate_kernel (rule (b)); lane 0 runs fence.proxy.async.global before its bulk load reads it.
+//  (b) cp.async.bulk.wait_group.read 0 returns once the sources of the issuing thread's bulk stores have been read; before
+//      that nothing may write that shared memory.  cp.async.bulk.wait_group 0 returns once the writes are complete; the
+//      implicit generic-async proxy fence that follows the completion of a bulk operation makes them visible to the issuer's
+//      generic proxy, and a barrier then carries them to the other threads.
+//  (c) A bulk load completes transactions on the warp's mbarrier.  A lane whose mbarrier.try_wait (.acquire, CTA scope)
+//      observes the phase complete sees the loaded bytes, so every lane that reads them waits itself (bulk_wait_loads).
+__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
+__device__ __forceinline__ void fence_async_shared() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+__device__ __forceinline__ void fence_async_global() { asm volatile("fence.proxy.async.global;" ::: "memory"); }
+__device__ __forceinline__ void bulk_store(double* g, const double* s, int doubles) {
+    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(g), "r"(smem_u32(s)), "r"(doubles * 8)
+                 : "memory");
+}
+__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
+__device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
+__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
+// the warp's mbarrier in the CTA's sync area
+__device__ __forceinline__ unsigned warp_bar() {
+    return smem_u32(smem_raw + frame().a.sync_off + kSyncBarOff) + 8u * (threadIdx.x >> 5);
+}
+// lane 0: arms the mbarrier for `bytes` of bulk loads; returns the token of the phase that they complete
+__device__ __forceinline__ unsigned long long bulk_expect(unsigned bar, int bytes) {
+    unsigned long long state;
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 %0, [%1], %2;" : "=l"(state) : "r"(bar), "r"(bytes) : "memory");
+    return state;
+}
+__device__ __forceinline__ void bulk_load(double* s, const double* g, int doubles, unsigned bar) {
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                 ::"r"(smem_u32(s)), "l"(g), "r"(doubles * 8), "r"(bar) : "memory");
+}
+// (c): every lane waits for the phase lane 0 armed (its token: no parity has to be carried from one load to the next)
+__device__ __forceinline__ void bulk_wait_loads(unsigned bar, unsigned long long state) {
+    state = __shfl_sync(FKS_FULL, state, 0);
+    unsigned done;
+    do {
+        asm volatile("{ .reg .pred p; mbarrier.try_wait.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
+                     : "=r"(done) : "r"(bar), "l"(state) : "memory");
+    } while (!done);
+}
 // global scratch slot of the particle context this warp has loaded (self-collision lists: written by the collision check of
 // a round, read by the collect of the following solve, which another warp may run)
 __device__ __forceinline__ char* context_scratch(int wb) {
@@ -1210,6 +1259,46 @@ __device__ __forceinline__ unsigned check_collision(int wb, int Xprev, int Xcur,
     return ((envc || has_self) ? 1u : 0u) | (has_self ? 2u : 0u);
 }
 
+// A collected system that outgrew the small shared-memory store (its rows < cap_s are there, the others in the warp's global
+// store): where it is factored.  In the larger shared-memory store (what a solve may overwrite once the corrections are
+// collected: world->voxel transforms, joint axes / origins, candidate list -- all rebuilt before they are read again) when
+// it fits, else in place in the global store, where every load of the in-place update is an L2 round trip.  Either way the
+// small store's rows first complete the global copy (the two shared stores overlap with different leading dimensions).
+// Every column moves as one bulk copy: leading dimensions are even, so columns start on 16 bytes.  Called at the end of
+// collect_corrections rather than from the main loop, which has no registers to spare.
+__device__ __forceinline__ void move_tall_system(int wb, int rows, int cols) {
+    const Frame& fr = frame();
+    const WarpLayout& wl = fr.a.wl;
+    const int lane = lane_id();
+    double* As = wsd(wb) + wl.jsm;
+    double* Ag = warp_jstore();
+    const int lds = wl.jsm_ld, cap_s = (wl.jsm_ld / 3) * 3, ldg = fr.a.sl.ldj, ldb = wl.jsm_big_ld;
+    // of an odd row count the lanes copy the last row: rounding the copies up would overwrite row cap_s of the global
+    // columns, which the collect wrote
+    const int nb = cap_s & ~1;
+    if (nb < cap_s && lane <= cols) Ag[(size_t)lane * ldg + nb] = As[lane * lds + nb];
+    fence_async_shared();  // (a): the collect's rows in both stores, and the row above
+    fence_async_global();
+    __syncwarp();
+    if (lane == 0) {
+        for (int c = 0; c <= cols; c++) bulk_store(Ag + (size_t)c * ldg, As + c * lds, nb);
+        bulk_commit();
+        bulk_wait_all();  // (b): complete, the global copy is read next
+    }
+    __syncwarp();
+    if (rows > ldb) return;
+    // an odd row count is rounded up by one row, which stays inside the column (ldb is even, ldg a multiple of 4, rows <= both)
+    const int n = (rows + 1) & ~1;
+    const unsigned bar = warp_bar();
+    unsigned long long state = 0ull;
+    if (lane == 0) {
+        fence_async_global();  // (a): the bulk stores above are visible to lane 0's generic proxy (b), the loads read them
+        state = bulk_expect(bar, (cols + 1) * n * 8);
+        for (int c = 0; c <= cols; c++) bulk_load(As + c * ldb, Ag + (size_t)c * ldg, n, bar);
+    }
+    bulk_wait_loads(bar, state);
+}
+
 // ------------------------------------------------------------------------------------------------
 // CollectPointCorrectionsAndJacobians (spcs:1818-1939): fills the stacked Jacobian (column major,
 // column D holds the corrections), rows in link-major point-minor order: the first rows into the warp's
@@ -1301,7 +1390,7 @@ __device__ __noinline__ int collect_corrections(int wb, int Xprev, int Xcur, boo
     __syncwarp();
     // Optimistic placement: rows go to the shared-memory store while they fit it (cap_s rows, a multiple of 3, so a point's
     // three rows never straddle) and to the global store beyond; most candidates turn out not to penetrate, so most systems
-    // end up entirely in shared memory.  The caller completes the global copy when the system outgrew the small store.
+    // end up entirely in shared memory.  A system that outgrew the small store is moved at the end (move_tall_system).
     double* As = ws + wl.jsm;
     const int lds = wl.jsm_ld, cap_s = (wl.jsm_ld / 3) * 3, ldg = fr.a.sl.ldj;
     // ---- pass 2 -----------------------------------------------------------------------------------
@@ -1412,40 +1501,8 @@ __device__ __noinline__ int collect_corrections(int wb, int Xprev, int Xcur, boo
         npts += __popc(mask);
     }
     __syncwarp();
+    if (3 * npts > cap_s) move_tall_system(wb, 3 * npts, D);
     return 3 * npts;
-}
-
-// A collected system that outgrew the small shared-memory store: complete its copy in the context's global store (the
-// rows < cap_s were written to shared memory).  It is factored in a later TALL cycle.
-__device__ __forceinline__ void spill_system(int wb, int cols) {
-    const Frame& fr = frame();
-    const WarpLayout& wl = fr.a.wl;
-    const int lane = lane_id();
-    const double* As = wsd(wb) + wl.jsm;
-    double* Ag = warp_jstore();
-    const int lds = wl.jsm_ld, cap_s = (wl.jsm_ld / 3) * 3, ldg = fr.a.sl.ldj;
-    for (int c = 0; c <= cols; c++)
-        for (int r = lane; r < cap_s; r += 32) Ag[(size_t)c * ldg + r] = As[c * lds + r];
-    __syncwarp();
-}
-// Where a spilled system is factored: in the larger shared-memory store (what a solve may overwrite once the corrections are
-// collected: world->voxel transforms, joint axes / origins, candidate list -- all rebuilt before they are read again) when
-// it fits, else in place in the global store, where every load of the in-place update is an L2 round trip.
-__device__ __forceinline__ void place_tall_system(int wb, int rows, int cols, double** store, int* store_ld) {
-    const Frame& fr = frame();
-    const WarpLayout& wl = fr.a.wl;
-    const int lane = lane_id();
-    double* As = wsd(wb) + wl.jsm;
-    double* Ag = warp_jstore();
-    const int ldg = fr.a.sl.ldj, ldb = wl.jsm_big_ld;
-    *store = Ag;
-    *store_ld = ldg;
-    if (rows > ldb) return;
-    for (int c = 0; c <= cols; c++)
-        for (int r = lane; r < rows; r += 32) As[c * ldb + r] = __ldcg(Ag + (size_t)c * ldg + r);
-    __syncwarp();
-    *store = As;
-    *store_ld = ldb;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1875,27 +1932,41 @@ enum { NEED_EMPTY = 0, NEED_ROUND = 1, NEED_SOLVE = 2, NEED_DEAD = 3 };  // what
 // changes the single-call kernel's code even where it is never taken.
 constexpr unsigned kLegPending = 0x80000000u;
 
-#ifndef FKS_COPY_UNROLL
-#define FKS_COPY_UNROLL 4
-#endif
-// a context's three ranges (fks_device_types.h) between the warp's shared block and its slot of the global context store
-__device__ __forceinline__ void context_copy(double* ws, double* g, const WarpLayout& wl, bool to_global) {
-    const int lane = lane_id();
-    const int n0 = wl.T + 2 * wl.L12 - wl.cfg, n1 = wl.L12, n2 = wl.save2_end - wl.target;
-    // (cache-global loads / stores: the slot is written and read by different warps of the CTA, the L1 is not coherent)
-    // Measured and NOT adopted (profiles/r2_kernel_experiments.md): explicit batches of 4 / 8 loads in flight, one fused
-    // park + load pass, a __noinline__ copy -- each made the whole kernel 3-13 % slower, free flight included: the extra
-    // live registers in this function cost more than the shorter copy wins.
-    if (to_global) {
-        for (int e = lane; e < n0; e += 32) __stcg(g + e, ws[wl.cfg + e]);
-        for (int e = lane; e < n1; e += 32) __stcg(g + n0 + e, ws[wl.G + e]);
-        for (int e = lane; e < n2; e += 32) __stcg(g + n0 + n1 + e, ws[wl.target + e]);
-    } else {
-        for (int e = lane; e < n0; e += 32) ws[wl.cfg + e] = __ldcg(g + e);
-        for (int e = lane; e < n1; e += 32) ws[wl.G + e] = __ldcg(g + n0 + e);
-        for (int e = lane; e < n2; e += 32) ws[wl.target + e] = __ldcg(g + n0 + n1 + e);
-    }
+// A context's three ranges (fks_device_types.h) between the warp's shared block and slots of the global context store, where
+// they lie back to back: parks the context in the block into the slot of context park_ctx, then loads context load_ctx
+// (-1: none).
+// Lane 0 issues three bulk copies per direction; the lanes wait for the load only.  The park's writes are waited for at the
+// end of the cycle (simulate_kernel): the next cycle's __syncthreads is where another warp may start to load that slot.
+// (A per-lane copy kept the loads in registers: batches of loads in flight made the whole kernel slower through spills of
+// the main loop, profiles/r2_kernel_experiments.md; the bulk copy holds nothing.)
+__device__ __forceinline__ void context_swap(double* ws, int park_ctx, int load_ctx, const WarpLayout& wl) {
+    const LaunchArgs& a = frame().a;
+    char* store = a.ctx_store + (size_t)blockIdx.x * a.pool * a.ctx_stride;  // the CTA's slots
+    double* park = reinterpret_cast<double*>(store + (size_t)park_ctx * a.ctx_stride);
+    const double* load = reinterpret_cast<const double*>(store + (size_t)load_ctx * a.ctx_stride);
+    const int n0 = wl.T + 2 * wl.L12 - wl.cfg, n1 = wl.L12, n2 = (wl.save2_end - wl.target + 1) & ~1;
+    const unsigned bar = warp_bar();
+    fence_async_shared();  // (a): every lane wrote the block (WarpVars included)
     __syncwarp();
+    unsigned long long state = 0ull;
+    if (lane_id() == 0) {
+        if (park_ctx >= 0) {
+            bulk_store(park, ws + wl.cfg, n0);
+            bulk_store(park + n0, ws + wl.G, n1);
+            bulk_store(park + n0 + n1, ws + wl.target, n2);
+            bulk_commit();
+            bulk_wait_read();  // (b): the load and a fresh context's set-up overwrite what the park reads
+        }
+        if (load_ctx >= 0) {
+            fence_async_global();  // (a): the slot was last written by a park of some warp
+            state = bulk_expect(bar, (n0 + n1 + n2) * 8);
+            bulk_load(ws + wl.cfg, load, n0, bar);
+            bulk_load(ws + wl.G, load + n0, n1, bar);
+            bulk_load(ws + wl.target, load + n0 + n1, n2, bar);
+        }
+    }
+    __syncwarp();  // (b) for the other lanes
+    if (load_ctx >= 0) bulk_wait_loads(bar, state);
 }
 }  // namespace
 
@@ -1964,7 +2035,6 @@ __global__ void __launch_bounds__(kThreadsPerBlock, FKS_MIN_BLOCKS) simulate_ker
     unsigned char* need = smem_raw + a.sync_off + 16;                     // [pool] NEED_*
     signed char* holds = reinterpret_cast<signed char*>(need + kMaxPool); // [warps] the context in the warp's block, -1: none
     volatile unsigned* exhausted = reinterpret_cast<volatile unsigned*>(smem_raw + a.sync_off);  // no particles left to admit
-    char* store = a.ctx_store + (size_t)blockIdx.x * pool * a.ctx_stride;
     for (int c = threadIdx.x; c < kMaxPool; c += blockDim.x) {
         need[c] = c < n_warps ? NEED_ROUND : (c < pool ? NEED_EMPTY : NEED_DEAD);  // context w starts out in warp w, about to fetch
         holds[c] = c < n_warps ? (signed char)c : (signed char)-1;
@@ -1980,6 +2050,9 @@ __global__ void __launch_bounds__(kThreadsPerBlock, FKS_MIN_BLOCKS) simulate_ker
         wv->m_result = 0.0;
         wv->ctx = warp;
         if (SEQ) wv->leg = 0u;
+        // the warp's mbarrier of its bulk loads (context_swap, move_tall_system): one arrival per phase, lane 0's
+        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(warp_bar()) : "memory");
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     __syncwarp();
 
@@ -2061,8 +2134,9 @@ __global__ void __launch_bounds__(kThreadsPerBlock, FKS_MIN_BLOCKS) simulate_ker
                 }
             }
             if (got >= 0) {
-                // the context in the block (if any) is not needed in this phase: it waits in the global store
-                if (my >= 0) context_copy(ws, reinterpret_cast<double*>(store + (size_t)my * a.ctx_stride), wl, true);
+                // the context in the block (if any) is not needed in this phase: it waits in the global store; the assigned
+                // one comes in unless it is fresh
+                context_swap(ws, my, fresh ? -1 : got, wl);
                 if (fresh) {
                     // a fresh context: its first round fetches a particle
                     if (lane == 0) {
@@ -2077,10 +2151,7 @@ __global__ void __launch_bounds__(kThreadsPerBlock, FKS_MIN_BLOCKS) simulate_ker
                         if (SEQ) wv->leg = 0u;
                     }
                     __syncwarp();
-                } else {
-                    context_copy(ws, reinterpret_cast<double*>(store + (size_t)got * a.ctx_stride), wl, false);
                 }
-                if (lane == 0) holds[warp] = (signed char)got;
                 active = true;
             }
         }
@@ -2439,13 +2510,17 @@ __global__ void __launch_bounds__(kThreadsPerBlock, FKS_MIN_BLOCKS) simulate_ker
             const long long tc0 = clock64();
             textra[1] += 1;
 #endif
-            double* jstore = ws + wl.jsm;
-            int jld = wl.jsm_ld;
             rows = collect_corrections<KIND>(wb, prev, cur, (cc & 2u) != 0u);
             if (lane == 0) add_stat(wb, FKS_STAT_TOTAL_CORRECTED_POINTS, (unsigned long long)(rows / 3));
-            if (rows > (wl.jsm_ld / 3) * 3) {  // too tall for the small store: the bigger one, or the warp's global slot
-                spill_system(wb, D);
-                place_tall_system(wb, rows, D, &jstore, &jld);
+            // where collect_corrections left the system: the small store, the bigger one, or the warp's global slot
+            double* jstore = ws + wl.jsm;
+            int jld = wl.jsm_ld;
+            if (rows > (wl.jsm_ld / 3) * 3) {
+                jld = wl.jsm_big_ld;
+                if (rows > jld) {
+                    jstore = warp_jstore();
+                    jld = a.sl.ldj;
+                }
             }
 #ifdef FKS_PHASE_TIMERS
             tacc[10] += clock64() - tc0;
@@ -2500,8 +2575,13 @@ __global__ void __launch_bounds__(kThreadsPerBlock, FKS_MIN_BLOCKS) simulate_ker
             wv->want_solve = want_solve ? 1 : 0;
             wv->cc = cc;
             wv->m_result = m_result;
+            // (written here, not when the context was taken over: other warps may still be reading the census)
+            holds[warp] = (signed char)ctx;
             need[ctx] = want_solve ? NEED_SOLVE : (after == AF_DONE ? NEED_DEAD : NEED_ROUND);
             if (after == AF_DONE) *exhausted = 1u;
+            // (b) of the bulk copies: a park of this cycle is complete before the next __syncthreads, after which any warp
+            // may load that slot (only a warp that runs a context parks one; none is outstanding when the CTA exits)
+            bulk_wait_all();
         }
         __syncwarp();
         }  // active
@@ -2753,7 +2833,14 @@ size_t simulate_smem_plan(LaunchArgs* args, int L, int J, int D, int P, int stri
     size_t off = warps_off + (size_t)warps_per_block * args->wl.total * 8;
     args->sync_off = (int)off;  // CTA-level scheduling state (context pool)
     off += kSyncBytes;
-    return off;
+    // Bulk copies (context_swap, move_tall_system) move whole 16-byte units between 16-byte boundaries: every
+    // warp block, range start and length, and store column they move has to sit on an even double.  0: it does not
+    const WarpLayout& w = args->wl;
+    const int ranges[] = {w.total, w.cfg, w.T + 2 * w.L12 - w.cfg, w.G, w.L12, w.target, w.jsm, w.jsm_ld, w.jsm_big_ld,
+                          args->sl.ldj};
+    bool aligned = warps_off % 16 == 0 && (w.save2_end + 1) / 2 * 2 <= w.total;
+    for (int v : ranges) aligned = aligned && v % 2 == 0;
+    return aligned ? off : 0;
 }
 
 template <int KIND>
@@ -2770,7 +2857,11 @@ static const void* kernel_ptr(int kind, bool trace = false, bool seq = false) {
     return nullptr;
 }
 
-size_t context_bytes(const WarpLayout& wl) { return (size_t)((wl.T + 2 * wl.L12 - wl.cfg) + wl.L12 + (wl.save2_end - wl.target)) * 8; }
+// (the third range rounded up to whole 16-byte units as context_swap moves it; slots on 128-byte boundaries)
+size_t context_bytes(const WarpLayout& wl) {
+    const size_t bytes = (size_t)((wl.T + 2 * wl.L12 - wl.cfg) + wl.L12 + ((wl.save2_end - wl.target + 1) & ~1)) * 8;
+    return (bytes + 127) & ~(size_t)127;
+}
 
 int simulate_kernel_info(int kind, size_t dyn_smem, int warps_per_block, KernelInfo* out) {
     const void* fn = kernel_ptr(kind);
