@@ -76,6 +76,8 @@ EXPORTS = (
     "fks_end_states_partition",
     "fks_end_states_pairwise_distance",
     "fks_end_states_cluster",
+    "fks_end_states_groups",
+    "fks_end_states_gather_starts",
     "fks_debug_qr_solve",
     "fks_measure_fp64_peak",
     "fks_measure_gather_rate",
@@ -155,6 +157,10 @@ lib.fks_end_states_partition.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c
 lib.fks_end_states_pairwise_distance.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]
 lib.fks_end_states_cluster.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, P(C.c_uint64), C.c_size_t, C.c_int, C.c_double, C.c_int,
                                        C.c_void_p, P(C.c_uint64), C.c_void_p]
+lib.fks_end_states_groups.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p,
+                                      C.c_void_p, C.c_void_p, P(C.c_uint64), C.c_void_p]
+lib.fks_end_states_gather_starts.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, P(C.c_uint32), C.c_size_t,
+                                             C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
 lib.fks_debug_qr_solve.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_size_t, C.c_void_p, C.c_void_p]
 lib.fks_measure_fp64_peak.argtypes = [C.c_int, P(C.c_double)]
 lib.fks_measure_gather_rate.argtypes = [C.c_int, C.c_size_t, P(C.c_double)]

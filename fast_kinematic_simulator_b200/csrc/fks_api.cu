@@ -123,6 +123,14 @@ struct fks_sim {
     size_t cap_clu = 0;
     double* d_clu_mat = nullptr;
     size_t cap_clu_mat = 0;
+    // fks_end_states_groups: [totals (2) | row maxima (m doubles) | cursors, state as u32]
+    unsigned long long* d_grp = nullptr;
+    size_t cap_grp = 0;
+    // fks_end_states_gather_starts: the selected group ids, and when the last launch that reads them is done
+    unsigned* d_sel = nullptr;
+    size_t cap_sel = 0;
+    cudaEvent_t sel_read = nullptr;
+    bool has_sel = false;
     unsigned long long* d_trace_buf = nullptr;  // fks_forward_simulate_traced: [counter word | records], grown on demand
     size_t cap_trace_buf = 0;
     size_t smem_limit;
@@ -684,6 +692,10 @@ void fks_sim_destroy(fks_sim* s) {
     cudaFree(s->d_part);
     cudaFree(s->d_clu);
     cudaFree(s->d_clu_mat);
+    if (s->has_sel) cudaEventSynchronize(s->sel_read);
+    cudaFree(s->d_grp);
+    cudaFree(s->d_sel);
+    if (s->sel_read) cudaEventDestroy(s->sel_read);
     cudaFree(s->d_ctx_store);
     cudaFree(s->d_results);
     if (s->last_done) cudaEventDestroy(s->last_done);
@@ -1190,6 +1202,91 @@ int fks_end_states_cluster(fks_sim* s, const void* d_results, const uint32_t* d_
     FKS_CUDA(cudaMemcpyAsync(&total, c.totals + 1, sizeof(total), cudaMemcpyDeviceToHost, stream));
     FKS_CUDA(cudaStreamSynchronize(stream));
     for (size_t i = 0; i < n_segments; i++) cluster_counts[i] = (i + 1 < n_segments ? base[i + 1] : total) - base[i];
+    return FKS_OK;
+}
+
+int fks_end_states_groups(fks_sim* s, const void* d_results, const uint32_t* d_order, size_t m, const uint32_t* d_labels, size_t n_clusters,
+                          uint32_t* d_group_offsets, uint32_t* d_members, uint32_t* d_representatives, double* d_radius,
+                          uint64_t* group_sizes, void* cuda_stream) {
+    if (!s) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_groups: null simulator");
+    if (m > 0xffffffffull) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_groups: 2^32 or more positions");
+    if (n_clusters > m) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_groups: more clusters than positions");
+    if (m == 0) return FKS_OK;
+    if (!d_results || !d_labels || !d_group_offsets || !d_members || !d_representatives || !d_radius || !group_sizes)
+        return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_groups: null buffer");
+    if (n_clusters == 0) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_groups: a label is not below n_clusters");
+    NvtxRange range("fks_end_states_groups");
+    DeviceGuard guard(s->device);
+    if (!guard.ok) return fail(FKS_ERR_CUDA, "fks_end_states_groups: cudaSetDevice failed");
+    cudaStream_t stream = (cudaStream_t)cuda_stream;
+    const size_t n_state = 2 + m / (kGroupSmallMax + 1) + 1;
+    int rc;
+    if ((rc = ensure(&s->d_grp, &s->cap_grp, 2 + m + (n_clusters + n_state + 1) / 2)) != FKS_OK) return rc;
+    GroupsLaunch g;
+    g.robot = s->robot->d_robot;
+    g.results = (const char*)d_results;
+    g.rec_stride = fks_sim_result_stride(s);
+    g.cfg_stride = s->robot->stride;
+    g.order = d_order;
+    g.labels = d_labels;
+    g.m = (unsigned)m;
+    g.n_clusters = (unsigned)n_clusters;
+    g.offsets = d_group_offsets;
+    g.members = d_members;
+    g.reps = d_representatives;
+    g.radius = d_radius;
+    g.totals = s->d_grp;
+    g.row_max = reinterpret_cast<double*>(s->d_grp + 2);
+    g.cursor = reinterpret_cast<unsigned*>(s->d_grp + 2 + m);
+    g.state = g.cursor + n_clusters;
+    FKS_CUDA(cudaMemsetAsync(d_group_offsets, 0, n_clusters * sizeof(uint32_t), stream));
+    FKS_CUDA(cudaMemsetAsync(g.cursor, 0, (n_clusters + 2) * sizeof(uint32_t), stream));
+    rc = launch_groups(s->robot->host.kind, g, stream);
+    if (rc != 0) return cuda_fail((cudaError_t)rc, "fks_end_states_groups: launch");
+    s->launches += kGroupLaunches;
+    std::vector<uint32_t> offsets(n_clusters + 1);
+    uint32_t err = 0;
+    FKS_CUDA(cudaMemcpyAsync(offsets.data(), d_group_offsets, offsets.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+    FKS_CUDA(cudaMemcpyAsync(&err, g.state + 1, sizeof(err), cudaMemcpyDeviceToHost, stream));
+    FKS_CUDA(cudaStreamSynchronize(stream));
+    if (err & kGroupErrLabel) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_groups: a label is not below n_clusters");
+    if (err & kGroupErrEmpty) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_groups: a cluster has no member");
+    if (err & kGroupErrLarge)
+        return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_groups: a cluster has more than " + std::to_string(kClusterMaxSegment) + " members");
+    for (size_t c = 0; c < n_clusters; c++) group_sizes[c] = offsets[c + 1] - offsets[c];
+    return FKS_OK;
+}
+
+int fks_end_states_gather_starts(fks_sim* s, const void* d_results, const uint32_t* d_group_offsets, const uint32_t* d_members,
+                                 size_t n_clusters, const uint32_t* selected, size_t n_selected, size_t per_group,
+                                 const double* d_group_targets, double* d_starts, double* d_targets, void* cuda_stream) {
+    if (!s) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_gather_starts: null simulator");
+    if (per_group == 0) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_gather_starts: per_group is 0");
+    if ((d_targets == nullptr) != (d_group_targets == nullptr))
+        return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_gather_starts: d_targets and d_group_targets go together");
+    if (n_selected == 0) return FKS_OK;
+    if (n_selected > 0xffffffffull / per_group) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_gather_starts: 2^32 or more starts");
+    if (!d_results || !d_group_offsets || !d_members || !selected || !d_starts)
+        return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_gather_starts: null buffer");
+    for (size_t i = 0; i < n_selected; i++)
+        if (selected[i] >= n_clusters) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_gather_starts: a selected group is not below n_clusters");
+    NvtxRange range("fks_end_states_gather_starts");
+    DeviceGuard guard(s->device);
+    if (!guard.ok) return fail(FKS_ERR_CUDA, "fks_end_states_gather_starts: cudaSetDevice failed");
+    cudaStream_t stream = (cudaStream_t)cuda_stream;
+    if (!s->sel_read) FKS_CUDA(cudaEventCreateWithFlags(&s->sel_read, cudaEventDisableTiming));
+    // the ids go through one buffer: a launch of an earlier call, perhaps on another stream, must have read it first
+    if (s->has_sel && n_selected > s->cap_sel) FKS_CUDA(cudaEventSynchronize(s->sel_read));
+    int rc;
+    if ((rc = ensure(&s->d_sel, &s->cap_sel, n_selected)) != FKS_OK) return rc;
+    if (s->has_sel) FKS_CUDA(cudaStreamWaitEvent(stream, s->sel_read, 0));
+    FKS_CUDA(cudaMemcpyAsync(s->d_sel, selected, n_selected * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
+    rc = launch_gather_starts((const char*)d_results, fks_sim_result_stride(s), s->robot->stride, d_group_offsets, d_members, s->d_sel,
+                              (unsigned)n_selected, (unsigned)per_group, d_group_targets, d_starts, d_targets, stream);
+    if (rc != 0) return cuda_fail((cudaError_t)rc, "fks_end_states_gather_starts: launch");
+    s->launches += 1;
+    FKS_CUDA(cudaEventRecord(s->sel_read, stream));
+    s->has_sel = true;
     return FKS_OK;
 }
 

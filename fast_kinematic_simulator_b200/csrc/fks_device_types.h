@@ -357,6 +357,35 @@ struct ClusterLaunch {
 };
 // the launches of one call: the two clustering kernels (those with segments), the scan of the counts and the relabel pass
 int launch_cluster(int kind, const ClusterLaunch& c, void* stream);
+// fks_end_states_groups: clusters of up to kGroupSmallMax members get their minimax representative from one CTA each, larger
+// ones (up to kClusterMaxSegment, the largest cluster fks_end_states_cluster makes) from row chunks spread over the grid.
+constexpr unsigned kGroupSmallMax = 256;
+constexpr unsigned kGroupErrLabel = 1, kGroupErrEmpty = 2, kGroupErrLarge = 4;  // bits of GroupsLaunch::state[1]
+struct GroupsLaunch {
+    const DevRobot* robot;
+    const char* results;
+    size_t rec_stride;
+    int cfg_stride;
+    const unsigned* order;          // device, or null
+    const unsigned* labels;         // device [m]
+    unsigned m, n_clusters;
+    unsigned* offsets;              // device [n_clusters + 1] (the caller's)
+    unsigned* members;              // device [m] (the caller's)
+    unsigned* reps;                 // device [n_clusters]
+    double* radius;                 // device [n_clusters]
+    unsigned long long* totals;     // workspace [2]
+    double* row_max;                // workspace [m]: r of every member of a large cluster, by slot
+    unsigned* cursor;               // workspace [n_clusters], zeroed
+    unsigned* state;                // workspace [2 + m / (kGroupSmallMax + 1) + 1], zeroed: large clusters, error bits, their list
+};
+// the launches of one call, whatever the number and sizes of the clusters: count, scan, scatter, sort + small search,
+// large rows, large argmin
+constexpr int kGroupLaunches = 6;
+int launch_groups(int kind, const GroupsLaunch& g, void* stream);
+// fks_end_states_gather_starts: one launch
+int launch_gather_starts(const char* results, size_t rec_stride, int cfg_stride, const unsigned* offsets, const unsigned* members,
+                         const unsigned* selected, unsigned n_selected, unsigned per_group, const double* group_targets, double* starts,
+                         double* targets, void* stream);
 int launch_dbg_copy(unsigned long long* out, void* stream);  // developer counters of the FKS_PHASE_TIMERS build
 int launch_fp64_peak(double* out, int grid, int iters, void* stream);
 int launch_gather(const float* data, unsigned long long n_mask, float* out, int grid, int iters, void* stream);

@@ -3371,6 +3371,240 @@ int launch_cluster(int kind, const ClusterLaunch& c, void* stream) {
     return (int)cudaGetLastError();
 }
 
+// ---------------------------------------------------------------------------------------------
+// fks_end_states_groups: the clusters of a labelled position range as particle groups.  Members: a stable counting sort by
+// label -- count, the partition's one-block scan, a scatter in arrival order, then each group sorted by position in shared
+// memory, so the result does not depend on the order of the scatter's atomics.  Representative: the member with the smallest
+// (r, position), r(p) = max over the other members q of d(min(p,q), max(p,q)), d = the pairwise kernel's entry (same
+// inlined config_distance, same operands), NaN as +inf.  Every pair is evaluated in both rows, so a row's maximum is a plain
+// warp reduction; max over non-NaN values and the (r, position) argmin are exact in any order, so every result is.
+// ---------------------------------------------------------------------------------------------
+constexpr int kGroupBlock = 256;
+constexpr unsigned kGroupWarps = kGroupBlock / 32;
+constexpr unsigned kGroupRowsPerTask = 32;  // rows of a large cluster per task of the row pass
+
+// pass 1: members per label into offsets[0 .. n_clusters) (zeroed), error bit for labels out of range
+__global__ void __launch_bounds__(kGroupBlock) groups_count_kernel(const unsigned* labels, unsigned m, unsigned n_clusters, unsigned* counts,
+                                                                   unsigned* state) {
+    for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < m; p += (size_t)gridDim.x * blockDim.x) {
+        const unsigned l = labels[p];
+        if (l < n_clusters) atomicAdd(&counts[l], 1u);
+        else atomicOr(&state[1], kGroupErrLabel);
+    }
+}
+
+// pass 3 (after the scan): positions into their group's range in arrival order; offsets[n_clusters] = positions with a valid label
+__global__ void __launch_bounds__(kGroupBlock) groups_scatter_kernel(const unsigned* labels, unsigned m, unsigned n_clusters, unsigned* offsets,
+                                                                     const unsigned long long* totals, unsigned* cursor, unsigned* members) {
+    if (blockIdx.x == 0 && threadIdx.x == 0) offsets[n_clusters] = (unsigned)totals[1];
+    for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < m; p += (size_t)gridDim.x * blockDim.x) {
+        const unsigned l = labels[p];
+        if (l < n_clusters) members[offsets[l] + atomicAdd(&cursor[l], 1u)] = (unsigned)p;
+    }
+}
+
+// one warp: r of member i of a group whose record ids are ids[0 .. k), in position order (every lane gets it)
+template <int KIND>
+__device__ __forceinline__ double group_row_max(const GroupsLaunch& g, const unsigned* ids, unsigned k, unsigned i) {
+    const unsigned lane = threadIdx.x & 31;
+    const double* rec_i = reinterpret_cast<const double*>(g.results + (size_t)ids[i] * g.rec_stride);
+    double r = -INFINITY;
+    for (unsigned j = lane; j < k; j += 32) {
+        if (j == i) continue;
+        const double* rec_j = reinterpret_cast<const double*>(g.results + (size_t)ids[j] * g.rec_stride);
+        double d = config_distance<KIND>(*g.robot, j > i ? rec_i : rec_j, j > i ? rec_j : rec_i);
+        if (isnan(d)) d = INFINITY;
+        if (d > r) r = d;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const double x = __shfl_xor_sync(FKS_FULL, r, o);
+        if (x > r) r = x;
+    }
+    return k == 1 ? 0.0 : r;
+}
+
+// the CTA's smallest (d, i) over its warps' (lane-uniform) candidates, in thread 0
+__device__ __forceinline__ void group_block_min(double& d, unsigned& i, double* wd, unsigned* wi) {
+    const unsigned lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (lane == 0) {
+        wd[warp] = d;
+        wi[warp] = i;
+    }
+    __syncthreads();
+    if (warp == 0) {
+        d = lane < kGroupWarps ? wd[lane] : INFINITY;
+        i = lane < kGroupWarps ? wi[lane] : 0xffffffffu;
+        cluster_warp_min(d, i);
+    }
+}
+
+// pass 4, one CTA per group: check its size, sort its positions (bitonic, padded to a power of two), write its record ids;
+// groups of up to kGroupSmallMax members get their representative here, larger ones go on the list of the row pass
+template <int KIND>
+__global__ void __launch_bounds__(kGroupBlock) groups_sort_small_kernel(GroupsLaunch g) {
+    __shared__ unsigned key[kClusterMaxSegment];
+    __shared__ double wd[kGroupWarps];
+    __shared__ unsigned wi[kGroupWarps];
+    const unsigned tid = threadIdx.x, warp = tid >> 5;
+    for (unsigned c = blockIdx.x; c < g.n_clusters; c += gridDim.x) {
+        const unsigned begin = g.offsets[c], k = g.offsets[c + 1] - begin;
+        if (k == 0 || k > kClusterMaxSegment) {
+            if (tid == 0) atomicOr(&g.state[1], k == 0 ? kGroupErrEmpty : kGroupErrLarge);
+            continue;
+        }
+        unsigned n2 = 1;
+        while (n2 < k) n2 <<= 1;
+        for (unsigned i = tid; i < n2; i += kGroupBlock) key[i] = i < k ? g.members[begin + i] : 0xffffffffu;
+        __syncthreads();
+        for (unsigned size = 2; size <= n2; size <<= 1) {
+            for (unsigned stride = size >> 1; stride > 0; stride >>= 1) {
+                for (unsigned t = tid; t < n2 / 2; t += kGroupBlock) {
+                    const unsigned i = 2 * stride * (t / stride) + t % stride, j = i + stride;
+                    const unsigned x = key[i], y = key[j];
+                    if ((x > y) == ((i & size) == 0)) {
+                        key[i] = y;
+                        key[j] = x;
+                    }
+                }
+                __syncthreads();
+            }
+        }
+        for (unsigned i = tid; i < k; i += kGroupBlock) {
+            const unsigned id = g.order ? g.order[key[i]] : key[i];
+            key[i] = id;
+            g.members[begin + i] = id;
+        }
+        __syncthreads();
+        if (k > kGroupSmallMax) {
+            if (tid == 0) g.state[2 + atomicAdd(&g.state[0], 1u)] = c;
+            continue;
+        }
+        double bd = INFINITY;
+        unsigned bi = k;
+        for (unsigned i = warp; i < k; i += kGroupWarps) {
+            const double r = group_row_max<KIND>(g, key, k, i);
+            if (cluster_key_less(r, i, bd, bi)) {
+                bd = r;
+                bi = i;
+            }
+        }
+        group_block_min(bd, bi, wd, wi);
+        if (tid == 0) {
+            g.reps[c] = key[bi];
+            g.radius[c] = bd;
+        }
+        __syncthreads();  // the next group reuses key, wd, wi
+    }
+}
+
+// pass 5: r of every member of the listed groups.  Group e's rows form tasks of kGroupRowsPerTask rows, numbered on from the
+// tasks of the groups before it; task T goes to CTA T mod gridDim.x.
+template <int KIND>
+__global__ void __launch_bounds__(kGroupBlock) groups_large_rows_kernel(GroupsLaunch g) {
+    const unsigned n_large = g.state[0], warp = threadIdx.x >> 5, lane = threadIdx.x & 31, G = gridDim.x;
+    unsigned shift = 0;  // (tasks of the groups before e) mod G
+    for (unsigned e = 0; e < n_large; e++) {
+        const unsigned c = g.state[2 + e], begin = g.offsets[c], k = g.offsets[c + 1] - begin;
+        const unsigned n_tasks = (k + kGroupRowsPerTask - 1) / kGroupRowsPerTask;
+        for (unsigned t = (blockIdx.x + G - shift) % G; t < n_tasks; t += G) {
+            const unsigned end = min(k, (t + 1) * kGroupRowsPerTask);
+            for (unsigned i = t * kGroupRowsPerTask + warp; i < end; i += kGroupWarps) {
+                const double r = group_row_max<KIND>(g, g.members + begin, k, i);
+                if (lane == 0) g.row_max[begin + i] = r;
+            }
+        }
+        shift = (shift + n_tasks) % G;
+    }
+}
+
+// pass 6: one CTA per listed group, the smallest (r, position)
+__global__ void __launch_bounds__(kGroupBlock) groups_large_argmin_kernel(GroupsLaunch g) {
+    __shared__ double wd[kGroupWarps];
+    __shared__ unsigned wi[kGroupWarps];
+    const unsigned n_large = g.state[0];
+    for (unsigned e = blockIdx.x; e < n_large; e += gridDim.x) {
+        const unsigned c = g.state[2 + e], begin = g.offsets[c], k = g.offsets[c + 1] - begin;
+        double bd = INFINITY;
+        unsigned bi = k;
+        for (unsigned i = threadIdx.x; i < k; i += kGroupBlock) {
+            const double r = g.row_max[begin + i];
+            if (cluster_key_less(r, i, bd, bi)) {
+                bd = r;
+                bi = i;
+            }
+        }
+        cluster_warp_min(bd, bi);
+        group_block_min(bd, bi, wd, wi);
+        if (threadIdx.x == 0) {
+            g.reps[c] = g.members[begin + bi];
+            g.radius[c] = bd;
+        }
+        __syncthreads();
+    }
+}
+
+template <typename Kernel>
+static unsigned groups_resident_ctas(Kernel k) {
+    int per_sm = 0, dev = 0, sms = 0;
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, kGroupBlock, 0);
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    return (unsigned)((per_sm > 0 ? per_sm : 1) * (sms > 0 ? sms : 1));
+}
+
+template <int KIND>
+static void groups_search(const GroupsLaunch& g, cudaStream_t st) {
+    // the host does not know how many groups are large: the row and argmin passes run a full grid and read the list
+    const unsigned resident = groups_resident_ctas(groups_sort_small_kernel<KIND>);
+    const unsigned rows_grid = groups_resident_ctas(groups_large_rows_kernel<KIND>);
+    groups_sort_small_kernel<KIND><<<g.n_clusters < resident ? g.n_clusters : resident, kGroupBlock, 0, st>>>(g);
+    groups_large_rows_kernel<KIND><<<rows_grid, kGroupBlock, 0, st>>>(g);
+    groups_large_argmin_kernel<<<rows_grid, kGroupBlock, 0, st>>>(g);
+}
+
+int launch_groups(int kind, const GroupsLaunch& g, void* stream) {
+    if (g.m == 0 || g.n_clusters == 0) return (int)cudaErrorInvalidValue;
+    void (*search)(const GroupsLaunch&, cudaStream_t);
+    switch (kind) {
+        case FKS_ROBOT_SE2: search = groups_search<FKS_ROBOT_SE2>; break;
+        case FKS_ROBOT_SE3: search = groups_search<FKS_ROBOT_SE3>; break;
+        case FKS_ROBOT_LINKED: search = groups_search<FKS_ROBOT_LINKED>; break;
+        default: return (int)cudaErrorInvalidValue;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t blocks = ((size_t)g.m + kGroupBlock - 1) / kGroupBlock;
+    const unsigned grid = blocks < 65535 ? (unsigned)blocks : 65535u;
+    groups_count_kernel<<<grid, kGroupBlock, 0, st>>>(g.labels, g.m, g.n_clusters, g.offsets, g.state);
+    partition_scan_kernel<<<1, kPartitionBlock, 0, st>>>(g.offsets, g.n_clusters, g.m, g.totals);
+    groups_scatter_kernel<<<grid, kGroupBlock, 0, st>>>(g.labels, g.m, g.n_clusters, g.offsets, g.totals, g.cursor, g.members);
+    search(g, st);
+    return (int)cudaGetLastError();
+}
+
+// fks_end_states_gather_starts: value v of the outputs is component v mod cfg_stride of slot v / cfg_stride
+__global__ void __launch_bounds__(256) gather_starts_kernel(const char* results, size_t rec_stride, int cfg_stride, const unsigned* offsets,
+                                                            const unsigned* members, const unsigned* selected, unsigned per_group,
+                                                            size_t n_values, const double* group_targets, double* starts, double* targets) {
+    for (size_t v = (size_t)blockIdx.x * blockDim.x + threadIdx.x; v < n_values; v += (size_t)gridDim.x * blockDim.x) {
+        const unsigned slot = (unsigned)(v / (unsigned)cfg_stride), t = (unsigned)(v % (unsigned)cfg_stride);
+        const unsigned s = slot / per_group, j = slot % per_group;
+        const unsigned g = selected[s], begin = offsets[g], k = offsets[g + 1] - begin;
+        starts[v] = k ? reinterpret_cast<const double*>(results + (size_t)members[begin + j % k] * rec_stride)[t] : NAN;
+        if (targets) targets[v] = group_targets[(size_t)s * cfg_stride + t];
+    }
+}
+
+int launch_gather_starts(const char* results, size_t rec_stride, int cfg_stride, const unsigned* offsets, const unsigned* members,
+                         const unsigned* selected, unsigned n_selected, unsigned per_group, const double* group_targets, double* starts,
+                         double* targets, void* stream) {
+    const size_t n_values = (size_t)n_selected * per_group * (size_t)cfg_stride;
+    const size_t grid = (n_values + 255) / 256 < 65535 ? (n_values + 255) / 256 : 65535;
+    gather_starts_kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(results, rec_stride, cfg_stride, offsets, members, selected, per_group,
+                                                                            n_values, group_targets, starts, targets);
+    return (int)cudaGetLastError();
+}
+
 #ifdef FKS_PHASE_TIMERS
 __global__ void dbg_copy_kernel(unsigned long long* out) {
     if (threadIdx.x < 64) {

@@ -333,6 +333,32 @@ class GpuParticleContactSimulator:
                                          _dev_ptr(d_labels), counts.ctypes.data_as(C.POINTER(C.c_uint64)), int(stream) if stream else None))
         return counts[:n_segments]
 
+    def end_states_groups(self, d_results, m, d_labels, n_clusters, d_group_offsets, d_members, d_representatives, d_radius, d_order=None,
+                          stream=0):
+        """The clusters of positions 0 .. m-1 (record d_order[p], or p; cluster d_labels[p]) as groups, on the device
+        (fks_end_states_groups): d_members[d_group_offsets[c] .. d_group_offsets[c+1]) = group c's record ids in position
+        order, d_representatives[c] / d_radius[c] = its minimax member and that member's largest distance to the others.
+        Device buffers (uint32 / float64) of n_clusters + 1, m, n_clusters, n_clusters entries; returns the group sizes
+        (numpy uint64)."""
+        sizes = np.zeros(max(int(n_clusters), 1), np.uint64)
+        check(lib.fks_end_states_groups(self._h, _dev_ptr(d_results), _dev_ptr(d_order), int(m), _dev_ptr(d_labels), int(n_clusters),
+                                        _dev_ptr(d_group_offsets), _dev_ptr(d_members), _dev_ptr(d_representatives), _dev_ptr(d_radius),
+                                        sizes.ctypes.data_as(C.POINTER(C.c_uint64)), int(stream) if stream else None))
+        return sizes[:int(n_clusters)]
+
+    def end_states_gather_starts(self, d_results, d_group_offsets, d_members, n_clusters, selected, per_group, d_starts,
+                                 d_group_targets=None, d_targets=None, stream=0):
+        """The next batch from groups (fks_end_states_gather_starts): slot s takes group selected[s] (host ids, repeats
+        allowed) and fills per_group starts with its members' configurations, cyclically; with d_group_targets
+        ([len(selected)][stride]), d_targets gets slot s's target per_group times.  Asynchronous on `stream`."""
+        sel = np.asarray(selected).reshape(-1)
+        if sel.size and (sel.min() < 0 or sel.max() > 0xFFFFFFFF):
+            raise capi.FksError(capi.ERR_INVALID_ARGUMENT, "end_states_gather_starts: a selected group id is not a uint32")
+        sel = np.ascontiguousarray(sel, dtype=np.uint32)
+        check(lib.fks_end_states_gather_starts(self._h, _dev_ptr(d_results), _dev_ptr(d_group_offsets), _dev_ptr(d_members), int(n_clusters),
+                                               sel.ctypes.data_as(C.POINTER(C.c_uint32)), sel.size, int(per_group), _dev_ptr(d_group_targets),
+                                               _dev_ptr(d_starts), _dev_ptr(d_targets), int(stream) if stream else None))
+
     def trace_dtype(self):
         width = (lib.fks_sim_trace_stride(self._h) - 16) // 8
         return np.dtype([("kind", np.uint32), ("step", np.uint32), ("microstep", np.uint32), ("iteration", np.uint32),

@@ -481,6 +481,35 @@ int fks_end_states_cluster(fks_sim* sim, const void* d_results, const uint32_t* 
                            size_t n_segments, int linkage, double max_cluster_distance, int separate_contact, uint32_t* d_labels,
                            uint64_t* cluster_counts, void* cuda_stream);
 
+/* fks_end_states_groups: clusters as particle groups -- the planner's child states.  Positions 0 .. m-1 name records as in
+ * fks_end_states_cluster (d_order[p], or p); d_labels[p] < n_clusters is position p's cluster (e.g. that call's output).
+ *  - members: d_members[d_group_offsets[c] .. d_group_offsets[c+1]) = the record ids of the positions labelled c, in
+ *    increasing order of position (a stable counting sort by label); d_group_offsets[0] = 0, [n_clusters] = m;
+ *  - d(p, q), p < q positions of one cluster = entry [p][q] of fks_end_states_pairwise_distance over the same ids (same
+ *    direction, same bits), +inf where that is NaN;
+ *  - representative: the minimax member, the p that minimises r(p) = max over the other members q of d(min(p,q), max(p,q)),
+ *    ties to the smallest position; d_representatives[c] = its record id, d_radius[c] = r(p) (0.0 for a singleton; +inf,
+ *    with the smallest position, when every r is +inf);
+ *  - group_sizes (HOST, n_clusters entries) = member counts.  The call returns after the stream has finished.
+ * Clusters of up to 256 members are searched one CTA each, larger ones (up to 8192) with their rows split over CTAs.
+ * FKS_ERR_INVALID_ARGUMENT: a label >= n_clusters, a cluster without members or with more than 8192, n_clusters > m,
+ * m >= 2^32, null buffers when m > 0; device outputs are then unspecified.  m == 0 launches nothing. */
+int fks_end_states_groups(fks_sim* sim, const void* d_results, const uint32_t* d_order, size_t m, const uint32_t* d_labels,
+                          size_t n_clusters, uint32_t* d_group_offsets, uint32_t* d_members, uint32_t* d_representatives,
+                          double* d_radius, uint64_t* group_sizes, void* cuda_stream);
+
+/* fks_end_states_gather_starts: the next batch from chosen groups.  For slot s < n_selected (g = selected[s], a HOST array;
+ * repeats and any order allowed), k = the size of group g and j < per_group:
+ *   d_starts[s * per_group + j]  = the configuration (cfg_stride doubles) of record d_members[d_group_offsets[g] + j mod k];
+ *   d_targets[s * per_group + j] = d_group_targets[s] (both NULL: no targets).
+ * The outputs are the starts / targets of fks_forward_simulate_device(n = n_targets = n_selected * per_group).  Groups as
+ * fks_end_states_groups writes them; a group of 0 members gets NaN starts.  Asynchronous on the stream.
+ * FKS_ERR_INVALID_ARGUMENT: per_group == 0, a selected id >= n_clusters, n_selected * per_group >= 2^32, null buffers when
+ * the output is not empty, or exactly one of d_targets / d_group_targets.  n_selected == 0 launches nothing. */
+int fks_end_states_gather_starts(fks_sim* sim, const void* d_results, const uint32_t* d_group_offsets, const uint32_t* d_members,
+                                 size_t n_clusters, const uint32_t* selected, size_t n_selected, size_t per_group,
+                                 const double* d_group_targets, double* d_starts, double* d_targets, void* cuda_stream);
+
 /* -------------------------------------------------------------------------------------------
  * Test entry: the device's stacked-Jacobian solver (ComputeResolverCorrectionStepStackedJacobian, spcs.hpp:1990-1998 =
  * J.colPivHouseholderQr().solve(c)) on caller-provided systems, one warp each.  System i has rows[i] rows and `cols`
