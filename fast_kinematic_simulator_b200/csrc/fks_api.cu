@@ -131,6 +131,11 @@ struct fks_sim {
     size_t cap_sel = 0;
     cudaEvent_t sel_read = nullptr;
     bool has_sel = false;
+    // fks_nearest_configurations: the split's per-chunk lists [distances | ids as u32], and when the last launch reading them is done
+    unsigned long long* d_near = nullptr;
+    size_t cap_near = 0;
+    cudaEvent_t near_done = nullptr;
+    bool has_near = false;
     unsigned long long* d_trace_buf = nullptr;  // fks_forward_simulate_traced: [counter word | records], grown on demand
     size_t cap_trace_buf = 0;
     size_t smem_limit;
@@ -696,6 +701,9 @@ void fks_sim_destroy(fks_sim* s) {
     cudaFree(s->d_grp);
     cudaFree(s->d_sel);
     if (s->sel_read) cudaEventDestroy(s->sel_read);
+    if (s->has_near) cudaEventSynchronize(s->near_done);
+    cudaFree(s->d_near);
+    if (s->near_done) cudaEventDestroy(s->near_done);
     cudaFree(s->d_ctx_store);
     cudaFree(s->d_results);
     if (s->last_done) cudaEventDestroy(s->last_done);
@@ -1287,6 +1295,55 @@ int fks_end_states_gather_starts(fks_sim* s, const void* d_results, const uint32
     s->launches += 1;
     FKS_CUDA(cudaEventRecord(s->sel_read, stream));
     s->has_sel = true;
+    return FKS_OK;
+}
+
+int fks_nearest_configurations(fks_sim* s, const double* d_candidates, size_t m, const double* d_queries, size_t n_queries, size_t k,
+                               uint32_t* d_ids, double* d_distances, void* cuda_stream) {
+    if (!s) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_nearest_configurations: null simulator");
+    if (k == 0 || k > kNearestMaxK) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_nearest_configurations: k is 0 or above " + std::to_string(kNearestMaxK));
+    if (m > 0xffffffffull) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_nearest_configurations: 2^32 or more candidates");
+    if (n_queries > 0xffffffffull / k) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_nearest_configurations: n_queries * k is 2^32 or more");
+    if (n_queries == 0) return FKS_OK;
+    if (!d_queries || !d_ids || !d_distances || (m > 0 && !d_candidates))
+        return fail(FKS_ERR_INVALID_ARGUMENT, "fks_nearest_configurations: null buffer");
+    NvtxRange range("fks_nearest_configurations");
+    DeviceGuard guard(s->device);
+    if (!guard.ok) return fail(FKS_ERR_CUDA, "fks_nearest_configurations: cudaSetDevice failed");
+    cudaStream_t stream = (cudaStream_t)cuda_stream;
+    NearestLaunch a;
+    a.robot = s->robot->d_robot;
+    a.candidates = d_candidates;
+    a.queries = d_queries;
+    a.cfg_stride = s->robot->stride;
+    a.m = (unsigned)m;
+    a.n_queries = (unsigned)n_queries;
+    a.k = (unsigned)k;
+    a.n_split = nearest_split(a.m, a.n_queries, s->num_sms);
+    a.chunk = (unsigned)((m + a.n_split - 1) / a.n_split);
+    if (a.n_split > 1) a.n_split = (unsigned)((m + a.chunk - 1) / a.chunk);  // no empty chunk
+    a.ids = d_ids;
+    a.distances = d_distances;
+    a.part_d = nullptr;
+    a.part_i = nullptr;
+    if (a.n_split > 1) {
+        const size_t n_keys = n_queries * a.n_split * k;
+        if (!s->near_done) FKS_CUDA(cudaEventCreateWithFlags(&s->near_done, cudaEventDisableTiming));
+        // the lists go through one buffer: the launches of an earlier call, perhaps on another stream, must be done with it
+        if (s->has_near && n_keys + (n_keys + 1) / 2 > s->cap_near) FKS_CUDA(cudaEventSynchronize(s->near_done));
+        int rc;
+        if ((rc = ensure(&s->d_near, &s->cap_near, n_keys + (n_keys + 1) / 2)) != FKS_OK) return rc;
+        if (s->has_near) FKS_CUDA(cudaStreamWaitEvent(stream, s->near_done, 0));
+        a.part_d = reinterpret_cast<double*>(s->d_near);
+        a.part_i = reinterpret_cast<unsigned*>(s->d_near + n_keys);
+    }
+    const int rc = launch_nearest(s->robot->host.kind, a, stream);
+    if (rc != 0) return cuda_fail((cudaError_t)rc, "fks_nearest_configurations: launch");
+    s->launches += a.n_split > 1 ? 2 : 1;
+    if (a.n_split > 1) {
+        FKS_CUDA(cudaEventRecord(s->near_done, stream));
+        s->has_near = true;
+    }
     return FKS_OK;
 }
 

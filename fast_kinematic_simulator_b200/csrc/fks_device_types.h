@@ -386,6 +386,25 @@ int launch_groups(int kind, const GroupsLaunch& g, void* stream);
 int launch_gather_starts(const char* results, size_t rec_stride, int cfg_stride, const unsigned* offsets, const unsigned* members,
                          const unsigned* selected, unsigned n_selected, unsigned per_group, const double* group_targets, double* starts,
                          double* targets, void* stream);
+// fks_nearest_configurations: the k <= kNearestMaxK nearest candidates per query under config_distance<KIND>.  With
+// n_split == 1 one scan launch writes the output (the query-tiled path); with n_split > 1 each query's candidates are cut
+// into n_split chunks of `chunk`, the scan writes a list per (query, chunk) to the workspace and a second launch merges them.
+constexpr unsigned kNearestMaxK = 64;
+struct NearestLaunch {
+    const DevRobot* robot;
+    const double* candidates;  // device [m][cfg_stride]
+    const double* queries;     // device [n_queries][cfg_stride]
+    int cfg_stride;
+    unsigned m, n_queries, k;
+    unsigned n_split, chunk;
+    unsigned* ids;             // device [n_queries * k] (the caller's)
+    double* distances;         // device [n_queries * k] (the caller's)
+    double* part_d;            // workspace [n_queries * n_split * k] when n_split > 1
+    unsigned* part_i;          // workspace [n_queries * n_split * k] when n_split > 1
+};
+// the chunks per query the host picks from n_queries and m (1: the query-tiled path)
+unsigned nearest_split(unsigned m, unsigned n_queries, int num_sms);
+int launch_nearest(int kind, const NearestLaunch& a, void* stream);
 int launch_dbg_copy(unsigned long long* out, void* stream);  // developer counters of the FKS_PHASE_TIMERS build
 int launch_fp64_peak(double* out, int grid, int iters, void* stream);
 int launch_gather(const float* data, unsigned long long n_mask, float* out, int grid, int iters, void* stream);

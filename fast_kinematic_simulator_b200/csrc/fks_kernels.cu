@@ -3605,6 +3605,192 @@ int launch_gather_starts(const char* results, size_t rec_stride, int cfg_stride,
     return (int)cudaGetLastError();
 }
 
+// ---------------------------------------------------------------------------------------------
+// fks_nearest_configurations: per query the k smallest keys (d, i), d = config_distance<KIND>(candidate i, query) -- the
+// pairwise kernel's inlined distance with the candidate as `cur`, as in its entry [i][m + j] -- NaN as +inf.  A warp keeps a
+// query's running list sorted by key over 64 positions, position p in lane p mod 32 (slot p / 32); a key enters only if it
+// is below the one at position k - 1.  Keys are a total order, so the k smallest of a union are the k smallest of the parts'
+// k smallest: any split of the candidates and any merge order give the same bits.
+// ---------------------------------------------------------------------------------------------
+constexpr int kNearestBlock = 256;
+constexpr unsigned kNearestWarps = kNearestBlock / 32;  // queries per CTA of the scan
+constexpr unsigned kNearestTileDoubles = 4096;          // the candidate tile in shared memory (32 KiB)
+constexpr int kNearestCfgMax = kMaxDof < 12 ? 12 : kMaxDof;
+constexpr unsigned kNearestCtasPerSm = 4;     // the scan's grid the split aims at
+constexpr unsigned kNearestMinChunk = 2048;   // fewest candidates per chunk of a split
+
+struct NearestList {
+    double d0, d1;    // keys at positions lane, 32 + lane
+    unsigned i0, i1;
+};
+
+struct NearestShared {
+    double d[kNearestWarps][kNearestMaxK];
+    unsigned i[kNearestWarps][kNearestMaxK];
+};
+
+__device__ __forceinline__ void nearest_list_init(NearestList& L, double& kd, unsigned& ki) {
+    L.d0 = L.d1 = kd = INFINITY;
+    L.i0 = L.i1 = ki = 0xffffffffu;
+}
+
+// (d, i), the same in every lane, goes to its rank; the key at position 63 drops out.  kd / ki = the key at position k - 1.
+__device__ __forceinline__ void nearest_insert(NearestList& L, unsigned k, double& kd, unsigned& ki, double d, unsigned i) {
+    const unsigned lane = threadIdx.x & 31;
+    const unsigned pos = __popc(__ballot_sync(FKS_FULL, cluster_key_less(L.d0, L.i0, d, i))) +
+                         __popc(__ballot_sync(FKS_FULL, cluster_key_less(L.d1, L.i1, d, i)));
+    const double up_d0 = __shfl_up_sync(FKS_FULL, L.d0, 1), last_d0 = __shfl_sync(FKS_FULL, L.d0, 31);
+    const unsigned up_i0 = __shfl_up_sync(FKS_FULL, L.i0, 1), last_i0 = __shfl_sync(FKS_FULL, L.i0, 31);
+    double up_d1 = __shfl_up_sync(FKS_FULL, L.d1, 1);
+    unsigned up_i1 = __shfl_up_sync(FKS_FULL, L.i1, 1);
+    if (lane == 0) {
+        up_d1 = last_d0;
+        up_i1 = last_i0;
+    }
+    if (lane == pos) {
+        L.d0 = d;
+        L.i0 = i;
+    } else if (lane > pos) {
+        L.d0 = up_d0;
+        L.i0 = up_i0;
+    }
+    if (lane + 32 == pos) {
+        L.d1 = d;
+        L.i1 = i;
+    } else if (lane + 32 > pos) {
+        L.d1 = up_d1;
+        L.i1 = up_i1;
+    }
+    kd = __shfl_sync(FKS_FULL, k > 32 ? L.d1 : L.d0, (k - 1) & 31);
+    ki = __shfl_sync(FKS_FULL, k > 32 ? L.i1 : L.i0, (k - 1) & 31);
+}
+
+// every lane offers one key; those below the k-th enter in lane order (invalid lanes offer (+inf, 0xffffffff))
+__device__ __forceinline__ void nearest_offer(NearestList& L, unsigned k, double& kd, unsigned& ki, double d, unsigned i) {
+    unsigned mask = __ballot_sync(FKS_FULL, cluster_key_less(d, i, kd, ki));
+    while (mask) {
+        const int src = __ffs(mask) - 1;
+        mask &= mask - 1;
+        const double bd = __shfl_sync(FKS_FULL, d, src);
+        const unsigned bi = __shfl_sync(FKS_FULL, i, src);
+        if (cluster_key_less(bd, bi, kd, ki)) nearest_insert(L, k, kd, ki, bd, bi);
+    }
+}
+
+// the first k keys of a stored list
+__device__ __forceinline__ void nearest_offer_list(NearestList& L, unsigned k, double& kd, unsigned& ki, const double* d, const unsigned* id) {
+    const unsigned lane = threadIdx.x & 31;
+    for (unsigned p0 = 0; p0 < k; p0 += 32) {
+        const unsigned p = p0 + lane;
+        nearest_offer(L, k, kd, ki, p < k ? d[p] : INFINITY, p < k ? id[p] : 0xffffffffu);
+    }
+}
+
+__device__ __forceinline__ void nearest_store(const NearestList& L, unsigned k, double* d, unsigned* id) {
+    const unsigned lane = threadIdx.x & 31;
+    if (lane < k) {
+        d[lane] = L.d0;
+        id[lane] = L.i0;
+    }
+    if (lane + 32 < k) {
+        d[lane + 32] = L.d1;
+        id[lane + 32] = L.i1;
+    }
+}
+
+// warps q + s * n_lists, 0 < s < per, hand their lists to warp q through shared memory (per is the same in the whole CTA)
+__device__ __forceinline__ void nearest_block_merge(NearestList& L, unsigned k, double& kd, unsigned& ki, unsigned n_lists, unsigned per,
+                                                    NearestShared& sh) {
+    const unsigned warp = threadIdx.x >> 5;
+    if (per == 1) return;
+    if (warp >= n_lists && warp < n_lists * per) nearest_store(L, k, sh.d[warp], sh.i[warp]);
+    __syncthreads();
+    if (warp < n_lists)
+        for (unsigned s = 1; s < per; s++) nearest_offer_list(L, k, kd, ki, sh.d[warp + s * n_lists], sh.i[warp + s * n_lists]);
+}
+
+// CTA (x, y): queries 8x .. 8x + qt - 1 against chunk y of the candidates, streamed through shared memory in coalesced tiles.
+// With qt < 8 queries, per = 8 / qt warps share a query, each taking every per-th group of 32 candidates of a tile.
+template <int KIND>
+__global__ void __launch_bounds__(kNearestBlock) nearest_scan_kernel(NearestLaunch a) {
+    __shared__ double cand[kNearestTileDoubles];
+    __shared__ double qry[kNearestWarps * kNearestCfgMax];
+    __shared__ NearestShared sh;
+    const unsigned tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, S = (unsigned)a.cfg_stride;
+    const unsigned q0 = blockIdx.x * kNearestWarps, qt = min(kNearestWarps, a.n_queries - q0), per = kNearestWarps / qt;
+    const unsigned qi = warp % qt, sub = warp / qt;
+    for (unsigned t = tid; t < qt * S; t += kNearestBlock) qry[t] = a.queries[(size_t)q0 * S + t];
+    const unsigned c_begin = blockIdx.y * a.chunk, c_end = (unsigned)min((size_t)a.m, (size_t)c_begin + a.chunk), tile = kNearestTileDoubles / S;
+    NearestList L;
+    double kd;
+    unsigned ki;
+    nearest_list_init(L, kd, ki);
+    for (unsigned c0 = c_begin, n; c0 < c_end; c0 += n) {
+        n = min(tile, c_end - c0);
+        __syncthreads();  // the previous tile is consumed (and the queries are in place)
+        const double* src = a.candidates + (size_t)c0 * S;
+        for (unsigned t = tid; t < n * S; t += kNearestBlock) cand[t] = src[t];
+        __syncthreads();
+        if (sub >= per) continue;
+        for (unsigned b = sub * 32; b < n; b += 32 * per) {
+            const unsigned c = b + lane;
+            double d = INFINITY;
+            unsigned id = 0xffffffffu;
+            if (c < n) {
+                d = config_distance<KIND>(*a.robot, cand + c * S, qry + qi * S);
+                if (isnan(d)) d = INFINITY;
+                id = c0 + c;
+            }
+            nearest_offer(L, a.k, kd, ki, d, id);
+        }
+    }
+    nearest_block_merge(L, a.k, kd, ki, qt, per, sh);
+    if (warp >= qt) return;
+    const size_t q = q0 + qi;
+    if (a.n_split == 1) nearest_store(L, a.k, a.distances + q * a.k, a.ids + q * a.k);
+    else nearest_store(L, a.k, a.part_d + (q * a.n_split + blockIdx.y) * a.k, a.part_i + (q * a.n_split + blockIdx.y) * a.k);
+}
+
+// one CTA per query: warp w takes the chunk lists w, w + 8, ..., then warp 0 takes the other warps' lists
+__global__ void __launch_bounds__(kNearestBlock) nearest_merge_kernel(NearestLaunch a) {
+    __shared__ NearestShared sh;
+    const unsigned warp = threadIdx.x >> 5;
+    const size_t q = blockIdx.x;
+    NearestList L;
+    double kd;
+    unsigned ki;
+    nearest_list_init(L, kd, ki);
+    for (unsigned s = warp; s < a.n_split; s += kNearestWarps)
+        nearest_offer_list(L, a.k, kd, ki, a.part_d + (q * a.n_split + s) * a.k, a.part_i + (q * a.n_split + s) * a.k);
+    nearest_block_merge(L, a.k, kd, ki, 1, kNearestWarps, sh);
+    if (warp == 0) nearest_store(L, a.k, a.distances + q * a.k, a.ids + q * a.k);
+}
+
+// Split only when the query tiles would fill at most half of a kNearestCtasPerSm grid: then up to the grid's worth of
+// chunks per tile, none below kNearestMinChunk candidates.
+unsigned nearest_split(unsigned m, unsigned n_queries, int num_sms) {
+    const size_t tiles = ((size_t)n_queries + kNearestWarps - 1) / kNearestWarps;
+    const size_t target = (size_t)kNearestCtasPerSm * (size_t)(num_sms > 0 ? num_sms : 1);
+    if (tiles == 0 || 2 * tiles > target) return 1;
+    const size_t by_m = ((size_t)m + kNearestMinChunk - 1) / kNearestMinChunk;
+    const size_t s = target / tiles < by_m ? target / tiles : by_m;
+    return s > 1 ? (unsigned)s : 1u;
+}
+
+int launch_nearest(int kind, const NearestLaunch& a, void* stream) {
+    if (a.n_queries == 0 || a.k == 0 || a.k > kNearestMaxK || a.n_split == 0 || a.cfg_stride > kNearestCfgMax) return (int)cudaErrorInvalidValue;
+    cudaStream_t st = (cudaStream_t)stream;
+    const dim3 grid((a.n_queries + kNearestWarps - 1) / kNearestWarps, a.n_split);
+    switch (kind) {
+        case FKS_ROBOT_SE2: nearest_scan_kernel<FKS_ROBOT_SE2><<<grid, kNearestBlock, 0, st>>>(a); break;
+        case FKS_ROBOT_SE3: nearest_scan_kernel<FKS_ROBOT_SE3><<<grid, kNearestBlock, 0, st>>>(a); break;
+        case FKS_ROBOT_LINKED: nearest_scan_kernel<FKS_ROBOT_LINKED><<<grid, kNearestBlock, 0, st>>>(a); break;
+        default: return (int)cudaErrorInvalidValue;
+    }
+    if (a.n_split > 1) nearest_merge_kernel<<<a.n_queries, kNearestBlock, 0, st>>>(a);
+    return (int)cudaGetLastError();
+}
+
 #ifdef FKS_PHASE_TIMERS
 __global__ void dbg_copy_kernel(unsigned long long* out) {
     if (threadIdx.x < 64) {

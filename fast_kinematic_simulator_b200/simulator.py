@@ -359,6 +359,14 @@ class GpuParticleContactSimulator:
                                                sel.ctypes.data_as(C.POINTER(C.c_uint32)), sel.size, int(per_group), _dev_ptr(d_group_targets),
                                                _dev_ptr(d_starts), _dev_ptr(d_targets), int(stream) if stream else None))
 
+    def nearest_configurations(self, d_candidates, m, d_queries, n_queries, k, d_ids, d_distances, stream=0):
+        """The k nearest of m candidate configurations to each of n_queries queries (fks_nearest_configurations), by the
+        robot's configuration distance from candidate to query: d_ids[j * k ..] (uint32) and d_distances[j * k ..] (float64)
+        in increasing order of (distance, index), padded with id 0xFFFFFFFF and +inf when m < k.  Device buffers of
+        [m][config_stride] and [n_queries][config_stride] float64; asynchronous on `stream`."""
+        check(lib.fks_nearest_configurations(self._h, _dev_ptr(d_candidates), int(m), _dev_ptr(d_queries), int(n_queries), int(k),
+                                             _dev_ptr(d_ids), _dev_ptr(d_distances), int(stream) if stream else None))
+
     def trace_dtype(self):
         width = (lib.fks_sim_trace_stride(self._h) - 16) // 8
         return np.dtype([("kind", np.uint32), ("step", np.uint32), ("microstep", np.uint32), ("iteration", np.uint32),

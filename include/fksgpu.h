@@ -510,6 +510,22 @@ int fks_end_states_gather_starts(fks_sim* sim, const void* d_results, const uint
                                  size_t n_clusters, const uint32_t* selected, size_t n_selected, size_t per_group,
                                  const double* d_group_targets, double* d_starts, double* d_targets, void* cuda_stream);
 
+/* fks_nearest_configurations: the k nearest candidates of every query -- the planner's nearest tree state to a sample.
+ * d_candidates [m][cfg_stride] and d_queries [n_queries][cfg_stride] are flat configurations (device), laid out like the
+ * starts and targets of fks_forward_simulate_device and the output of fks_end_states_gather_starts.
+ *  - d(i, j) = ComputeConfigurationDistanceTo from candidate i to query j: the bits of entry [i][m + j] of
+ *    fks_end_states_pairwise_distance over records holding the candidates and then the queries; +inf where that is NaN;
+ *  - d_ids[j*k .. j*k+k) = the k candidates with the smallest keys (d(i, j), i), in increasing order of key, and
+ *    d_distances[j*k ..] their d (NaN written as +inf).  Candidates at +inf are ranked too, by index; when m < k the
+ *    last k - m slots get id UINT32_MAX and +inf.
+ * The search is exact and deterministic: the same bits on every run, stream and device.  Few queries against many
+ * candidates split the candidates over the grid, through a workspace the simulator keeps; a later call on another stream
+ * waits for an earlier one's use of it.  Asynchronous on the stream.
+ * FKS_ERR_INVALID_ARGUMENT: k == 0 or k > 64, m >= 2^32, n_queries * k >= 2^32, null buffers when n_queries > 0 (d_candidates
+ * may be NULL when m == 0).  n_queries == 0 launches nothing; m == 0 writes the padding only. */
+int fks_nearest_configurations(fks_sim* sim, const double* d_candidates, size_t m, const double* d_queries, size_t n_queries,
+                               size_t k, uint32_t* d_ids, double* d_distances, void* cuda_stream);
+
 /* -------------------------------------------------------------------------------------------
  * Test entry: the device's stacked-Jacobian solver (ComputeResolverCorrectionStepStackedJacobian, spcs.hpp:1990-1998 =
  * J.colPivHouseholderQr().solve(c)) on caller-provided systems, one warp each.  System i has rows[i] rows and `cols`
