@@ -1,10 +1,10 @@
 // C ABI of libfksgpu.so (include/fksgpu.h): uploads, launch plumbing, statistics.
-// The computation itself is in fks_kernels.cu; the environment builder in host/environment_builder.cpp.
+// The computation itself is in fks_kernels.cu, the calls that consume a batch on the device in fks_consumers.cu, the
+// environment builder in host/environment_builder.cpp.
 // There is NO CPU fallback: every compute entry point fails with FKS_ERR_NO_DEVICE / FKS_ERR_CUDA when
 // the device path cannot run.
 
 #include <cuda_runtime.h>
-#include <nvtx3/nvToolsExt.h>  // header-only: named host ranges for Nsight Systems / ncu --nvtx, free without a tool attached
 
 #include <algorithm>
 #include <cmath>
@@ -38,31 +38,6 @@ void finish_env_l2_window(fks_env* env) {
 
 namespace {
 
-int fail(int code, const std::string& msg) {
-    fks_host::set_last_error(msg);
-    return code;
-}
-int cuda_fail(cudaError_t err, const char* what) {
-    return fail(FKS_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(err));
-}
-#define FKS_CUDA(call)                                        \
-    do {                                                      \
-        cudaError_t _e = (call);                              \
-        if (_e != cudaSuccess) return cuda_fail(_e, #call);   \
-    } while (0)
-
-struct DeviceGuard {
-    int prev;
-    bool ok;
-    explicit DeviceGuard(int dev) : prev(-1), ok(false) {
-        if (cudaGetDevice(&prev) != cudaSuccess) prev = -1;
-        ok = (cudaSetDevice(dev) == cudaSuccess);
-    }
-    ~DeviceGuard() {
-        if (prev >= 0) cudaSetDevice(prev);
-    }
-};
-
 template <typename T>
 int upload(T** dst, const T* src, size_t n) {
     *dst = nullptr;
@@ -72,104 +47,9 @@ int upload(T** dst, const T* src, size_t n) {
     return FKS_OK;
 }
 
-template <typename T>
-int ensure(T** ptr, size_t* cap, size_t need) {
-    if (need <= *cap) return FKS_OK;
-    cudaFree(*ptr);
-    *ptr = nullptr;
-    *cap = 0;
-    const size_t want = need + need / 4;
-    FKS_CUDA(cudaMalloc((void**)ptr, want * sizeof(T)));
-    *cap = want;
-    return FKS_OK;
-}
-
 }  // namespace
-
-struct fks_robot {
-    int device;
-    DevRobot host;
-    DevRobot* d_robot;
-    double2* d_pxy;
-    PointZL* d_pzl;
-    int stride;
-};
-
-struct fks_sim {
-    int device;
-    const fks_env* env;
-    const fks_robot* robot;
-    DevSolver sp;
-    uint64_t seed;
-    int32_t debug_level;
-    cudaStream_t stream;
-    int grid_max, num_sms;
-    size_t dyn_smem;
-    KernelInfo kinfo;
-    LaunchArgs plan;  // layouts and shared-memory offsets (simulate_smem_plan)
-    char* d_scratch;
-    char* d_jscratch = nullptr;
-    unsigned long long* d_stats;
-    unsigned int* d_counter;
-    // staging for the host-buffer entry point (grown on demand)
-    double *d_starts, *d_targets, *d_tape;
-    unsigned long long *d_tape_off, *d_dec, *d_dec_off;
-    char* d_results;
-    size_t cap_starts, cap_targets, cap_tape, cap_tape_off, cap_results, cap_dec, cap_dec_off;
-    unsigned int* d_part = nullptr;  // fks_end_states_partition: totals + per-block counts
-    size_t cap_part = 0;
-    // fks_end_states_cluster: [offsets | totals | counts, segment lists] and the distance matrices of the large segments
-    unsigned long long* d_clu = nullptr;
-    size_t cap_clu = 0;
-    double* d_clu_mat = nullptr;
-    size_t cap_clu_mat = 0;
-    // fks_end_states_groups: [totals (2) | row maxima (m doubles) | cursors, state as u32]
-    unsigned long long* d_grp = nullptr;
-    size_t cap_grp = 0;
-    // fks_end_states_gather_starts: the selected group ids, and when the last launch that reads them is done
-    unsigned* d_sel = nullptr;
-    size_t cap_sel = 0;
-    cudaEvent_t sel_read = nullptr;
-    bool has_sel = false;
-    // fks_nearest_configurations: the split's per-chunk lists [distances | ids as u32], and when the last launch reading them is done
-    unsigned long long* d_near = nullptr;
-    size_t cap_near = 0;
-    cudaEvent_t near_done = nullptr;
-    bool has_near = false;
-    unsigned long long* d_trace_buf = nullptr;  // fks_forward_simulate_traced: [counter word | records], grown on demand
-    size_t cap_trace_buf = 0;
-    size_t smem_limit;
-    // context pool of the simulate kernel: global store of parked particle contexts and their scratch slots
-    char* d_ctx_store;
-    int pool;
-    int pool_eighths = 16;
-    // device time of the simulate kernel of the last batch call (fks_sim_kernel_times), recorded only after
-    // fks_sim_enable_kernel_timing
-    cudaEvent_t tev[2];
-    int timing, timed_kernels;
-    // launches of one simulator share its particle counter, scratch slots and statistics: a launch on another stream waits
-    // for the previous one (fks_forward_simulate_device takes the caller's stream)
-    cudaEvent_t last_done;
-    cudaStream_t last_stream;
-    bool has_last;
-    uint64_t launches;
-    std::string info;
-    // set by fks_forward_simulate_traced around its launch, null otherwise
-    char* d_trace;
-    unsigned int* d_trace_count;
-    unsigned int trace_capacity;
-};
 
 extern "C" {
-
-namespace {
-struct NvtxRange {  // one named range per C-ABI call and per stage inside it
-    explicit NvtxRange(const char* name) { nvtxRangePushA(name); }
-    ~NvtxRange() { nvtxRangePop(); }
-    NvtxRange(const NvtxRange&) = delete;
-    NvtxRange& operator=(const NvtxRange&) = delete;
-};
-}  // namespace
 
 int fks_abi_version(void) { return FKS_ABI_VERSION; }
 
@@ -697,13 +577,9 @@ void fks_sim_destroy(fks_sim* s) {
     cudaFree(s->d_part);
     cudaFree(s->d_clu);
     cudaFree(s->d_clu_mat);
-    if (s->has_sel) cudaEventSynchronize(s->sel_read);
     cudaFree(s->d_grp);
-    cudaFree(s->d_sel);
-    if (s->sel_read) cudaEventDestroy(s->sel_read);
-    if (s->has_near) cudaEventSynchronize(s->near_done);
-    cudaFree(s->d_near);
-    if (s->near_done) cudaEventDestroy(s->near_done);
+    s->sel.destroy();
+    s->near.destroy();
     cudaFree(s->d_ctx_store);
     cudaFree(s->d_results);
     if (s->last_done) cudaEventDestroy(s->last_done);
@@ -1083,269 +959,6 @@ int fks_debug_phase_cycles(fks_sim* s, uint64_t* out16) {
 }
 
 const char* fks_sim_kernel_info(fks_sim* s) { return s ? s->info.c_str() : ""; }
-
-// ---------------------------------------------------------------------------------------------
-// first consumer of a batch on the device (fksgpu.h, SURVEY.md 8f-3)
-// ---------------------------------------------------------------------------------------------
-int fks_end_states_partition(fks_sim* s, const void* d_results, size_t n, uint32_t* d_order, uint64_t* counts, void* cuda_stream) {
-    if (!s || !counts) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_partition: null argument");
-    counts[0] = counts[1] = 0;
-    if (n == 0) return FKS_OK;
-    if (!d_results || !d_order || n > 0xffffffffull) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_partition: bad buffer or count");
-    NvtxRange range("fks_end_states_partition");
-    DeviceGuard guard(s->device);
-    if (!guard.ok) return fail(FKS_ERR_CUDA, "fks_end_states_partition: cudaSetDevice failed");
-    cudaStream_t stream = (cudaStream_t)cuda_stream;
-    int rc;
-    const size_t n_blocks = (n + 1023) / 1024;
-    if ((rc = ensure(&s->d_part, &s->cap_part, n_blocks + 4)) != FKS_OK) return rc;  // [2 x u64 totals | block counts]
-    unsigned long long* totals = reinterpret_cast<unsigned long long*>(s->d_part);
-    rc = launch_partition((const char*)d_results, fks_sim_result_stride(s), s->robot->stride, n, s->d_part + 4, totals, d_order, stream);
-    if (rc != 0) return cuda_fail((cudaError_t)rc, "fks_end_states_partition: launch");
-    s->launches += 3;
-    unsigned long long host[2] = {0, 0};
-    FKS_CUDA(cudaMemcpyAsync(host, totals, sizeof(host), cudaMemcpyDeviceToHost, stream));
-    FKS_CUDA(cudaStreamSynchronize(stream));
-    counts[0] = host[0];
-    counts[1] = host[1];
-    return FKS_OK;
-}
-
-int fks_end_states_pairwise_distance(fks_sim* s, const void* d_results, const uint32_t* d_subset, size_t m, double* d_out, void* cuda_stream) {
-    if (!s) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_pairwise_distance: null simulator");
-    if (m == 0) return FKS_OK;
-    if (!d_results || !d_out || m > 65535) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_pairwise_distance: bad buffer, or more than 65535 records");
-    NvtxRange range("fks_end_states_pairwise_distance");
-    DeviceGuard guard(s->device);
-    if (!guard.ok) return fail(FKS_ERR_CUDA, "fks_end_states_pairwise_distance: cudaSetDevice failed");
-    const int rc = launch_pairwise_distance(s->robot->host.kind, s->robot->d_robot, (const char*)d_results, fks_sim_result_stride(s),
-                                            s->robot->stride, d_subset, (unsigned)m, d_out, cuda_stream);
-    if (rc != 0) return cuda_fail((cudaError_t)rc, "fks_end_states_pairwise_distance: launch");
-    s->launches += 1;
-    return FKS_OK;
-}
-
-int fks_end_states_cluster(fks_sim* s, const void* d_results, const uint32_t* d_order, const uint64_t* segment_offsets, size_t n_segments,
-                           int linkage, double max_cluster_distance, int separate_contact, uint32_t* d_labels, uint64_t* cluster_counts,
-                           void* cuda_stream) {
-    if (!s) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_cluster: null simulator");
-    if (std::isnan(max_cluster_distance)) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_cluster: max_cluster_distance is NaN");
-    if (linkage != FKS_LINKAGE_SINGLE && linkage != FKS_LINKAGE_COMPLETE) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_cluster: unknown linkage");
-    if (n_segments == 0) return FKS_OK;
-    if (!segment_offsets || !cluster_counts) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_cluster: null segment offsets or counts");
-    if (n_segments > 0xffffffffull) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_cluster: more than 2^32 - 1 segments");
-    if (segment_offsets[0] != 0) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_cluster: segment_offsets[0] must be 0");
-    std::vector<uint32_t> small_segs, large_segs;
-    unsigned small_cap = 0, large_cap = 0;
-    for (size_t i = 0; i < n_segments; i++) {
-        if (segment_offsets[i + 1] < segment_offsets[i]) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_cluster: segment_offsets decrease");
-        const uint64_t len = segment_offsets[i + 1] - segment_offsets[i];
-        if (len > kClusterMaxSegment)
-            return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_cluster: a segment is longer than " + std::to_string(kClusterMaxSegment) + " positions");
-        if (len == 0) continue;
-        if (len <= kClusterSmallMax) {
-            small_segs.push_back((uint32_t)i);
-            small_cap = std::max(small_cap, (unsigned)len);
-        } else {
-            large_segs.push_back((uint32_t)i);
-            large_cap = std::max(large_cap, (unsigned)len);
-        }
-    }
-    const uint64_t m = segment_offsets[n_segments];
-    if (m > 0xffffffffull) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_cluster: 2^32 or more positions");
-    std::fill(cluster_counts, cluster_counts + n_segments, (uint64_t)0);
-    if (m == 0) return FKS_OK;
-    if (!d_results || !d_labels) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_cluster: null records or labels");
-    NvtxRange range("fks_end_states_cluster");
-    DeviceGuard guard(s->device);
-    if (!guard.ok) return fail(FKS_ERR_CUDA, "fks_end_states_cluster: cudaSetDevice failed");
-    cudaStream_t stream = (cudaStream_t)cuda_stream;
-
-    // one upload: [offsets (n + 1) | totals (2) | counts (n, zero), small segments, large segments as u32]
-    const size_t n_u32 = n_segments + small_segs.size() + large_segs.size();
-    std::vector<unsigned long long> meta(n_segments + 3 + (n_u32 + 1) / 2, 0ull);
-    std::memcpy(meta.data(), segment_offsets, (n_segments + 1) * sizeof(uint64_t));
-    uint32_t* meta32 = reinterpret_cast<uint32_t*>(meta.data() + n_segments + 3);
-    std::copy(small_segs.begin(), small_segs.end(), meta32 + n_segments);
-    std::copy(large_segs.begin(), large_segs.end(), meta32 + n_segments + small_segs.size());
-    int rc;
-    if ((rc = ensure(&s->d_clu, &s->cap_clu, meta.size())) != FKS_OK) return rc;
-    // large segments: one matrix slot per CTA, as many CTAs as SMs, segments and a 1 GiB workspace allow (at least one)
-    int large_slots = 0;
-    if (!large_segs.empty()) {
-        const size_t slot = (size_t)large_cap * large_cap;
-        large_slots = (int)std::max<size_t>(1, std::min<size_t>({large_segs.size(), (size_t)s->num_sms, ((size_t)1 << 30) / (slot * sizeof(double))}));
-        if ((rc = ensure(&s->d_clu_mat, &s->cap_clu_mat, slot * large_slots)) != FKS_OK) return rc;
-    }
-    FKS_CUDA(cudaMemcpyAsync(s->d_clu, meta.data(), meta.size() * sizeof(unsigned long long), cudaMemcpyHostToDevice, stream));
-    unsigned* d32 = reinterpret_cast<unsigned*>(s->d_clu + n_segments + 3);
-    ClusterLaunch c;
-    c.robot = s->robot->d_robot;
-    c.results = (const char*)d_results;
-    c.rec_stride = fks_sim_result_stride(s);
-    c.cfg_stride = s->robot->stride;
-    c.complete = linkage == FKS_LINKAGE_COMPLETE;
-    c.separate_contact = separate_contact != 0;
-    c.threshold = max_cluster_distance;
-    c.order = d_order;
-    c.offsets = s->d_clu;
-    c.n_segments = (unsigned)n_segments;
-    c.small_segs = d32 + n_segments;
-    c.n_small = (unsigned)small_segs.size();
-    c.small_cap = small_cap;
-    c.large_segs = d32 + n_segments + small_segs.size();
-    c.n_large = (unsigned)large_segs.size();
-    c.large_cap = large_cap;
-    c.work = s->d_clu_mat;
-    c.large_slots = large_slots;
-    c.labels = d_labels;
-    c.counts = d32;
-    c.totals = s->d_clu + n_segments + 1;
-    rc = launch_cluster(s->robot->host.kind, c, stream);
-    if (rc != 0) return cuda_fail((cudaError_t)rc, "fks_end_states_cluster: launch");
-    s->launches += 2 + (small_segs.empty() ? 0 : 1) + (large_segs.empty() ? 0 : 1);
-    std::vector<unsigned> base(n_segments);
-    unsigned long long total = 0;
-    FKS_CUDA(cudaMemcpyAsync(base.data(), d32, n_segments * sizeof(unsigned), cudaMemcpyDeviceToHost, stream));
-    FKS_CUDA(cudaMemcpyAsync(&total, c.totals + 1, sizeof(total), cudaMemcpyDeviceToHost, stream));
-    FKS_CUDA(cudaStreamSynchronize(stream));
-    for (size_t i = 0; i < n_segments; i++) cluster_counts[i] = (i + 1 < n_segments ? base[i + 1] : total) - base[i];
-    return FKS_OK;
-}
-
-int fks_end_states_groups(fks_sim* s, const void* d_results, const uint32_t* d_order, size_t m, const uint32_t* d_labels, size_t n_clusters,
-                          uint32_t* d_group_offsets, uint32_t* d_members, uint32_t* d_representatives, double* d_radius,
-                          uint64_t* group_sizes, void* cuda_stream) {
-    if (!s) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_groups: null simulator");
-    if (m > 0xffffffffull) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_groups: 2^32 or more positions");
-    if (n_clusters > m) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_groups: more clusters than positions");
-    if (m == 0) return FKS_OK;
-    if (!d_results || !d_labels || !d_group_offsets || !d_members || !d_representatives || !d_radius || !group_sizes)
-        return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_groups: null buffer");
-    if (n_clusters == 0) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_groups: a label is not below n_clusters");
-    NvtxRange range("fks_end_states_groups");
-    DeviceGuard guard(s->device);
-    if (!guard.ok) return fail(FKS_ERR_CUDA, "fks_end_states_groups: cudaSetDevice failed");
-    cudaStream_t stream = (cudaStream_t)cuda_stream;
-    const size_t n_state = 2 + m / (kGroupSmallMax + 1) + 1;
-    int rc;
-    if ((rc = ensure(&s->d_grp, &s->cap_grp, 2 + m + (n_clusters + n_state + 1) / 2)) != FKS_OK) return rc;
-    GroupsLaunch g;
-    g.robot = s->robot->d_robot;
-    g.results = (const char*)d_results;
-    g.rec_stride = fks_sim_result_stride(s);
-    g.cfg_stride = s->robot->stride;
-    g.order = d_order;
-    g.labels = d_labels;
-    g.m = (unsigned)m;
-    g.n_clusters = (unsigned)n_clusters;
-    g.offsets = d_group_offsets;
-    g.members = d_members;
-    g.reps = d_representatives;
-    g.radius = d_radius;
-    g.totals = s->d_grp;
-    g.row_max = reinterpret_cast<double*>(s->d_grp + 2);
-    g.cursor = reinterpret_cast<unsigned*>(s->d_grp + 2 + m);
-    g.state = g.cursor + n_clusters;
-    FKS_CUDA(cudaMemsetAsync(d_group_offsets, 0, n_clusters * sizeof(uint32_t), stream));
-    FKS_CUDA(cudaMemsetAsync(g.cursor, 0, (n_clusters + 2) * sizeof(uint32_t), stream));
-    rc = launch_groups(s->robot->host.kind, g, stream);
-    if (rc != 0) return cuda_fail((cudaError_t)rc, "fks_end_states_groups: launch");
-    s->launches += kGroupLaunches;
-    std::vector<uint32_t> offsets(n_clusters + 1);
-    uint32_t err = 0;
-    FKS_CUDA(cudaMemcpyAsync(offsets.data(), d_group_offsets, offsets.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
-    FKS_CUDA(cudaMemcpyAsync(&err, g.state + 1, sizeof(err), cudaMemcpyDeviceToHost, stream));
-    FKS_CUDA(cudaStreamSynchronize(stream));
-    if (err & kGroupErrLabel) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_groups: a label is not below n_clusters");
-    if (err & kGroupErrEmpty) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_groups: a cluster has no member");
-    if (err & kGroupErrLarge)
-        return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_groups: a cluster has more than " + std::to_string(kClusterMaxSegment) + " members");
-    for (size_t c = 0; c < n_clusters; c++) group_sizes[c] = offsets[c + 1] - offsets[c];
-    return FKS_OK;
-}
-
-int fks_end_states_gather_starts(fks_sim* s, const void* d_results, const uint32_t* d_group_offsets, const uint32_t* d_members,
-                                 size_t n_clusters, const uint32_t* selected, size_t n_selected, size_t per_group,
-                                 const double* d_group_targets, double* d_starts, double* d_targets, void* cuda_stream) {
-    if (!s) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_gather_starts: null simulator");
-    if (per_group == 0) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_gather_starts: per_group is 0");
-    if ((d_targets == nullptr) != (d_group_targets == nullptr))
-        return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_gather_starts: d_targets and d_group_targets go together");
-    if (n_selected == 0) return FKS_OK;
-    if (n_selected > 0xffffffffull / per_group) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_gather_starts: 2^32 or more starts");
-    if (!d_results || !d_group_offsets || !d_members || !selected || !d_starts)
-        return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_gather_starts: null buffer");
-    for (size_t i = 0; i < n_selected; i++)
-        if (selected[i] >= n_clusters) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_end_states_gather_starts: a selected group is not below n_clusters");
-    NvtxRange range("fks_end_states_gather_starts");
-    DeviceGuard guard(s->device);
-    if (!guard.ok) return fail(FKS_ERR_CUDA, "fks_end_states_gather_starts: cudaSetDevice failed");
-    cudaStream_t stream = (cudaStream_t)cuda_stream;
-    if (!s->sel_read) FKS_CUDA(cudaEventCreateWithFlags(&s->sel_read, cudaEventDisableTiming));
-    // the ids go through one buffer: a launch of an earlier call, perhaps on another stream, must have read it first
-    if (s->has_sel && n_selected > s->cap_sel) FKS_CUDA(cudaEventSynchronize(s->sel_read));
-    int rc;
-    if ((rc = ensure(&s->d_sel, &s->cap_sel, n_selected)) != FKS_OK) return rc;
-    if (s->has_sel) FKS_CUDA(cudaStreamWaitEvent(stream, s->sel_read, 0));
-    FKS_CUDA(cudaMemcpyAsync(s->d_sel, selected, n_selected * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
-    rc = launch_gather_starts((const char*)d_results, fks_sim_result_stride(s), s->robot->stride, d_group_offsets, d_members, s->d_sel,
-                              (unsigned)n_selected, (unsigned)per_group, d_group_targets, d_starts, d_targets, stream);
-    if (rc != 0) return cuda_fail((cudaError_t)rc, "fks_end_states_gather_starts: launch");
-    s->launches += 1;
-    FKS_CUDA(cudaEventRecord(s->sel_read, stream));
-    s->has_sel = true;
-    return FKS_OK;
-}
-
-int fks_nearest_configurations(fks_sim* s, const double* d_candidates, size_t m, const double* d_queries, size_t n_queries, size_t k,
-                               uint32_t* d_ids, double* d_distances, void* cuda_stream) {
-    if (!s) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_nearest_configurations: null simulator");
-    if (k == 0 || k > kNearestMaxK) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_nearest_configurations: k is 0 or above " + std::to_string(kNearestMaxK));
-    if (m > 0xffffffffull) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_nearest_configurations: 2^32 or more candidates");
-    if (n_queries > 0xffffffffull / k) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_nearest_configurations: n_queries * k is 2^32 or more");
-    if (n_queries == 0) return FKS_OK;
-    if (!d_queries || !d_ids || !d_distances || (m > 0 && !d_candidates))
-        return fail(FKS_ERR_INVALID_ARGUMENT, "fks_nearest_configurations: null buffer");
-    NvtxRange range("fks_nearest_configurations");
-    DeviceGuard guard(s->device);
-    if (!guard.ok) return fail(FKS_ERR_CUDA, "fks_nearest_configurations: cudaSetDevice failed");
-    cudaStream_t stream = (cudaStream_t)cuda_stream;
-    NearestLaunch a;
-    a.robot = s->robot->d_robot;
-    a.candidates = d_candidates;
-    a.queries = d_queries;
-    a.cfg_stride = s->robot->stride;
-    a.m = (unsigned)m;
-    a.n_queries = (unsigned)n_queries;
-    a.k = (unsigned)k;
-    a.n_split = nearest_split(a.m, a.n_queries, s->num_sms);
-    a.chunk = (unsigned)((m + a.n_split - 1) / a.n_split);
-    if (a.n_split > 1) a.n_split = (unsigned)((m + a.chunk - 1) / a.chunk);  // no empty chunk
-    a.ids = d_ids;
-    a.distances = d_distances;
-    a.part_d = nullptr;
-    a.part_i = nullptr;
-    if (a.n_split > 1) {
-        const size_t n_keys = n_queries * a.n_split * k;
-        if (!s->near_done) FKS_CUDA(cudaEventCreateWithFlags(&s->near_done, cudaEventDisableTiming));
-        // the lists go through one buffer: the launches of an earlier call, perhaps on another stream, must be done with it
-        if (s->has_near && n_keys + (n_keys + 1) / 2 > s->cap_near) FKS_CUDA(cudaEventSynchronize(s->near_done));
-        int rc;
-        if ((rc = ensure(&s->d_near, &s->cap_near, n_keys + (n_keys + 1) / 2)) != FKS_OK) return rc;
-        if (s->has_near) FKS_CUDA(cudaStreamWaitEvent(stream, s->near_done, 0));
-        a.part_d = reinterpret_cast<double*>(s->d_near);
-        a.part_i = reinterpret_cast<unsigned*>(s->d_near + n_keys);
-    }
-    const int rc = launch_nearest(s->robot->host.kind, a, stream);
-    if (rc != 0) return cuda_fail((cudaError_t)rc, "fks_nearest_configurations: launch");
-    s->launches += a.n_split > 1 ? 2 : 1;
-    if (a.n_split > 1) {
-        FKS_CUDA(cudaEventRecord(s->near_done, stream));
-        s->has_near = true;
-    }
-    return FKS_OK;
-}
 
 // ---------------------------------------------------------------------------------------------
 // test entry: the device's stacked-Jacobian solver on caller-provided systems (fksgpu.h)

@@ -1,4 +1,4 @@
-// Device-side data model of the particle contact simulator (shared by fks_kernels.cu and fks_api.cu).
+// Device-side data model of the particle contact simulator (shared by the library's translation units).
 //
 // Layout in HBM (uploaded once per environment / robot, read-only afterwards):
 //   SDF            float[nx*ny*nz], x-major (same linear index as VoxelGrid), L2-persisting window
@@ -326,85 +326,6 @@ size_t simulate_smem_plan(LaunchArgs* args, int L, int J, int D, int P, int stri
 int launch_check_config(int kind, const LaunchArgs& args, int grid, size_t dyn_smem, void* stream, double inflation_ratio, unsigned char* out);
 int launch_qr_solve(double* work, const unsigned long long* offsets, const int* rows, int cols, int n, double* x_out, unsigned* flags_out,
                     void* stream);
-int launch_partition(const char* results, size_t rec_stride, int cfg_stride, size_t n, unsigned* block_counts, unsigned long long* totals,
-                     unsigned* order, void* stream);
-int launch_pairwise_distance(int kind, const DevRobot* robot, const char* results, size_t rec_stride, int cfg_stride, const unsigned* subset,
-                             unsigned m, double* out, void* stream);
-// fks_end_states_cluster: segments of up to kClusterSmallMax positions keep their distance matrix in shared memory (160^2
-// doubles = 200 KiB of the 227 KiB a CTA can have), longer ones in a global slot of large_cap^2 doubles per CTA; the
-// per-position state of a segment (20 bytes each) stays in shared memory, which bounds a segment at kClusterMaxSegment.
-constexpr unsigned kClusterSmallMax = 160;
-constexpr unsigned kClusterMaxSegment = 8192;
-struct ClusterLaunch {
-    const DevRobot* robot;
-    const char* results;
-    size_t rec_stride;
-    int cfg_stride;
-    int complete, separate_contact;
-    double threshold;
-    const unsigned* order;              // device, or null
-    const unsigned long long* offsets;  // device [n_segments + 1]
-    unsigned n_segments;
-    const unsigned* small_segs;         // device: the non-empty segments of at most kClusterSmallMax positions
-    unsigned n_small, small_cap;        // their number and the longest one
-    const unsigned* large_segs;         // device: the longer segments
-    unsigned n_large, large_cap;
-    double* work;                       // large_slots * large_cap^2 doubles
-    int large_slots;
-    unsigned* labels;                   // [m]
-    unsigned* counts;                   // device [n_segments], zeroed: clusters per segment, then their exclusive scan
-    unsigned long long* totals;         // device [2]: totals[1] = all clusters
-};
-// the launches of one call: the two clustering kernels (those with segments), the scan of the counts and the relabel pass
-int launch_cluster(int kind, const ClusterLaunch& c, void* stream);
-// fks_end_states_groups: clusters of up to kGroupSmallMax members get their minimax representative from one CTA each, larger
-// ones (up to kClusterMaxSegment, the largest cluster fks_end_states_cluster makes) from row chunks spread over the grid.
-constexpr unsigned kGroupSmallMax = 256;
-constexpr unsigned kGroupErrLabel = 1, kGroupErrEmpty = 2, kGroupErrLarge = 4;  // bits of GroupsLaunch::state[1]
-struct GroupsLaunch {
-    const DevRobot* robot;
-    const char* results;
-    size_t rec_stride;
-    int cfg_stride;
-    const unsigned* order;          // device, or null
-    const unsigned* labels;         // device [m]
-    unsigned m, n_clusters;
-    unsigned* offsets;              // device [n_clusters + 1] (the caller's)
-    unsigned* members;              // device [m] (the caller's)
-    unsigned* reps;                 // device [n_clusters]
-    double* radius;                 // device [n_clusters]
-    unsigned long long* totals;     // workspace [2]
-    double* row_max;                // workspace [m]: r of every member of a large cluster, by slot
-    unsigned* cursor;               // workspace [n_clusters], zeroed
-    unsigned* state;                // workspace [2 + m / (kGroupSmallMax + 1) + 1], zeroed: large clusters, error bits, their list
-};
-// the launches of one call, whatever the number and sizes of the clusters: count, scan, scatter, sort + small search,
-// large rows, large argmin
-constexpr int kGroupLaunches = 6;
-int launch_groups(int kind, const GroupsLaunch& g, void* stream);
-// fks_end_states_gather_starts: one launch
-int launch_gather_starts(const char* results, size_t rec_stride, int cfg_stride, const unsigned* offsets, const unsigned* members,
-                         const unsigned* selected, unsigned n_selected, unsigned per_group, const double* group_targets, double* starts,
-                         double* targets, void* stream);
-// fks_nearest_configurations: the k <= kNearestMaxK nearest candidates per query under config_distance<KIND>.  With
-// n_split == 1 one scan launch writes the output (the query-tiled path); with n_split > 1 each query's candidates are cut
-// into n_split chunks of `chunk`, the scan writes a list per (query, chunk) to the workspace and a second launch merges them.
-constexpr unsigned kNearestMaxK = 64;
-struct NearestLaunch {
-    const DevRobot* robot;
-    const double* candidates;  // device [m][cfg_stride]
-    const double* queries;     // device [n_queries][cfg_stride]
-    int cfg_stride;
-    unsigned m, n_queries, k;
-    unsigned n_split, chunk;
-    unsigned* ids;             // device [n_queries * k] (the caller's)
-    double* distances;         // device [n_queries * k] (the caller's)
-    double* part_d;            // workspace [n_queries * n_split * k] when n_split > 1
-    unsigned* part_i;          // workspace [n_queries * n_split * k] when n_split > 1
-};
-// the chunks per query the host picks from n_queries and m (1: the query-tiled path)
-unsigned nearest_split(unsigned m, unsigned n_queries, int num_sms);
-int launch_nearest(int kind, const NearestLaunch& a, void* stream);
 int launch_dbg_copy(unsigned long long* out, void* stream);  // developer counters of the FKS_PHASE_TIMERS build
 int launch_fp64_peak(double* out, int grid, int iters, void* stream);
 int launch_gather(const float* data, unsigned long long n_mask, float* out, int grid, int iters, void* stream);

@@ -422,11 +422,6 @@ __global__ void __launch_bounds__(256) distance_field_check_kernel(const float* 
     if (!good) *ok = 0;
 }
 
-int fail(int code, const std::string& msg) {
-    fks_host::set_last_error(msg);
-    return code;
-}
-
 struct Temps {
     std::vector<void*> ptrs;
     std::vector<cudaEvent_t> events;

@@ -2,6 +2,9 @@
 #ifndef FKS_INTERNAL_H
 #define FKS_INTERNAL_H
 
+#include <cuda_runtime.h>
+#include <nvtx3/nvToolsExt.h>  // header-only: named host ranges for Nsight Systems / ncu --nvtx, free without a tool attached
+
 #include <cstdint>
 #include <string>
 #include <vector>
@@ -33,7 +36,132 @@ int check_sequence(const char* fn, const void* targets, size_t n, size_t n_legs,
 int simulate_host_async(fks_sim* s, const double* starts, const double* targets, size_t targets_pitch, size_t n, size_t n_targets,
                         size_t n_legs, uint64_t leg_id_stride, int allow_contacts, int noise_mode, const fks_noise_tape* tape,
                         uint64_t first_particle_id, void* results, size_t results_pitch);
+
+// A workspace that calls on any stream use in turn: acquire() makes `stream` wait for the launches of the previous call that
+// used it (and, when it has to grow, the host as well, since those launches may still read the old allocation); release()
+// marks the end of this call's launches on `stream`.  Both return FKS_OK or an FKS_ERR_* code (message set).
+struct StreamBuffer {
+    unsigned char* ptr = nullptr;
+    size_t cap = 0;  // bytes
+    cudaEvent_t done = nullptr;
+    bool pending = false;
+    int acquire(size_t bytes, cudaStream_t stream);
+    int release(cudaStream_t stream);
+    void destroy();  // waits for the last user
+};
 }  // namespace fks_host
+
+namespace {
+
+inline int fail(int code, const std::string& msg) {
+    fks_host::set_last_error(msg);
+    return code;
+}
+inline int cuda_fail(cudaError_t err, const char* what) {
+    return fail(FKS_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(err));
+}
+#define FKS_CUDA(call)                                        \
+    do {                                                      \
+        cudaError_t _e = (call);                              \
+        if (_e != cudaSuccess) return cuda_fail(_e, #call);   \
+    } while (0)
+
+struct DeviceGuard {
+    int prev;
+    bool ok;
+    explicit DeviceGuard(int dev) : prev(-1), ok(false) {
+        if (cudaGetDevice(&prev) != cudaSuccess) prev = -1;
+        ok = (cudaSetDevice(dev) == cudaSuccess);
+    }
+    ~DeviceGuard() {
+        if (prev >= 0) cudaSetDevice(prev);
+    }
+};
+
+struct NvtxRange {  // one named range per C-ABI call and per stage inside it
+    explicit NvtxRange(const char* name) { nvtxRangePushA(name); }
+    ~NvtxRange() { nvtxRangePop(); }
+    NvtxRange(const NvtxRange&) = delete;
+    NvtxRange& operator=(const NvtxRange&) = delete;
+};
+
+template <typename T>
+int ensure(T** ptr, size_t* cap, size_t need) {
+    if (need <= *cap) return FKS_OK;
+    cudaFree(*ptr);
+    *ptr = nullptr;
+    *cap = 0;
+    const size_t want = need + need / 4;
+    FKS_CUDA(cudaMalloc((void**)ptr, want * sizeof(T)));
+    *cap = want;
+    return FKS_OK;
+}
+
+}  // namespace
+
+struct fks_robot {
+    int device;
+    fksdev::DevRobot host;
+    fksdev::DevRobot* d_robot;
+    double2* d_pxy;
+    fksdev::PointZL* d_pzl;
+    int stride;
+};
+
+struct fks_sim {
+    int device;
+    const fks_env* env;
+    const fks_robot* robot;
+    fksdev::DevSolver sp;
+    uint64_t seed;
+    int32_t debug_level;
+    cudaStream_t stream;
+    int grid_max, num_sms;
+    size_t dyn_smem;
+    fksdev::KernelInfo kinfo;
+    fksdev::LaunchArgs plan;  // layouts and shared-memory offsets (simulate_smem_plan)
+    char* d_scratch;
+    char* d_jscratch = nullptr;
+    unsigned long long* d_stats;
+    unsigned int* d_counter;
+    // staging for the host-buffer entry point (grown on demand)
+    double *d_starts, *d_targets, *d_tape;
+    unsigned long long *d_tape_off, *d_dec, *d_dec_off;
+    char* d_results;
+    size_t cap_starts, cap_targets, cap_tape, cap_tape_off, cap_results, cap_dec, cap_dec_off;
+    // workspaces of the batch consumers (fks_consumers.cu, where their layouts are)
+    unsigned int* d_part = nullptr;
+    size_t cap_part = 0;
+    unsigned long long* d_clu = nullptr;
+    size_t cap_clu = 0;
+    double* d_clu_mat = nullptr;
+    size_t cap_clu_mat = 0;
+    unsigned long long* d_grp = nullptr;
+    size_t cap_grp = 0;
+    fks_host::StreamBuffer sel, near;  // fks_end_states_gather_starts, fks_nearest_configurations
+    unsigned long long* d_trace_buf = nullptr;  // fks_forward_simulate_traced: [counter word | records], grown on demand
+    size_t cap_trace_buf = 0;
+    size_t smem_limit;
+    // context pool of the simulate kernel: global store of parked particle contexts and their scratch slots
+    char* d_ctx_store;
+    int pool;
+    int pool_eighths = 16;
+    // device time of the simulate kernel of the last batch call (fks_sim_kernel_times), recorded only after
+    // fks_sim_enable_kernel_timing
+    cudaEvent_t tev[2];
+    int timing, timed_kernels;
+    // launches of one simulator share its particle counter, scratch slots and statistics: a launch on another stream waits
+    // for the previous one (fks_forward_simulate_device takes the caller's stream)
+    cudaEvent_t last_done;
+    cudaStream_t last_stream;
+    bool has_last;
+    uint64_t launches;
+    std::string info;
+    // set by fks_forward_simulate_traced around its launch, null otherwise
+    char* d_trace;
+    unsigned int* d_trace_count;
+    unsigned int trace_capacity;
+};
 
 // Device environment (fks_env_create / fks_env_build_device).
 struct fks_env {

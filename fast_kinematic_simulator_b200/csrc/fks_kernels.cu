@@ -31,10 +31,10 @@
 
 #include "fks_device_types.h"
 #include "fks_philox.h"
+#include "fks_robot_kind.cuh"
 
 namespace fksdev {
 
-#define FKS_FULL 0xffffffffu
 #ifndef FKS_SKIP_SINGLE_ESTIMATE
 #define FKS_SKIP_SINGLE_ESTIMATE 1
 #endif
@@ -45,8 +45,6 @@ namespace fksdev {
 extern __shared__ __align__(16) unsigned char smem_raw[];
 
 namespace {
-
-constexpr double kPi = 3.14159265358979323846;
 
 // ---- shared-memory accessors -------------------------------------------------------------------
 __device__ __forceinline__ const Frame& frame() { return *reinterpret_cast<const Frame*>(smem_raw); }
@@ -159,17 +157,6 @@ __device__ __forceinline__ double warp_max(double v) {
     return v;
 }
 
-// EigenHelpers::EnforceContinuousRevoluteBounds: wrap to (-pi, pi]
-__device__ __forceinline__ double wrap_angle(double value) {
-    if ((value <= -kPi) || (value > kPi)) {
-        const double remainder = fmod(value, 2.0 * kPi);
-        if (remainder <= -kPi) return remainder + (2.0 * kPi);
-        if (remainder > kPi) return remainder - (2.0 * kPi);
-        return remainder;
-    }
-    return value;
-}
-
 // (T is 16-byte aligned wherever it lives: 128-bit loads halve the shared-memory instructions and wavefronts of the point loops)
 __device__ __forceinline__ void apply_T(const double* T, double x, double y, double z, double& ox, double& oy, double& oz) {
     const double2 t01 = *reinterpret_cast<const double2*>(T + 0), t23 = *reinterpret_cast<const double2*>(T + 2);
@@ -201,24 +188,6 @@ __device__ __forceinline__ void rot_axis(double angle, double ax, double ay, dou
     R[9] = tyz + twx;
     R[10] = 1.0 - (txx + tyy);
     R[11] = 0.0;
-}
-
-// C = A * B for rigid transforms stored row-major 3x4
-__device__ __forceinline__ void iso_mul(const double* A, const double* B, double* C) {
-#pragma unroll
-    for (int r = 0; r < 3; r++) {
-#pragma unroll
-        for (int c = 0; c < 3; c++) C[4 * r + c] = A[4 * r + 0] * B[c] + A[4 * r + 1] * B[4 + c] + A[4 * r + 2] * B[8 + c];
-        C[4 * r + 3] = A[4 * r + 0] * B[3] + A[4 * r + 1] * B[7] + A[4 * r + 2] * B[11] + A[4 * r + 3];
-    }
-}
-__device__ __forceinline__ void iso_inverse(const double* A, double* C) {
-#pragma unroll
-    for (int r = 0; r < 3; r++)
-#pragma unroll
-        for (int c = 0; c < 3; c++) C[4 * r + c] = A[4 * c + r];
-#pragma unroll
-    for (int r = 0; r < 3; r++) C[4 * r + 3] = -(C[4 * r + 0] * A[3] + C[4 * r + 1] * A[7] + C[4 * r + 2] * A[11]);
 }
 
 // EigenHelpers::ExpTwist(twist, 1.0) (call sites tnuva:360,378): twist = (v, w)
@@ -331,41 +300,6 @@ __device__ __noinline__ void twist_between(const double* a, const double* b, dou
     twist[3] = wx;
     twist[4] = wy;
     twist[5] = wz;
-}
-
-// robot->ComputeConfigurationDistanceTo(target) (the call at spcs:898; the robot classes are upstream, so this follows the
-// oracle's restatement `Robot::distance_to`): SE2 / SE3 weigh translation and rotation angle, the linked robot takes the
-// weighted joint-space norm with continuous joints wrapped.
-template <int KIND>
-__device__ __forceinline__ double config_distance(const DevRobot& rb, const double* cur, const double* target) {
-    if (KIND == FKS_ROBOT_SE2) {
-        const double dx = fabs(target[0] - cur[0]), dy = fabs(target[1] - cur[1]);
-        const double dr = fabs(wrap_angle(target[2] - cur[2]));
-        return (sqrt(dx * dx + dy * dy) * rb.pos_w) + (dr * rb.rot_w);
-    } else if (KIND == FKS_ROBOT_SE3) {
-        double c12[12], tg[12], ci[12], Dm[12];
-#pragma unroll
-        for (int i = 0; i < 12; i++) {
-            c12[i] = cur[i];
-            tg[i] = target[i];
-        }
-        const double dx = tg[3] - c12[3], dy = tg[7] - c12[7], dz = tg[11] - c12[11];
-        iso_inverse(c12, ci);
-        iso_mul(ci, tg, Dm);
-        const double cs = fmin(fmax(0.5 * (Dm[0] + Dm[5] + Dm[10] - 1.0), -1.0), 1.0);
-        return (sqrt(dx * dx + dy * dy + dz * dz) * rb.pos_w) + (acos(cs) * rb.rot_w);
-    } else {
-        double sacc = 0.0;
-        for (int j = 0; j < rb.J; j++) {
-            const DevJoint& jd = rb.joints[j];
-            if (jd.active < 0) continue;
-            double dj = target[jd.active] - cur[jd.active];
-            if (jd.type == FKS_JOINT_CONTINUOUS) dj = wrap_angle(dj);
-            const double wd = dj * jd.weight;
-            sacc += wd * wd;
-        }
-        return sqrt(sacc);
-    }
 }
 
 // TruncatedNormalUncertainVelocityActuator::GetControlValue (unc:70-75 noiseless, :77-90 noisy)
@@ -2917,24 +2851,13 @@ int launch_simulate(int kind, const LaunchArgs& args, int grid, size_t dyn_smem,
 
 int launch_check_config(int kind, const LaunchArgs& args, int grid, size_t dyn_smem, void* stream, double inflation_ratio, unsigned char* out) {
     const int threads = 32 * args.warps_per_block;
-    cudaError_t err;
-    switch (kind) {
-        case FKS_ROBOT_SE2:
-            if ((err = cudaFuncSetAttribute(check_config_kernel<FKS_ROBOT_SE2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn_smem)) != cudaSuccess) return (int)err;
-            check_config_kernel<FKS_ROBOT_SE2><<<grid, threads, dyn_smem, (cudaStream_t)stream>>>(args, inflation_ratio, out);
-            break;
-        case FKS_ROBOT_SE3:
-            if ((err = cudaFuncSetAttribute(check_config_kernel<FKS_ROBOT_SE3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn_smem)) != cudaSuccess) return (int)err;
-            check_config_kernel<FKS_ROBOT_SE3><<<grid, threads, dyn_smem, (cudaStream_t)stream>>>(args, inflation_ratio, out);
-            break;
-        case FKS_ROBOT_LINKED:
-            if ((err = cudaFuncSetAttribute(check_config_kernel<FKS_ROBOT_LINKED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn_smem)) != cudaSuccess) return (int)err;
-            check_config_kernel<FKS_ROBOT_LINKED><<<grid, threads, dyn_smem, (cudaStream_t)stream>>>(args, inflation_ratio, out);
-            break;
-        default:
-            return (int)cudaErrorInvalidValue;
-    }
-    return (int)cudaGetLastError();
+    return for_kind(kind, [&](auto K) {
+        const auto kernel = check_config_kernel<decltype(K)::value>;
+        const cudaError_t err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn_smem);
+        if (err != cudaSuccess) return (int)err;
+        kernel<<<grid, threads, dyn_smem, (cudaStream_t)stream>>>(args, inflation_ratio, out);
+        return (int)cudaGetLastError();
+    });
 }
 
 int launch_qr_solve(double* work, const unsigned long long* offsets, const int* rows, int cols, int n, double* x_out, unsigned* flags_out,
@@ -2946,848 +2869,6 @@ int launch_qr_solve(double* work, const unsigned long long* offsets, const int* 
     if (err != cudaSuccess) return (int)err;
     const int grid = (n + warps - 1) / warps < 4096 ? (n + warps - 1) / warps : 4096;
     qr_solve_kernel<<<grid, 32 * warps, smem, (cudaStream_t)stream>>>(work, offsets, rows, cols, n, x_out, flags_out);
-    return (int)cudaGetLastError();
-}
-
-// ---------------------------------------------------------------------------------------------
-// SURVEY 8(f)-3: the first consumer of a batch, on the device.  The planner (uncertainty_planning_core.cpp:97-99) splits the
-// returned particles by did_contact and groups them by configuration distance; with these two kernels the end-state records
-// stay in HBM between ForwardSimulateRobots and that step.  Records are cfg_stride doubles + fks_result_tail.
-// ---------------------------------------------------------------------------------------------
-constexpr int kPartitionBlock = 1024;
-
-__device__ __forceinline__ bool record_in_contact(const char* results, size_t rec_stride, int cfg_stride, size_t i) {
-    return (reinterpret_cast<const fks_result_tail*>(results + i * rec_stride + (size_t)cfg_stride * 8)->flags & FKS_FLAG_DID_CONTACT) != 0u;
-}
-// pass 1: particles in contact per block of 1024 records
-__global__ void __launch_bounds__(kPartitionBlock) partition_count_kernel(const char* results, size_t rec_stride, int cfg_stride, size_t n,
-                                                                          unsigned* block_counts) {
-    const size_t i = (size_t)blockIdx.x * kPartitionBlock + threadIdx.x;
-    const int c = __syncthreads_count(i < n && record_in_contact(results, rec_stride, cfg_stride, i));
-    if (threadIdx.x == 0) block_counts[blockIdx.x] = (unsigned)c;
-}
-// pass 2 (one block): exclusive scan of the block counts in place; totals[0] = particles without contact, totals[1] = with
-__global__ void __launch_bounds__(kPartitionBlock) partition_scan_kernel(unsigned* block_counts, unsigned n_blocks, size_t n,
-                                                                         unsigned long long* totals) {
-    __shared__ unsigned warp_sums[32];
-    __shared__ unsigned carry;
-    if (threadIdx.x == 0) carry = 0u;
-    __syncthreads();
-    for (unsigned base = 0; base < n_blocks; base += kPartitionBlock) {
-        const unsigned i = base + threadIdx.x;
-        const unsigned v = i < n_blocks ? block_counts[i] : 0u;
-        unsigned incl = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const unsigned t = __shfl_up_sync(FKS_FULL, incl, o);
-            if ((threadIdx.x & 31) >= o) incl += t;
-        }
-        if ((threadIdx.x & 31) == 31) warp_sums[threadIdx.x >> 5] = incl;
-        __syncthreads();
-        if (threadIdx.x < 32) {
-            unsigned w = warp_sums[threadIdx.x];
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                const unsigned t = __shfl_up_sync(FKS_FULL, w, o);
-                if (threadIdx.x >= o) w += t;
-            }
-            warp_sums[threadIdx.x] = w;  // inclusive over warps
-        }
-        __syncthreads();
-        const unsigned before = carry + ((threadIdx.x >> 5) ? warp_sums[(threadIdx.x >> 5) - 1] : 0u) + (incl - v);
-        if (i < n_blocks) block_counts[i] = before;
-        __syncthreads();
-        if (threadIdx.x == 0) carry += warp_sums[31];
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) {
-        totals[1] = carry;
-        totals[0] = (unsigned long long)n - carry;
-    }
-}
-// pass 3: ids without contact first, ids in contact after them, ascending inside each part
-__global__ void __launch_bounds__(kPartitionBlock) partition_scatter_kernel(const char* results, size_t rec_stride, int cfg_stride, size_t n,
-                                                                            const unsigned* block_offsets, const unsigned long long* totals,
-                                                                            unsigned* order) {
-    __shared__ unsigned warp_counts[32];
-    const size_t i = (size_t)blockIdx.x * kPartitionBlock + threadIdx.x;
-    const bool valid = i < n, contact = valid && record_in_contact(results, rec_stride, cfg_stride, i);
-    const unsigned ballot = __ballot_sync(FKS_FULL, contact);
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    if (lane == 0) warp_counts[warp] = (unsigned)__popc(ballot);
-    __syncthreads();
-    unsigned before_in_block = (unsigned)__popc(ballot & ((1u << lane) - 1u));
-    for (int w = 0; w < warp; w++) before_in_block += warp_counts[w];
-    if (!valid) return;
-    const size_t contact_before = (size_t)block_offsets[blockIdx.x] + before_in_block;  // ids in contact below i
-    if (contact) order[(size_t)totals[0] + contact_before] = (unsigned)i;
-    else order[i - contact_before] = (unsigned)i;
-}
-
-// out[a * m + b] = distance from the configuration of record subset[a] to that of record subset[b] (subset == nullptr: identity)
-template <int KIND>
-__global__ void __launch_bounds__(256) pairwise_distance_kernel(const DevRobot* robot, const char* results, size_t rec_stride, int cfg_stride,
-                                                                const unsigned* subset, unsigned m, double* out) {
-    __shared__ double from[kMaxDof < 12 ? 12 : kMaxDof];
-    const unsigned a = blockIdx.y, b = blockIdx.x * blockDim.x + threadIdx.x;
-    const size_t ia = subset ? subset[a] : a;
-    if ((int)threadIdx.x < cfg_stride) from[threadIdx.x] = reinterpret_cast<const double*>(results + ia * rec_stride)[threadIdx.x];
-    __syncthreads();
-    if (b >= m) return;
-    const size_t ib = subset ? subset[b] : b;
-    out[(size_t)a * m + b] = config_distance<KIND>(*robot, from, reinterpret_cast<const double*>(results + ib * rec_stride));
-}
-
-int launch_partition(const char* results, size_t rec_stride, int cfg_stride, size_t n, unsigned* block_counts, unsigned long long* totals,
-                     unsigned* order, void* stream) {
-    const unsigned n_blocks = (unsigned)((n + kPartitionBlock - 1) / kPartitionBlock);
-    cudaStream_t st = (cudaStream_t)stream;
-    partition_count_kernel<<<n_blocks, kPartitionBlock, 0, st>>>(results, rec_stride, cfg_stride, n, block_counts);
-    partition_scan_kernel<<<1, kPartitionBlock, 0, st>>>(block_counts, n_blocks, n, totals);
-    partition_scatter_kernel<<<n_blocks, kPartitionBlock, 0, st>>>(results, rec_stride, cfg_stride, n, block_counts, totals, order);
-    return (int)cudaGetLastError();
-}
-int launch_pairwise_distance(int kind, const DevRobot* robot, const char* results, size_t rec_stride, int cfg_stride, const unsigned* subset,
-                             unsigned m, double* out, void* stream) {
-    const dim3 grid((m + 255) / 256, m);
-    cudaStream_t st = (cudaStream_t)stream;
-    switch (kind) {
-        case FKS_ROBOT_SE2: pairwise_distance_kernel<FKS_ROBOT_SE2><<<grid, 256, 0, st>>>(robot, results, rec_stride, cfg_stride, subset, m, out); break;
-        case FKS_ROBOT_SE3: pairwise_distance_kernel<FKS_ROBOT_SE3><<<grid, 256, 0, st>>>(robot, results, rec_stride, cfg_stride, subset, m, out); break;
-        case FKS_ROBOT_LINKED: pairwise_distance_kernel<FKS_ROBOT_LINKED><<<grid, 256, 0, st>>>(robot, results, rec_stride, cfg_stride, subset, m, out); break;
-        default: return (int)cudaErrorInvalidValue;
-    }
-    return (int)cudaGetLastError();
-}
-
-// ---------------------------------------------------------------------------------------------
-// fks_end_states_cluster: flat agglomerative clustering (single / complete linkage, distance cutoff) of every segment of a
-// position range, one CTA per segment.  A segment's distances form the upper triangle of an n x n matrix D (row pitch n):
-// D[p][q], p < q, is the pairwise kernel's entry [p][q] for the same records, +inf where that is NaN or the contact flags
-// differ under separate_contact.  Small segments keep D in shared memory, large ones in a global slot of the CTA.
-//
-// Merge loop.  A cluster is named by its smallest position (its representative); only representatives' rows and columns of D
-// are finite, the others are +inf.  nn[i] / nnd[i] cache the smallest (D[i][j], j) over j > i, so the smallest
-// (nnd[i], i, nn[i]) over i is the smallest merge key (L, min rep, max rep).  Merging a < b writes op(D[a][k], D[b][k]) into
-// a's row and column (op = min for single, max for complete linkage: the Lance-Williams update of the two, exact), sets b's
-// to +inf, and repairs the cache: row a is rescanned, so is every row whose neighbour was a or b (b is gone; under complete
-// linkage a's distances grew), and a row i < a with another neighbour only compares its cache with the new D[i][a] -- under
-// single linkage it can only have shrunk, under complete linkage it grew from a value that already lost.
-// ---------------------------------------------------------------------------------------------
-constexpr int kClusterSmallBlock = 256;
-constexpr int kClusterLargeBlock = 1024;
-
-struct ClusterArgs {
-    const DevRobot* robot;
-    const char* results;
-    size_t rec_stride;
-    int cfg_stride;
-    int complete;
-    int separate_contact;
-    double threshold;
-    const unsigned* order;                // position -> record id, or null (identity)
-    const unsigned long long* offsets;    // [n_segments + 1]
-    const unsigned* segs;                 // segment ids this launch clusters
-    unsigned n_segs;
-    unsigned n_cap;                       // largest segment of this launch
-    double* work;                         // large path: one n_cap x n_cap slot per CTA
-    unsigned* labels;                     // [m]: segment-local cluster ids (the relabel kernel adds the segment's base)
-    unsigned* counts;                     // [n_segments]: clusters per segment
-};
-
-// per-segment state in shared memory behind the matrix (small path) or at the start of it (large path)
-struct ClusterSmem {
-    unsigned* rep;   // [n_cap] representative of each position
-    unsigned* nn;    // [n_cap] cached nearest j > i (n = none), reused for the ranks of the representatives at the end
-    double* nnd;     // [n_cap] D[i][nn[i]]
-    unsigned* list;  // [n_cap] rows to rescan
-};
-__host__ __device__ inline size_t cluster_state_bytes(unsigned n_cap) { return (size_t)n_cap * (8 + 4 + 4 + 4); }
-
-struct ClusterShared {
-    double wd[32];
-    unsigned wi[32];
-    unsigned a, b, go, n_list, carry;
-};
-
-__device__ __forceinline__ bool cluster_key_less(double d, unsigned i, double e, unsigned j) { return d < e || (d == e && i < j); }
-
-// (d, i) of the warp's smallest key, in every lane
-__device__ __forceinline__ void cluster_warp_min(double& d, unsigned& i) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        const double od = __shfl_xor_sync(FKS_FULL, d, o);
-        const unsigned oi = __shfl_xor_sync(FKS_FULL, i, o);
-        if (cluster_key_less(od, oi, d, i)) {
-            d = od;
-            i = oi;
-        }
-    }
-}
-
-// one warp: nn[i] / nnd[i] = smallest (D[i][j], j) over j > i (none: n / +inf)
-__device__ __forceinline__ void cluster_rescan_row(const double* D, unsigned n, unsigned i, ClusterSmem& st) {
-    const int lane = threadIdx.x & 31;
-    const double* row = D + (size_t)i * n;
-    double bd = INFINITY;
-    unsigned bj = n;
-    for (unsigned j = i + 1 + lane; j < n; j += 32) {
-        const double d = row[j];
-        if (d < bd) {
-            bd = d;
-            bj = j;
-        }
-    }
-    cluster_warp_min(bd, bj);
-    if (lane == 0) {
-        st.nn[i] = bj;
-        st.nnd[i] = bd;
-    }
-}
-
-template <int KIND>
-__device__ void cluster_segment(const ClusterArgs& a, unsigned s, double* D, ClusterSmem& st, ClusterShared& sh) {
-    const unsigned begin = (unsigned)a.offsets[s], n = (unsigned)(a.offsets[s + 1] - a.offsets[s]);
-    const unsigned tid = threadIdx.x, nt = blockDim.x, lane = tid & 31, warp = tid >> 5, n_warps = nt >> 5;
-    // distances, upper triangle, one warp per row: the operands and the inlined config_distance of pairwise_distance_kernel,
-    // so the same bits
-    for (unsigned p = warp; p < n; p += n_warps) {
-        const size_t ip = a.order ? a.order[begin + p] : begin + p;
-        const double* from = reinterpret_cast<const double*>(a.results + ip * a.rec_stride);
-        const bool from_contact = record_in_contact(a.results, a.rec_stride, a.cfg_stride, ip);
-        for (unsigned q = p + 1 + lane; q < n; q += 32) {
-            const size_t iq = a.order ? a.order[begin + q] : begin + q;
-            double d = config_distance<KIND>(*a.robot, from, reinterpret_cast<const double*>(a.results + iq * a.rec_stride));
-            if (isnan(d) || (a.separate_contact && record_in_contact(a.results, a.rec_stride, a.cfg_stride, iq) != from_contact)) d = INFINITY;
-            D[(size_t)p * n + q] = d;
-        }
-    }
-    for (unsigned p = tid; p < n; p += nt) st.rep[p] = p;
-    __syncthreads();
-    for (unsigned i = warp; i < n; i += n_warps) cluster_rescan_row(D, n, i, st);
-    __syncthreads();
-
-    unsigned merges = 0;
-    for (;;) {
-        // smallest (nnd[i], i)
-        double bd = INFINITY;
-        unsigned bi = n;
-        for (unsigned i = tid; i < n; i += nt) {
-            const double d = st.nnd[i];
-            if (d < bd) {
-                bd = d;
-                bi = i;
-            }
-        }
-        cluster_warp_min(bd, bi);
-        if (lane == 0) {
-            sh.wd[warp] = bd;
-            sh.wi[warp] = bi;
-        }
-        __syncthreads();
-        if (warp == 0) {
-            bd = lane < n_warps ? sh.wd[lane] : INFINITY;
-            bi = lane < n_warps ? sh.wi[lane] : n;
-            cluster_warp_min(bd, bi);
-            if (lane == 0) {
-                sh.go = bd < INFINITY && bd <= a.threshold;
-                sh.a = bi;
-                sh.b = sh.go ? st.nn[bi] : 0u;
-                sh.n_list = 0;
-            }
-        }
-        __syncthreads();
-        if (!sh.go) break;
-        const unsigned ca = sh.a, cb = sh.b;
-        merges++;
-        // row / column a <- op(a, b); b -> +inf; b's members join a
-        for (unsigned k = tid; k < n; k += nt) {
-            if (st.rep[k] == cb) st.rep[k] = ca;
-            if (k == ca) continue;
-            const size_t bk = k < cb ? (size_t)k * n + cb : (size_t)cb * n + k;
-            if (k == cb) {
-                D[(size_t)ca * n + cb] = INFINITY;
-                continue;
-            }
-            const size_t ak = k < ca ? (size_t)k * n + ca : (size_t)ca * n + k;
-            const double x = D[ak], y = D[bk];
-            D[ak] = a.complete ? fmax(x, y) : fmin(x, y);
-            D[bk] = INFINITY;
-        }
-        __syncthreads();
-        // cache repair (rows of merged-away positions are all +inf and stay out of the argmin through nnd = +inf)
-        for (unsigned i = tid; i < n; i += nt) {
-            if (i == cb) {
-                st.nnd[i] = INFINITY;
-                st.nn[i] = n;
-                continue;
-            }
-            if (st.rep[i] != i) continue;
-            const unsigned j = st.nn[i];
-            bool rescan = i == ca || j == cb;
-            if (i < ca && !rescan) {
-                if (j == ca) {
-                    rescan = true;
-                } else {
-                    const double d = D[(size_t)i * n + ca];
-                    if (cluster_key_less(d, ca, st.nnd[i], j)) {
-                        st.nnd[i] = d;
-                        st.nn[i] = ca;
-                    }
-                }
-            }
-            if (rescan) st.list[atomicAdd(&sh.n_list, 1u)] = i;
-        }
-        __syncthreads();
-        for (unsigned r = warp; r < sh.n_list; r += n_warps) cluster_rescan_row(D, n, st.list[r], st);
-        __syncthreads();
-    }
-
-    // dense ids in representative order: exclusive count of representatives below each position
-    if (tid == 0) sh.carry = 0;
-    __syncthreads();
-    for (unsigned base = 0; base < n; base += nt) {
-        const unsigned p = base + tid;
-        const bool is_rep = p < n && st.rep[p] == p;
-        const unsigned ballot = __ballot_sync(FKS_FULL, is_rep);
-        if (lane == 0) sh.wi[warp] = (unsigned)__popc(ballot);
-        __syncthreads();
-        unsigned before = sh.carry + (unsigned)__popc(ballot & ((1u << lane) - 1u));
-        for (unsigned w = 0; w < warp; w++) before += sh.wi[w];
-        if (p < n) st.nn[p] = before;
-        __syncthreads();
-        if (tid == 0)
-            for (unsigned w = 0; w < n_warps; w++) sh.carry += sh.wi[w];
-        __syncthreads();
-    }
-    for (unsigned p = tid; p < n; p += nt) a.labels[begin + p] = st.nn[st.rep[p]];
-    if (tid == 0) a.counts[s] = n - merges;
-    __syncthreads();  // the next segment reuses the shared state
-}
-
-// segments of at most kClusterSmallMax positions: D, then the per-position state, in dynamic shared memory
-template <int KIND>
-__global__ void __launch_bounds__(kClusterSmallBlock) cluster_small_kernel(ClusterArgs a) {
-    extern __shared__ __align__(16) unsigned char cluster_smem[];
-    __shared__ ClusterShared sh;
-    double* D = reinterpret_cast<double*>(cluster_smem);
-    const unsigned n_cap = a.n_cap;
-    ClusterSmem st;
-    st.nnd = D + (size_t)n_cap * n_cap;
-    st.rep = reinterpret_cast<unsigned*>(st.nnd + n_cap);
-    st.nn = st.rep + n_cap;
-    st.list = st.nn + n_cap;
-    for (unsigned t = blockIdx.x; t < a.n_segs; t += gridDim.x) cluster_segment<KIND>(a, a.segs[t], D, st, sh);
-}
-
-// larger segments: D in the CTA's slot of the global workspace, the per-position state in dynamic shared memory
-template <int KIND>
-__global__ void __launch_bounds__(kClusterLargeBlock) cluster_large_kernel(ClusterArgs a) {
-    extern __shared__ __align__(16) unsigned char cluster_smem[];
-    __shared__ ClusterShared sh;
-    const unsigned n_cap = a.n_cap;
-    double* D = a.work + (size_t)blockIdx.x * n_cap * n_cap;
-    ClusterSmem st;
-    st.nnd = reinterpret_cast<double*>(cluster_smem);
-    st.rep = reinterpret_cast<unsigned*>(st.nnd + n_cap);
-    st.nn = st.rep + n_cap;
-    st.list = st.nn + n_cap;
-    for (unsigned t = blockIdx.x; t < a.n_segs; t += gridDim.x) cluster_segment<KIND>(a, a.segs[t], D, st, sh);
-}
-
-// labels of segment s += the clusters of the segments before it (exclusive scan of the counts)
-__global__ void __launch_bounds__(256) cluster_relabel_kernel(const unsigned long long* offsets, unsigned n_segments, const unsigned* base,
-                                                              unsigned* labels) {
-    for (unsigned s = blockIdx.x; s < n_segments; s += gridDim.x) {
-        const unsigned add = base[s];
-        for (unsigned long long p = offsets[s] + threadIdx.x; p < offsets[s + 1]; p += blockDim.x) labels[p] += add;
-    }
-}
-
-size_t cluster_small_smem(unsigned n_cap) { return (size_t)n_cap * n_cap * 8 + cluster_state_bytes(n_cap); }
-
-template <typename Kernel>
-static int cluster_launch(Kernel k, const ClusterArgs& a, int block, size_t smem, int max_grid, void* stream) {
-    if (a.n_segs == 0) return 0;
-    cudaError_t err = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (err != cudaSuccess) return (int)err;
-    int per_sm = 0;
-    err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, block, smem);
-    if (err != cudaSuccess) return (int)err;
-    int dev = 0, sms = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    long long grid = (long long)(per_sm > 0 ? per_sm : 1) * sms;
-    if (grid > (long long)a.n_segs) grid = a.n_segs;
-    if (max_grid > 0 && grid > max_grid) grid = max_grid;
-    k<<<(unsigned)grid, block, smem, (cudaStream_t)stream>>>(a);
-    return (int)cudaGetLastError();
-}
-
-int launch_cluster(int kind, const ClusterLaunch& c, void* stream) {
-    ClusterArgs a;
-    a.robot = c.robot;
-    a.results = c.results;
-    a.rec_stride = c.rec_stride;
-    a.cfg_stride = c.cfg_stride;
-    a.complete = c.complete;
-    a.separate_contact = c.separate_contact;
-    a.threshold = c.threshold;
-    a.order = c.order;
-    a.offsets = c.offsets;
-    a.labels = c.labels;
-    a.counts = c.counts;
-    cudaStream_t st = (cudaStream_t)stream;
-    int rc = 0;
-    ClusterArgs sm = a, lg = a;
-    sm.segs = c.small_segs;
-    sm.n_segs = c.n_small;
-    sm.n_cap = c.small_cap;
-    sm.work = nullptr;
-    lg.segs = c.large_segs;
-    lg.n_segs = c.n_large;
-    lg.n_cap = c.large_cap;
-    lg.work = c.work;
-    const size_t small_smem = cluster_small_smem(c.small_cap), large_smem = cluster_state_bytes(c.large_cap);
-    switch (kind) {
-        case FKS_ROBOT_SE2:
-            if ((rc = cluster_launch(cluster_small_kernel<FKS_ROBOT_SE2>, sm, kClusterSmallBlock, small_smem, 0, stream)) != 0) return rc;
-            if ((rc = cluster_launch(cluster_large_kernel<FKS_ROBOT_SE2>, lg, kClusterLargeBlock, large_smem, c.large_slots, stream)) != 0) return rc;
-            break;
-        case FKS_ROBOT_SE3:
-            if ((rc = cluster_launch(cluster_small_kernel<FKS_ROBOT_SE3>, sm, kClusterSmallBlock, small_smem, 0, stream)) != 0) return rc;
-            if ((rc = cluster_launch(cluster_large_kernel<FKS_ROBOT_SE3>, lg, kClusterLargeBlock, large_smem, c.large_slots, stream)) != 0) return rc;
-            break;
-        case FKS_ROBOT_LINKED:
-            if ((rc = cluster_launch(cluster_small_kernel<FKS_ROBOT_LINKED>, sm, kClusterSmallBlock, small_smem, 0, stream)) != 0) return rc;
-            if ((rc = cluster_launch(cluster_large_kernel<FKS_ROBOT_LINKED>, lg, kClusterLargeBlock, large_smem, c.large_slots, stream)) != 0) return rc;
-            break;
-        default: return (int)cudaErrorInvalidValue;
-    }
-    // base of every segment's ids: partition's exclusive scan, in place over the counts (totals[1] = all clusters)
-    partition_scan_kernel<<<1, kPartitionBlock, 0, st>>>(c.counts, c.n_segments, 0, c.totals);
-    const unsigned relabel_grid = c.n_segments < 65535u ? c.n_segments : 65535u;
-    cluster_relabel_kernel<<<relabel_grid, 256, 0, st>>>(c.offsets, c.n_segments, c.counts, c.labels);
-    return (int)cudaGetLastError();
-}
-
-// ---------------------------------------------------------------------------------------------
-// fks_end_states_groups: the clusters of a labelled position range as particle groups.  Members: a stable counting sort by
-// label -- count, the partition's one-block scan, a scatter in arrival order, then each group sorted by position in shared
-// memory, so the result does not depend on the order of the scatter's atomics.  Representative: the member with the smallest
-// (r, position), r(p) = max over the other members q of d(min(p,q), max(p,q)), d = the pairwise kernel's entry (same
-// inlined config_distance, same operands), NaN as +inf.  Every pair is evaluated in both rows, so a row's maximum is a plain
-// warp reduction; max over non-NaN values and the (r, position) argmin are exact in any order, so every result is.
-// ---------------------------------------------------------------------------------------------
-constexpr int kGroupBlock = 256;
-constexpr unsigned kGroupWarps = kGroupBlock / 32;
-constexpr unsigned kGroupRowsPerTask = 32;  // rows of a large cluster per task of the row pass
-
-// pass 1: members per label into offsets[0 .. n_clusters) (zeroed), error bit for labels out of range
-__global__ void __launch_bounds__(kGroupBlock) groups_count_kernel(const unsigned* labels, unsigned m, unsigned n_clusters, unsigned* counts,
-                                                                   unsigned* state) {
-    for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < m; p += (size_t)gridDim.x * blockDim.x) {
-        const unsigned l = labels[p];
-        if (l < n_clusters) atomicAdd(&counts[l], 1u);
-        else atomicOr(&state[1], kGroupErrLabel);
-    }
-}
-
-// pass 3 (after the scan): positions into their group's range in arrival order; offsets[n_clusters] = positions with a valid label
-__global__ void __launch_bounds__(kGroupBlock) groups_scatter_kernel(const unsigned* labels, unsigned m, unsigned n_clusters, unsigned* offsets,
-                                                                     const unsigned long long* totals, unsigned* cursor, unsigned* members) {
-    if (blockIdx.x == 0 && threadIdx.x == 0) offsets[n_clusters] = (unsigned)totals[1];
-    for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < m; p += (size_t)gridDim.x * blockDim.x) {
-        const unsigned l = labels[p];
-        if (l < n_clusters) members[offsets[l] + atomicAdd(&cursor[l], 1u)] = (unsigned)p;
-    }
-}
-
-// one warp: r of member i of a group whose record ids are ids[0 .. k), in position order (every lane gets it)
-template <int KIND>
-__device__ __forceinline__ double group_row_max(const GroupsLaunch& g, const unsigned* ids, unsigned k, unsigned i) {
-    const unsigned lane = threadIdx.x & 31;
-    const double* rec_i = reinterpret_cast<const double*>(g.results + (size_t)ids[i] * g.rec_stride);
-    double r = -INFINITY;
-    for (unsigned j = lane; j < k; j += 32) {
-        if (j == i) continue;
-        const double* rec_j = reinterpret_cast<const double*>(g.results + (size_t)ids[j] * g.rec_stride);
-        double d = config_distance<KIND>(*g.robot, j > i ? rec_i : rec_j, j > i ? rec_j : rec_i);
-        if (isnan(d)) d = INFINITY;
-        if (d > r) r = d;
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        const double x = __shfl_xor_sync(FKS_FULL, r, o);
-        if (x > r) r = x;
-    }
-    return k == 1 ? 0.0 : r;
-}
-
-// the CTA's smallest (d, i) over its warps' (lane-uniform) candidates, in thread 0
-__device__ __forceinline__ void group_block_min(double& d, unsigned& i, double* wd, unsigned* wi) {
-    const unsigned lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (lane == 0) {
-        wd[warp] = d;
-        wi[warp] = i;
-    }
-    __syncthreads();
-    if (warp == 0) {
-        d = lane < kGroupWarps ? wd[lane] : INFINITY;
-        i = lane < kGroupWarps ? wi[lane] : 0xffffffffu;
-        cluster_warp_min(d, i);
-    }
-}
-
-// pass 4, one CTA per group: check its size, sort its positions (bitonic, padded to a power of two), write its record ids;
-// groups of up to kGroupSmallMax members get their representative here, larger ones go on the list of the row pass
-template <int KIND>
-__global__ void __launch_bounds__(kGroupBlock) groups_sort_small_kernel(GroupsLaunch g) {
-    __shared__ unsigned key[kClusterMaxSegment];
-    __shared__ double wd[kGroupWarps];
-    __shared__ unsigned wi[kGroupWarps];
-    const unsigned tid = threadIdx.x, warp = tid >> 5;
-    for (unsigned c = blockIdx.x; c < g.n_clusters; c += gridDim.x) {
-        const unsigned begin = g.offsets[c], k = g.offsets[c + 1] - begin;
-        if (k == 0 || k > kClusterMaxSegment) {
-            if (tid == 0) atomicOr(&g.state[1], k == 0 ? kGroupErrEmpty : kGroupErrLarge);
-            continue;
-        }
-        unsigned n2 = 1;
-        while (n2 < k) n2 <<= 1;
-        for (unsigned i = tid; i < n2; i += kGroupBlock) key[i] = i < k ? g.members[begin + i] : 0xffffffffu;
-        __syncthreads();
-        for (unsigned size = 2; size <= n2; size <<= 1) {
-            for (unsigned stride = size >> 1; stride > 0; stride >>= 1) {
-                for (unsigned t = tid; t < n2 / 2; t += kGroupBlock) {
-                    const unsigned i = 2 * stride * (t / stride) + t % stride, j = i + stride;
-                    const unsigned x = key[i], y = key[j];
-                    if ((x > y) == ((i & size) == 0)) {
-                        key[i] = y;
-                        key[j] = x;
-                    }
-                }
-                __syncthreads();
-            }
-        }
-        for (unsigned i = tid; i < k; i += kGroupBlock) {
-            const unsigned id = g.order ? g.order[key[i]] : key[i];
-            key[i] = id;
-            g.members[begin + i] = id;
-        }
-        __syncthreads();
-        if (k > kGroupSmallMax) {
-            if (tid == 0) g.state[2 + atomicAdd(&g.state[0], 1u)] = c;
-            continue;
-        }
-        double bd = INFINITY;
-        unsigned bi = k;
-        for (unsigned i = warp; i < k; i += kGroupWarps) {
-            const double r = group_row_max<KIND>(g, key, k, i);
-            if (cluster_key_less(r, i, bd, bi)) {
-                bd = r;
-                bi = i;
-            }
-        }
-        group_block_min(bd, bi, wd, wi);
-        if (tid == 0) {
-            g.reps[c] = key[bi];
-            g.radius[c] = bd;
-        }
-        __syncthreads();  // the next group reuses key, wd, wi
-    }
-}
-
-// pass 5: r of every member of the listed groups.  Group e's rows form tasks of kGroupRowsPerTask rows, numbered on from the
-// tasks of the groups before it; task T goes to CTA T mod gridDim.x.
-template <int KIND>
-__global__ void __launch_bounds__(kGroupBlock) groups_large_rows_kernel(GroupsLaunch g) {
-    const unsigned n_large = g.state[0], warp = threadIdx.x >> 5, lane = threadIdx.x & 31, G = gridDim.x;
-    unsigned shift = 0;  // (tasks of the groups before e) mod G
-    for (unsigned e = 0; e < n_large; e++) {
-        const unsigned c = g.state[2 + e], begin = g.offsets[c], k = g.offsets[c + 1] - begin;
-        const unsigned n_tasks = (k + kGroupRowsPerTask - 1) / kGroupRowsPerTask;
-        for (unsigned t = (blockIdx.x + G - shift) % G; t < n_tasks; t += G) {
-            const unsigned end = min(k, (t + 1) * kGroupRowsPerTask);
-            for (unsigned i = t * kGroupRowsPerTask + warp; i < end; i += kGroupWarps) {
-                const double r = group_row_max<KIND>(g, g.members + begin, k, i);
-                if (lane == 0) g.row_max[begin + i] = r;
-            }
-        }
-        shift = (shift + n_tasks) % G;
-    }
-}
-
-// pass 6: one CTA per listed group, the smallest (r, position)
-__global__ void __launch_bounds__(kGroupBlock) groups_large_argmin_kernel(GroupsLaunch g) {
-    __shared__ double wd[kGroupWarps];
-    __shared__ unsigned wi[kGroupWarps];
-    const unsigned n_large = g.state[0];
-    for (unsigned e = blockIdx.x; e < n_large; e += gridDim.x) {
-        const unsigned c = g.state[2 + e], begin = g.offsets[c], k = g.offsets[c + 1] - begin;
-        double bd = INFINITY;
-        unsigned bi = k;
-        for (unsigned i = threadIdx.x; i < k; i += kGroupBlock) {
-            const double r = g.row_max[begin + i];
-            if (cluster_key_less(r, i, bd, bi)) {
-                bd = r;
-                bi = i;
-            }
-        }
-        cluster_warp_min(bd, bi);
-        group_block_min(bd, bi, wd, wi);
-        if (threadIdx.x == 0) {
-            g.reps[c] = g.members[begin + bi];
-            g.radius[c] = bd;
-        }
-        __syncthreads();
-    }
-}
-
-template <typename Kernel>
-static unsigned groups_resident_ctas(Kernel k) {
-    int per_sm = 0, dev = 0, sms = 0;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, kGroupBlock, 0);
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    return (unsigned)((per_sm > 0 ? per_sm : 1) * (sms > 0 ? sms : 1));
-}
-
-template <int KIND>
-static void groups_search(const GroupsLaunch& g, cudaStream_t st) {
-    // the host does not know how many groups are large: the row and argmin passes run a full grid and read the list
-    const unsigned resident = groups_resident_ctas(groups_sort_small_kernel<KIND>);
-    const unsigned rows_grid = groups_resident_ctas(groups_large_rows_kernel<KIND>);
-    groups_sort_small_kernel<KIND><<<g.n_clusters < resident ? g.n_clusters : resident, kGroupBlock, 0, st>>>(g);
-    groups_large_rows_kernel<KIND><<<rows_grid, kGroupBlock, 0, st>>>(g);
-    groups_large_argmin_kernel<<<rows_grid, kGroupBlock, 0, st>>>(g);
-}
-
-int launch_groups(int kind, const GroupsLaunch& g, void* stream) {
-    if (g.m == 0 || g.n_clusters == 0) return (int)cudaErrorInvalidValue;
-    void (*search)(const GroupsLaunch&, cudaStream_t);
-    switch (kind) {
-        case FKS_ROBOT_SE2: search = groups_search<FKS_ROBOT_SE2>; break;
-        case FKS_ROBOT_SE3: search = groups_search<FKS_ROBOT_SE3>; break;
-        case FKS_ROBOT_LINKED: search = groups_search<FKS_ROBOT_LINKED>; break;
-        default: return (int)cudaErrorInvalidValue;
-    }
-    cudaStream_t st = (cudaStream_t)stream;
-    const size_t blocks = ((size_t)g.m + kGroupBlock - 1) / kGroupBlock;
-    const unsigned grid = blocks < 65535 ? (unsigned)blocks : 65535u;
-    groups_count_kernel<<<grid, kGroupBlock, 0, st>>>(g.labels, g.m, g.n_clusters, g.offsets, g.state);
-    partition_scan_kernel<<<1, kPartitionBlock, 0, st>>>(g.offsets, g.n_clusters, g.m, g.totals);
-    groups_scatter_kernel<<<grid, kGroupBlock, 0, st>>>(g.labels, g.m, g.n_clusters, g.offsets, g.totals, g.cursor, g.members);
-    search(g, st);
-    return (int)cudaGetLastError();
-}
-
-// fks_end_states_gather_starts: value v of the outputs is component v mod cfg_stride of slot v / cfg_stride
-__global__ void __launch_bounds__(256) gather_starts_kernel(const char* results, size_t rec_stride, int cfg_stride, const unsigned* offsets,
-                                                            const unsigned* members, const unsigned* selected, unsigned per_group,
-                                                            size_t n_values, const double* group_targets, double* starts, double* targets) {
-    for (size_t v = (size_t)blockIdx.x * blockDim.x + threadIdx.x; v < n_values; v += (size_t)gridDim.x * blockDim.x) {
-        const unsigned slot = (unsigned)(v / (unsigned)cfg_stride), t = (unsigned)(v % (unsigned)cfg_stride);
-        const unsigned s = slot / per_group, j = slot % per_group;
-        const unsigned g = selected[s], begin = offsets[g], k = offsets[g + 1] - begin;
-        starts[v] = k ? reinterpret_cast<const double*>(results + (size_t)members[begin + j % k] * rec_stride)[t] : NAN;
-        if (targets) targets[v] = group_targets[(size_t)s * cfg_stride + t];
-    }
-}
-
-int launch_gather_starts(const char* results, size_t rec_stride, int cfg_stride, const unsigned* offsets, const unsigned* members,
-                         const unsigned* selected, unsigned n_selected, unsigned per_group, const double* group_targets, double* starts,
-                         double* targets, void* stream) {
-    const size_t n_values = (size_t)n_selected * per_group * (size_t)cfg_stride;
-    const size_t grid = (n_values + 255) / 256 < 65535 ? (n_values + 255) / 256 : 65535;
-    gather_starts_kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(results, rec_stride, cfg_stride, offsets, members, selected, per_group,
-                                                                            n_values, group_targets, starts, targets);
-    return (int)cudaGetLastError();
-}
-
-// ---------------------------------------------------------------------------------------------
-// fks_nearest_configurations: per query the k smallest keys (d, i), d = config_distance<KIND>(candidate i, query) -- the
-// pairwise kernel's inlined distance with the candidate as `cur`, as in its entry [i][m + j] -- NaN as +inf.  A warp keeps a
-// query's running list sorted by key over 64 positions, position p in lane p mod 32 (slot p / 32); a key enters only if it
-// is below the one at position k - 1.  Keys are a total order, so the k smallest of a union are the k smallest of the parts'
-// k smallest: any split of the candidates and any merge order give the same bits.
-// ---------------------------------------------------------------------------------------------
-constexpr int kNearestBlock = 256;
-constexpr unsigned kNearestWarps = kNearestBlock / 32;  // queries per CTA of the scan
-constexpr unsigned kNearestTileDoubles = 4096;          // the candidate tile in shared memory (32 KiB)
-constexpr int kNearestCfgMax = kMaxDof < 12 ? 12 : kMaxDof;
-constexpr unsigned kNearestCtasPerSm = 4;     // the scan's grid the split aims at
-constexpr unsigned kNearestMinChunk = 2048;   // fewest candidates per chunk of a split
-
-struct NearestList {
-    double d0, d1;    // keys at positions lane, 32 + lane
-    unsigned i0, i1;
-};
-
-struct NearestShared {
-    double d[kNearestWarps][kNearestMaxK];
-    unsigned i[kNearestWarps][kNearestMaxK];
-};
-
-__device__ __forceinline__ void nearest_list_init(NearestList& L, double& kd, unsigned& ki) {
-    L.d0 = L.d1 = kd = INFINITY;
-    L.i0 = L.i1 = ki = 0xffffffffu;
-}
-
-// (d, i), the same in every lane, goes to its rank; the key at position 63 drops out.  kd / ki = the key at position k - 1.
-__device__ __forceinline__ void nearest_insert(NearestList& L, unsigned k, double& kd, unsigned& ki, double d, unsigned i) {
-    const unsigned lane = threadIdx.x & 31;
-    const unsigned pos = __popc(__ballot_sync(FKS_FULL, cluster_key_less(L.d0, L.i0, d, i))) +
-                         __popc(__ballot_sync(FKS_FULL, cluster_key_less(L.d1, L.i1, d, i)));
-    const double up_d0 = __shfl_up_sync(FKS_FULL, L.d0, 1), last_d0 = __shfl_sync(FKS_FULL, L.d0, 31);
-    const unsigned up_i0 = __shfl_up_sync(FKS_FULL, L.i0, 1), last_i0 = __shfl_sync(FKS_FULL, L.i0, 31);
-    double up_d1 = __shfl_up_sync(FKS_FULL, L.d1, 1);
-    unsigned up_i1 = __shfl_up_sync(FKS_FULL, L.i1, 1);
-    if (lane == 0) {
-        up_d1 = last_d0;
-        up_i1 = last_i0;
-    }
-    if (lane == pos) {
-        L.d0 = d;
-        L.i0 = i;
-    } else if (lane > pos) {
-        L.d0 = up_d0;
-        L.i0 = up_i0;
-    }
-    if (lane + 32 == pos) {
-        L.d1 = d;
-        L.i1 = i;
-    } else if (lane + 32 > pos) {
-        L.d1 = up_d1;
-        L.i1 = up_i1;
-    }
-    kd = __shfl_sync(FKS_FULL, k > 32 ? L.d1 : L.d0, (k - 1) & 31);
-    ki = __shfl_sync(FKS_FULL, k > 32 ? L.i1 : L.i0, (k - 1) & 31);
-}
-
-// every lane offers one key; those below the k-th enter in lane order (invalid lanes offer (+inf, 0xffffffff))
-__device__ __forceinline__ void nearest_offer(NearestList& L, unsigned k, double& kd, unsigned& ki, double d, unsigned i) {
-    unsigned mask = __ballot_sync(FKS_FULL, cluster_key_less(d, i, kd, ki));
-    while (mask) {
-        const int src = __ffs(mask) - 1;
-        mask &= mask - 1;
-        const double bd = __shfl_sync(FKS_FULL, d, src);
-        const unsigned bi = __shfl_sync(FKS_FULL, i, src);
-        if (cluster_key_less(bd, bi, kd, ki)) nearest_insert(L, k, kd, ki, bd, bi);
-    }
-}
-
-// the first k keys of a stored list
-__device__ __forceinline__ void nearest_offer_list(NearestList& L, unsigned k, double& kd, unsigned& ki, const double* d, const unsigned* id) {
-    const unsigned lane = threadIdx.x & 31;
-    for (unsigned p0 = 0; p0 < k; p0 += 32) {
-        const unsigned p = p0 + lane;
-        nearest_offer(L, k, kd, ki, p < k ? d[p] : INFINITY, p < k ? id[p] : 0xffffffffu);
-    }
-}
-
-__device__ __forceinline__ void nearest_store(const NearestList& L, unsigned k, double* d, unsigned* id) {
-    const unsigned lane = threadIdx.x & 31;
-    if (lane < k) {
-        d[lane] = L.d0;
-        id[lane] = L.i0;
-    }
-    if (lane + 32 < k) {
-        d[lane + 32] = L.d1;
-        id[lane + 32] = L.i1;
-    }
-}
-
-// warps q + s * n_lists, 0 < s < per, hand their lists to warp q through shared memory (per is the same in the whole CTA)
-__device__ __forceinline__ void nearest_block_merge(NearestList& L, unsigned k, double& kd, unsigned& ki, unsigned n_lists, unsigned per,
-                                                    NearestShared& sh) {
-    const unsigned warp = threadIdx.x >> 5;
-    if (per == 1) return;
-    if (warp >= n_lists && warp < n_lists * per) nearest_store(L, k, sh.d[warp], sh.i[warp]);
-    __syncthreads();
-    if (warp < n_lists)
-        for (unsigned s = 1; s < per; s++) nearest_offer_list(L, k, kd, ki, sh.d[warp + s * n_lists], sh.i[warp + s * n_lists]);
-}
-
-// CTA (x, y): queries 8x .. 8x + qt - 1 against chunk y of the candidates, streamed through shared memory in coalesced tiles.
-// With qt < 8 queries, per = 8 / qt warps share a query, each taking every per-th group of 32 candidates of a tile.
-template <int KIND>
-__global__ void __launch_bounds__(kNearestBlock) nearest_scan_kernel(NearestLaunch a) {
-    __shared__ double cand[kNearestTileDoubles];
-    __shared__ double qry[kNearestWarps * kNearestCfgMax];
-    __shared__ NearestShared sh;
-    const unsigned tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, S = (unsigned)a.cfg_stride;
-    const unsigned q0 = blockIdx.x * kNearestWarps, qt = min(kNearestWarps, a.n_queries - q0), per = kNearestWarps / qt;
-    const unsigned qi = warp % qt, sub = warp / qt;
-    for (unsigned t = tid; t < qt * S; t += kNearestBlock) qry[t] = a.queries[(size_t)q0 * S + t];
-    const unsigned c_begin = blockIdx.y * a.chunk, c_end = (unsigned)min((size_t)a.m, (size_t)c_begin + a.chunk), tile = kNearestTileDoubles / S;
-    NearestList L;
-    double kd;
-    unsigned ki;
-    nearest_list_init(L, kd, ki);
-    for (unsigned c0 = c_begin, n; c0 < c_end; c0 += n) {
-        n = min(tile, c_end - c0);
-        __syncthreads();  // the previous tile is consumed (and the queries are in place)
-        const double* src = a.candidates + (size_t)c0 * S;
-        for (unsigned t = tid; t < n * S; t += kNearestBlock) cand[t] = src[t];
-        __syncthreads();
-        if (sub >= per) continue;
-        for (unsigned b = sub * 32; b < n; b += 32 * per) {
-            const unsigned c = b + lane;
-            double d = INFINITY;
-            unsigned id = 0xffffffffu;
-            if (c < n) {
-                d = config_distance<KIND>(*a.robot, cand + c * S, qry + qi * S);
-                if (isnan(d)) d = INFINITY;
-                id = c0 + c;
-            }
-            nearest_offer(L, a.k, kd, ki, d, id);
-        }
-    }
-    nearest_block_merge(L, a.k, kd, ki, qt, per, sh);
-    if (warp >= qt) return;
-    const size_t q = q0 + qi;
-    if (a.n_split == 1) nearest_store(L, a.k, a.distances + q * a.k, a.ids + q * a.k);
-    else nearest_store(L, a.k, a.part_d + (q * a.n_split + blockIdx.y) * a.k, a.part_i + (q * a.n_split + blockIdx.y) * a.k);
-}
-
-// one CTA per query: warp w takes the chunk lists w, w + 8, ..., then warp 0 takes the other warps' lists
-__global__ void __launch_bounds__(kNearestBlock) nearest_merge_kernel(NearestLaunch a) {
-    __shared__ NearestShared sh;
-    const unsigned warp = threadIdx.x >> 5;
-    const size_t q = blockIdx.x;
-    NearestList L;
-    double kd;
-    unsigned ki;
-    nearest_list_init(L, kd, ki);
-    for (unsigned s = warp; s < a.n_split; s += kNearestWarps)
-        nearest_offer_list(L, a.k, kd, ki, a.part_d + (q * a.n_split + s) * a.k, a.part_i + (q * a.n_split + s) * a.k);
-    nearest_block_merge(L, a.k, kd, ki, 1, kNearestWarps, sh);
-    if (warp == 0) nearest_store(L, a.k, a.distances + q * a.k, a.ids + q * a.k);
-}
-
-// Split only when the query tiles would fill at most half of a kNearestCtasPerSm grid: then up to the grid's worth of
-// chunks per tile, none below kNearestMinChunk candidates.
-unsigned nearest_split(unsigned m, unsigned n_queries, int num_sms) {
-    const size_t tiles = ((size_t)n_queries + kNearestWarps - 1) / kNearestWarps;
-    const size_t target = (size_t)kNearestCtasPerSm * (size_t)(num_sms > 0 ? num_sms : 1);
-    if (tiles == 0 || 2 * tiles > target) return 1;
-    const size_t by_m = ((size_t)m + kNearestMinChunk - 1) / kNearestMinChunk;
-    const size_t s = target / tiles < by_m ? target / tiles : by_m;
-    return s > 1 ? (unsigned)s : 1u;
-}
-
-int launch_nearest(int kind, const NearestLaunch& a, void* stream) {
-    if (a.n_queries == 0 || a.k == 0 || a.k > kNearestMaxK || a.n_split == 0 || a.cfg_stride > kNearestCfgMax) return (int)cudaErrorInvalidValue;
-    cudaStream_t st = (cudaStream_t)stream;
-    const dim3 grid((a.n_queries + kNearestWarps - 1) / kNearestWarps, a.n_split);
-    switch (kind) {
-        case FKS_ROBOT_SE2: nearest_scan_kernel<FKS_ROBOT_SE2><<<grid, kNearestBlock, 0, st>>>(a); break;
-        case FKS_ROBOT_SE3: nearest_scan_kernel<FKS_ROBOT_SE3><<<grid, kNearestBlock, 0, st>>>(a); break;
-        case FKS_ROBOT_LINKED: nearest_scan_kernel<FKS_ROBOT_LINKED><<<grid, kNearestBlock, 0, st>>>(a); break;
-        default: return (int)cudaErrorInvalidValue;
-    }
-    if (a.n_split > 1) nearest_merge_kernel<<<a.n_queries, kNearestBlock, 0, st>>>(a);
     return (int)cudaGetLastError();
 }
 

@@ -24,11 +24,6 @@
 
 namespace {
 
-int mfail(int code, const std::string& msg) {
-    fks_host::set_last_error(msg);
-    return code;
-}
-
 // ---- NCCL through dlopen --------------------------------------------------------------------------------------------
 struct Nccl {
     void* handle = nullptr;
@@ -90,17 +85,17 @@ int fks_multi_sim_create(const int32_t* devices, int32_t n_devices, const fks_en
                          const fks_solver_params* params, double simulation_controller_frequency, uint64_t prng_seed,
                          int32_t debug_level, fks_multi_sim** out) {
     if (!out || !env || !robot || !params || n_devices < 1 || n_devices > 64)
-        return mfail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_sim_create: bad argument");
+        return fail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_sim_create: bad argument");
     *out = nullptr;
     int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return mfail(FKS_ERR_NO_DEVICE, "fks_multi_sim_create: no CUDA device");
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(FKS_ERR_NO_DEVICE, "fks_multi_sim_create: no CUDA device");
     fks_multi_sim* m = new (std::nothrow) fks_multi_sim();
-    if (!m) return mfail(FKS_ERR_OUT_OF_MEMORY, "fks_multi_sim_create: out of host memory");
+    if (!m) return fail(FKS_ERR_OUT_OF_MEMORY, "fks_multi_sim_create: out of host memory");
     for (int d = 0; d < n_devices; d++) {
         const int dev = devices ? devices[d] : d;
         if (dev < 0 || dev >= ndev || std::find(m->devices.begin(), m->devices.end(), dev) != m->devices.end()) {
             fks_multi_sim_destroy(m);
-            return mfail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_sim_create: bad or repeated device index");
+            return fail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_sim_create: bad or repeated device index");
         }
         m->devices.push_back(dev);
     }
@@ -139,14 +134,14 @@ static void shard_of(size_t n, size_t G, size_t d, size_t* lo, size_t* hi) {
 // its Philox ids by the whole batch (leg_id_stride = n) and writes its [n_legs][shard] records into the caller's [n_legs][n] array
 static int multi_simulate(fks_multi_sim* m, const double* starts, const double* targets, size_t n, size_t n_targets, size_t n_legs,
                           int allow_contacts, int noise_mode, const fks_noise_tape* tape, uint64_t first_particle_id, void* results) {
-    if (!m) return mfail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_forward_simulate: null simulator");
+    if (!m) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_forward_simulate: null simulator");
     if (n == 0) return FKS_OK;
     if (!starts || !targets || !results || !(n_targets == 1 || n_targets == n))
-        return mfail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_forward_simulate: need buffers and 1 target or one per start");
+        return fail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_forward_simulate: need buffers and 1 target or one per start");
     if (noise_mode != FKS_NOISE_PHILOX && noise_mode != FKS_NOISE_INJECTED && noise_mode != FKS_NOISE_NONE)
-        return mfail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_forward_simulate: unknown noise mode");
+        return fail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_forward_simulate: unknown noise mode");
     if (noise_mode == FKS_NOISE_INJECTED && (!tape || !tape->draws || !tape->offsets))
-        return mfail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_forward_simulate: injected noise needs a tape");
+        return fail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_forward_simulate: injected noise needs a tape");
     const size_t G = m->devices.size();
     const size_t stride = (size_t)m->cfg_stride;
     int rc = FKS_OK;
@@ -202,26 +197,26 @@ int fks_multi_forward_simulate_sequence(fks_multi_sim* m, const double* starts, 
 
 int fks_multi_forward_simulate_device(fks_multi_sim* m, const double* const* d_starts, const double* const* d_targets, size_t n,
                                       size_t n_targets, int allow_contacts, uint64_t first_particle_id, void* const* d_results) {
-    if (!m || !d_starts || !d_targets || !d_results) return mfail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_forward_simulate_device: null argument");
+    if (!m || !d_starts || !d_targets || !d_results) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_forward_simulate_device: null argument");
     if (n == 0) return FKS_OK;
-    if (!(n_targets == 1 || n_targets == n)) return mfail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_forward_simulate_device: need 1 target or one per start");
+    if (!(n_targets == 1 || n_targets == n)) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_forward_simulate_device: need 1 target or one per start");
     const size_t G = m->devices.size();
-    if (n % G != 0) return mfail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_forward_simulate_device: the all-gather needs equal shards (n divisible by the device count)");
+    if (n % G != 0) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_forward_simulate_device: the all-gather needs equal shards (n divisible by the device count)");
     Nccl& nc = nccl();
-    if (G > 1 && !nc.ok) return mfail(FKS_ERR_UNSUPPORTED, "fks_multi_forward_simulate_device: libnccl.so.2 not found");
+    if (G > 1 && !nc.ok) return fail(FKS_ERR_UNSUPPORTED, "fks_multi_forward_simulate_device: libnccl.so.2 not found");
     if (m->streams.empty()) {
         m->streams.assign(G, nullptr);
         for (size_t d = 0; d < G; d++) {
             cudaSetDevice(m->devices[d]);
             if (cudaStreamCreateWithFlags(&m->streams[d], cudaStreamNonBlocking) != cudaSuccess)
-                return mfail(FKS_ERR_CUDA, "fks_multi_forward_simulate_device: stream creation failed");
+                return fail(FKS_ERR_CUDA, "fks_multi_forward_simulate_device: stream creation failed");
         }
         if (G > 1) {
             m->comms.assign(G, nullptr);
             const ncclResult_t r = nc.CommInitAll(m->comms.data(), (int)G, m->devices.data());
             if (r != ncclSuccess) {
                 m->comms.clear();
-                return mfail(FKS_ERR_CUDA, std::string("ncclCommInitAll: ") + nc.GetErrorString(r));
+                return fail(FKS_ERR_CUDA, std::string("ncclCommInitAll: ") + nc.GetErrorString(r));
             }
         }
     }
@@ -241,20 +236,20 @@ int fks_multi_forward_simulate_device(fks_multi_sim* m, const double* const* d_s
             cudaSetDevice(m->devices[d]);
             const ncclResult_t r = nc.AllGather((const char*)d_results[d] + d * per * m->rec_stride, d_results[d], per * m->rec_stride, ncclChar,
                                                 m->comms[d], m->streams[d]);
-            if (r != ncclSuccess && rc == FKS_OK) rc = mfail(FKS_ERR_CUDA, std::string("ncclAllGather: ") + nc.GetErrorString(r));
+            if (r != ncclSuccess && rc == FKS_OK) rc = fail(FKS_ERR_CUDA, std::string("ncclAllGather: ") + nc.GetErrorString(r));
         }
         nc.GroupEnd();
     }
     for (size_t d = 0; d < G; d++) {
         cudaSetDevice(m->devices[d]);
         const cudaError_t e = cudaStreamSynchronize(m->streams[d]);
-        if (e != cudaSuccess && rc == FKS_OK) rc = mfail(FKS_ERR_CUDA, std::string("fks_multi_forward_simulate_device: ") + cudaGetErrorString(e));
+        if (e != cudaSuccess && rc == FKS_OK) rc = fail(FKS_ERR_CUDA, std::string("fks_multi_forward_simulate_device: ") + cudaGetErrorString(e));
     }
     return rc;
 }
 
 int fks_multi_get_statistics(fks_multi_sim* m, uint64_t* out) {
-    if (!m || !out) return mfail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_get_statistics: null argument");
+    if (!m || !out) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_get_statistics: null argument");
     std::memset(out, 0, FKS_NUM_STATS * sizeof(uint64_t));
     for (fks_sim* s : m->sims) {
         uint64_t part[FKS_NUM_STATS];
@@ -266,7 +261,7 @@ int fks_multi_get_statistics(fks_multi_sim* m, uint64_t* out) {
 }
 
 int fks_multi_reset_statistics(fks_multi_sim* m) {
-    if (!m) return mfail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_reset_statistics: null argument");
+    if (!m) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_multi_reset_statistics: null argument");
     for (fks_sim* s : m->sims) {
         const int rc = fks_reset_statistics(s);
         if (rc != FKS_OK) return rc;

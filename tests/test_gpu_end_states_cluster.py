@@ -11,48 +11,12 @@ from fast_kinematic_simulator_b200 import capi, workloads as W
 from scipy.cluster.hierarchy import fcluster, linkage
 
 import cluster_reference as CR
+import device_records as DR
 
 pytestmark = pytest.mark.gpu
 
-SMALL_MAX = 160  # segments up to this many positions are clustered in shared memory (fks_device_types.h)
+SMALL_MAX = 160  # segments up to this many positions are clustered in shared memory (fks_consumers.cu)
 MAX_SEGMENT = 8192
-
-
-def _stream():
-    return torch.cuda.current_stream().cuda_stream
-
-
-def _ids_tensor(ids):
-    return torch.from_numpy(np.ascontiguousarray(ids, dtype=np.uint32).view(np.int32)).cuda()
-
-
-def _simulated(name, n):
-    w = W.make(name, n_particles=n)
-    sim = w.make_simulator()
-    dr = torch.empty(n * sim.result_stride, dtype=torch.uint8, device="cuda")
-    sim.forward_simulate_device(torch.from_numpy(w.starts).cuda(), torch.from_numpy(w.targets).cuda(), n, w.targets.shape[0], dr, True,
-                                capi.NOISE_PHILOX, stream=_stream())
-    torch.cuda.synchronize()
-    return sim, dr, dr.cpu().numpy().view(sim.dtype)
-
-
-def _synthetic_se2(cfg, contact):
-    """SE(2) records written straight into a device buffer: configurations and contact flags of our choosing."""
-    sim = W.make("se2_arena", n_particles=4).make_simulator()
-    rec = np.zeros(len(cfg), dtype=sim.dtype)
-    rec["cfg"] = cfg
-    rec["flags"] = np.where(contact, capi.FLAG_DID_CONTACT, 0)
-    return sim, torch.from_numpy(rec.view(np.uint8).copy()).cuda(), rec
-
-
-def _gpu_matrix(sim, dr, ids):
-    m = len(ids)
-    if m == 0:
-        return np.zeros((0, 0))
-    out = torch.empty(m, m, dtype=torch.float64, device="cuda")
-    sim.end_states_pairwise_distance(dr, m, out, _ids_tensor(ids), stream=_stream())
-    torch.cuda.synchronize()
-    return out.cpu().numpy()
 
 
 class Segments:
@@ -63,8 +27,8 @@ class Segments:
         self.segments = [np.asarray(s, dtype=np.uint32) for s in segments]
         self.offsets = np.concatenate([[0], np.cumsum([len(s) for s in self.segments])]).astype(np.uint64)
         self.ids = np.concatenate(self.segments) if self.segments else np.zeros(0, np.uint32)
-        self.d_order = _ids_tensor(self.ids) if len(self.ids) else None
-        self.mats = [_gpu_matrix(sim, dr, s) for s in self.segments]
+        self.d_order = DR.u32(self.ids) if len(self.ids) else None
+        self.mats = [DR.gpu_matrix(sim, dr, s) for s in self.segments]
         contact = (rec["flags"] & capi.FLAG_DID_CONTACT) != 0
         self.contacts = [contact[s] for s in self.segments]
 
@@ -77,7 +41,7 @@ class Segments:
     def run(self, lk, t, separate=False, stream=None):
         labels = torch.full((max(len(self.ids), 1),), -1, dtype=torch.int32, device="cuda")
         counts = self.sim.end_states_cluster(self.dr, self.offsets, labels, t, lk, self.d_order, separate,
-                                             stream=stream if stream is not None else _stream())
+                                             stream=stream if stream is not None else DR.stream())
         return labels[:len(self.ids)].cpu().numpy().view(np.uint32), counts
 
     def check(self, lk, t, separate=False):
@@ -99,9 +63,9 @@ def _chunks(ids, sizes):
 
 @pytest.mark.parametrize("name,n", [("arm_table", 700), ("se2_arena", 800), ("se3_narrow_passage", 800)])
 def test_workload_end_states_match_the_reference(name, n):
-    sim, dr, rec = _simulated(name, n)
+    _, sim, dr, rec = DR.simulated(name, n)
     order = torch.empty(n, dtype=torch.int32, device="cuda")
-    n_free, _ = sim.end_states_partition(dr, n, order, stream=_stream())
+    n_free, _ = sim.end_states_partition(dr, n, order, stream=DR.stream())
     order = order.cpu().numpy().view(np.uint32)
     # the planner's split: parts of the partition, cut into segments on both sides of the shared-memory limit
     parts = _chunks(order[:n_free], [40, SMALL_MAX, 250]) + _chunks(order[n_free:], [SMALL_MAX + 1, 90])
@@ -118,7 +82,7 @@ def test_workload_end_states_match_the_reference(name, n):
 
 
 def test_segment_sizes_across_the_shared_memory_limit():
-    sim, dr, rec = _simulated("se2_arena", 2100)
+    _, sim, dr, rec = DR.simulated("se2_arena", 2100)
     sizes = [0, 1, 2, 31, 33, SMALL_MAX - 1, SMALL_MAX, SMALL_MAX + 1, 1500]
     segs = Segments(sim, dr, rec, np.split(np.arange(sum(sizes), dtype=np.uint32), np.cumsum(sizes)[:-1]))
     for lk in (CR.LINKAGE_SINGLE, CR.LINKAGE_COMPLETE):
@@ -132,8 +96,8 @@ def test_one_segment_of_8192_against_scipy():
     n = MAX_SEGMENT
     rng = np.random.default_rng(8192)
     cfg = np.stack([rng.uniform(0, 10, n), rng.uniform(0, 10, n), rng.uniform(-3, 3, n)], axis=1)
-    sim, dr, rec = _synthetic_se2(cfg, np.zeros(n, bool))
-    mat = _gpu_matrix(sim, dr, np.arange(n, dtype=np.uint32))
+    sim, dr, rec = DR.synthetic_se2(cfg, np.zeros(n, bool))
+    mat = DR.gpu_matrix(sim, dr, np.arange(n, dtype=np.uint32))
     cond = mat[np.triu_indices(n, 1)]
     del mat
     assert np.all(np.isfinite(cond)) and len(np.unique(cond)) == len(cond)  # tie-free: scipy's order is then ours
@@ -142,7 +106,7 @@ def test_one_segment_of_8192_against_scipy():
     for lk, method in ((CR.LINKAGE_COMPLETE, "complete"), (CR.LINKAGE_SINGLE, "single")):
         z = linkage(cond, method=method)
         for t in (z[n // 2, 2], z[n - n // 50, 2], float(np.quantile(z[:, 2], 0.9))):
-            counts = sim.end_states_cluster(dr, offsets, labels, t, lk, stream=_stream())
+            counts = sim.end_states_cluster(dr, offsets, labels, t, lk, stream=DR.stream())
             want = CR.canonical(fcluster(z, t, criterion="distance"))
             assert np.array_equal(labels.cpu().numpy().view(np.uint32), want), (method, t)
             assert counts.tolist() == [len(np.unique(want))]
@@ -155,7 +119,7 @@ def test_ties_nan_and_contact_flags_on_synthetic_records():
     # SE(2) configurations on a small integer grid: most distances tie with many others
     cfg = np.stack([rng.integers(0, 3, n), rng.integers(0, 3, n), rng.integers(-1, 2, n) * (np.pi / 2)], axis=1).astype(np.float64)
     cfg[rng.random(n) < 0.05] = np.nan  # NaN configurations: their distances are NaN, clustered as +inf
-    sim, dr, rec = _synthetic_se2(cfg, rng.random(n) < 0.4)
+    sim, dr, rec = DR.synthetic_se2(cfg, rng.random(n) < 0.4)
     segs = Segments(sim, dr, rec, _chunks(np.arange(n, dtype=np.uint32), [100, 400, 37, 63]))
     values = np.unique(np.concatenate([m[np.isfinite(m)] for m in segs.mats]))
     for lk in (CR.LINKAGE_SINGLE, CR.LINKAGE_COMPLETE):
@@ -174,11 +138,11 @@ def test_all_legs_of_a_sequence_in_one_call():
     legs = np.stack([there, w.starts.reshape(n, stride), there])  # out, back, out again
     dr = torch.empty(m_legs * n * sim.result_stride, dtype=torch.uint8, device="cuda")
     sim.forward_simulate_sequence_device(torch.from_numpy(w.starts).cuda(), torch.from_numpy(np.ascontiguousarray(legs)).cuda(), n, n,
-                                         m_legs, dr, stream=_stream())
+                                         m_legs, dr, stream=DR.stream())
     segments = []
     for k in range(m_legs):
         order = torch.empty(n, dtype=torch.int32, device="cuda")
-        n_free, _ = sim.end_states_partition(dr[k * n * sim.result_stride:], n, order, stream=_stream())
+        n_free, _ = sim.end_states_partition(dr[k * n * sim.result_stride:], n, order, stream=DR.stream())
         ids = order.cpu().numpy().view(np.uint32) + np.uint32(k * n)  # leg-major records from the base pointer
         segments += [ids[:n_free], ids[n_free:]]
     rec = dr.cpu().numpy().view(sim.dtype)
@@ -194,7 +158,7 @@ def test_repeated_calls_and_a_side_stream_agree():
     rng = np.random.default_rng(5)
     n = 64 * 20 + 700
     cfg = np.stack([rng.uniform(0, 4, n), rng.uniform(0, 4, n), rng.uniform(-3, 3, n)], axis=1)
-    sim, dr, rec = _synthetic_se2(cfg, rng.random(n) < 0.5)
+    sim, dr, rec = DR.synthetic_se2(cfg, rng.random(n) < 0.5)
     segs = Segments(sim, dr, rec, _chunks(np.arange(n, dtype=np.uint32), [64] * 20 + [700]))
     t = segs.entries([0.1])[0]
     first = segs.run(capi.LINKAGE_COMPLETE, t, True)
@@ -210,7 +174,7 @@ def test_repeated_calls_and_a_side_stream_agree():
 
 def test_invalid_arguments_and_empty_calls():
     rng = np.random.default_rng(6)
-    sim, dr, rec = _synthetic_se2(rng.uniform(0, 1, (MAX_SEGMENT + 1, 3)), np.zeros(MAX_SEGMENT + 1, bool))
+    sim, dr, rec = DR.synthetic_se2(rng.uniform(0, 1, (MAX_SEGMENT + 1, 3)), np.zeros(MAX_SEGMENT + 1, bool))
     labels = torch.empty(MAX_SEGMENT + 1, dtype=torch.int32, device="cuda")
     ok = np.array([0, 10], dtype=np.uint64)
 

@@ -9,49 +9,17 @@ import torch
 from fast_kinematic_simulator_b200 import capi, workloads as W
 
 import cluster_reference as CR
+import device_records as DR
 import group_reference as GR
 
 pytestmark = pytest.mark.gpu
 
-SMALL_MAX = 256  # groups up to this many members are searched by one CTA (fks_device_types.h)
+SMALL_MAX = 256  # groups up to this many members are searched by one CTA (fks_consumers.cu)
 MAX_GROUP = 8192
-
-
-def _stream():
-    return torch.cuda.current_stream().cuda_stream
-
-
-def _u32(a):
-    return torch.from_numpy(np.ascontiguousarray(a, dtype=np.uint32).view(np.int32)).cuda()
 
 
 def _host_u32(t):
     return t.cpu().numpy().view(np.uint32)
-
-
-def _simulated(name, n):
-    w = W.make(name, n_particles=n)
-    sim = w.make_simulator()
-    dr = torch.empty(n * sim.result_stride, dtype=torch.uint8, device="cuda")
-    sim.forward_simulate_device(torch.from_numpy(w.starts).cuda(), torch.from_numpy(w.targets).cuda(), n, w.targets.shape[0], dr, True,
-                                capi.NOISE_PHILOX, stream=_stream())
-    torch.cuda.synchronize()
-    return w, sim, dr
-
-
-def _synthetic_se2(cfg):
-    sim = W.make("se2_arena", n_particles=4).make_simulator()
-    rec = np.zeros(len(cfg), dtype=sim.dtype)
-    rec["cfg"] = cfg
-    return sim, torch.from_numpy(rec.view(np.uint8).copy()).cuda()
-
-
-def _gpu_matrix(sim, dr, ids):
-    m = len(ids)
-    out = torch.empty(m, m, dtype=torch.float64, device="cuda")
-    sim.end_states_pairwise_distance(dr, m, out, _u32(ids), stream=_stream())
-    torch.cuda.synchronize()
-    return out.cpu().numpy()
 
 
 def run_groups(sim, dr, labels, n_clusters, ids=None, stream=None):
@@ -60,8 +28,8 @@ def run_groups(sim, dr, labels, n_clusters, ids=None, stream=None):
     mem = torch.full((max(m, 1),), -1, dtype=torch.int32, device="cuda")
     reps = torch.full((max(n_clusters, 1),), -1, dtype=torch.int32, device="cuda")
     radius = torch.full((max(n_clusters, 1),), -1.0, dtype=torch.float64, device="cuda")
-    sizes = sim.end_states_groups(dr, m, _u32(labels), n_clusters, off, mem, reps, radius, None if ids is None else _u32(ids),
-                                  stream=stream if stream is not None else _stream())
+    sizes = sim.end_states_groups(dr, m, DR.u32(labels), n_clusters, off, mem, reps, radius, None if ids is None else DR.u32(ids),
+                                  stream=stream if stream is not None else DR.stream())
     return (_host_u32(off), _host_u32(mem)[:m], _host_u32(reps)[:n_clusters], radius.cpu().numpy()[:n_clusters], sizes), (off, mem)
 
 
@@ -71,7 +39,7 @@ def check_groups(sim, dr, labels, n_clusters, ids=None, matrix_of=None):
     ids_np = np.arange(len(labels), dtype=np.uint32) if ids is None else np.asarray(ids, dtype=np.uint32)
     if matrix_of is None:
         def matrix_of(c, pos):
-            return _gpu_matrix(sim, dr, ids_np[pos])
+            return DR.gpu_matrix(sim, dr, ids_np[pos])
     got, dev = run_groups(sim, dr, labels, n_clusters, ids)
     want = GR.groups(labels, n_clusters, matrix_of, ids_np)
     off, mem, reps, radius, sizes = got
@@ -87,7 +55,7 @@ def segment_matrices(sim, dr, ids, offsets):
     """matrix_of for groups that stay inside segments: the submatrix of the segment's GPU pairwise matrix (an entry depends
     only on its two records, so the bits are those of a matrix over the group alone)."""
     seg_of = np.repeat(np.arange(len(offsets) - 1), np.diff(offsets).astype(np.int64))
-    mats = [_gpu_matrix(sim, dr, ids[offsets[s]:offsets[s + 1]]) if offsets[s + 1] > offsets[s] else None for s in range(len(offsets) - 1)]
+    mats = [DR.gpu_matrix(sim, dr, ids[offsets[s]:offsets[s + 1]]) if offsets[s + 1] > offsets[s] else None for s in range(len(offsets) - 1)]
 
     def matrix_of(c, pos):
         s = seg_of[pos[0]]
@@ -100,7 +68,7 @@ def segment_matrices(sim, dr, ids, offsets):
 
 def _cluster(sim, dr, ids, offsets, lk, t):
     labels = torch.empty(max(len(ids), 1), dtype=torch.int32, device="cuda")
-    counts = sim.end_states_cluster(dr, np.asarray(offsets, np.uint64), labels, t, lk, _u32(ids), stream=_stream())
+    counts = sim.end_states_cluster(dr, np.asarray(offsets, np.uint64), labels, t, lk, DR.u32(ids), stream=DR.stream())
     return _host_u32(labels)[:len(ids)], int(counts.sum())
 
 
@@ -112,9 +80,9 @@ def _entries(mats, q):
 
 @pytest.mark.parametrize("name,n", [("se2_arena", 2000), ("se3_narrow_passage", 1500), ("arm_table", 1200)])
 def test_workload_end_states_through_partition_and_cluster(name, n):
-    _, sim, dr = _simulated(name, n)
+    _, sim, dr, _ = DR.simulated(name, n)
     order = torch.empty(n, dtype=torch.int32, device="cuda")
-    n_free, _ = sim.end_states_partition(dr, n, order, stream=_stream())
+    n_free, _ = sim.end_states_partition(dr, n, order, stream=DR.stream())
     ids = _host_u32(order)
     offsets = np.array([0, n_free, n], dtype=np.int64)
     mats, matrix_of = segment_matrices(sim, dr, ids, offsets)
@@ -137,11 +105,11 @@ def test_all_legs_of_a_sequence_in_one_call():
     legs = np.stack([there, w.starts.reshape(n, stride), there])
     dr = torch.empty(m_legs * n * sim.result_stride, dtype=torch.uint8, device="cuda")
     sim.forward_simulate_sequence_device(torch.from_numpy(w.starts).cuda(), torch.from_numpy(np.ascontiguousarray(legs)).cuda(), n, n,
-                                         m_legs, dr, stream=_stream())
+                                         m_legs, dr, stream=DR.stream())
     ids, offsets = [], [0]
     for k in range(m_legs):
         order = torch.empty(n, dtype=torch.int32, device="cuda")
-        n_free, _ = sim.end_states_partition(dr[k * n * sim.result_stride:], n, order, stream=_stream())
+        n_free, _ = sim.end_states_partition(dr[k * n * sim.result_stride:], n, order, stream=DR.stream())
         leg = _host_u32(order) + np.uint32(k * n)
         ids.append(leg)
         offsets += [offsets[-1] + n_free, offsets[-1] + n]
@@ -167,7 +135,7 @@ def test_ties_and_nan_configurations():
     rng.shuffle(labels)
     nan_rows = np.flatnonzero(labels == 0)
     cfg[nan_rows] = np.nan
-    sim, dr = _synthetic_se2(cfg)
+    sim, dr, _ = DR.synthetic_se2(cfg)
     got, _ = check_groups(sim, dr, labels, k)
     assert got[3][0] == np.inf and got[2][0] == nan_rows[0]
     assert got[4].max() > SMALL_MAX
@@ -182,7 +150,7 @@ def test_group_sizes_across_the_kernel_boundary_up_to_8192():
     n = sum(sizes)
     rng = np.random.default_rng(8192)
     cfg = np.stack([rng.uniform(0, 10, n), rng.uniform(0, 10, n), rng.uniform(-3, 3, n)], axis=1)
-    sim, dr = _synthetic_se2(cfg)
+    sim, dr, _ = DR.synthetic_se2(cfg)
     labels = np.repeat(np.arange(len(sizes)), sizes).astype(np.uint32)
     rng.shuffle(labels)
     ids = rng.permutation(n).astype(np.uint32)
@@ -195,7 +163,7 @@ def test_repeated_calls_and_a_side_stream_agree():
     rng = np.random.default_rng(5)
     n, k = 6000, 700
     cfg = np.stack([rng.uniform(0, 4, n), rng.uniform(0, 4, n), rng.uniform(-3, 3, n)], axis=1)
-    sim, dr = _synthetic_se2(cfg)
+    sim, dr, _ = DR.synthetic_se2(cfg)
     labels = np.concatenate([np.arange(k), rng.integers(0, k, n - k - 600), np.full(600, 3)]).astype(np.uint32)
     rng.shuffle(labels)
     first, _ = run_groups(sim, dr, labels, k)
@@ -219,7 +187,7 @@ def _gather(sim, dr, dev, n_clusters, selected, per_group, group_targets=None, s
     targets = None if group_targets is None else torch.full((max(n_out, 1), stride), -7.0, dtype=torch.float64, device="cuda")
     gt = None if group_targets is None else torch.from_numpy(np.ascontiguousarray(group_targets, dtype=np.float64)).cuda()
     sim.end_states_gather_starts(dr, off, mem, n_clusters, selected, per_group, starts, gt, targets,
-                                 stream=stream if stream is not None else _stream())
+                                 stream=stream if stream is not None else DR.stream())
     torch.cuda.synchronize()
     return starts.cpu().numpy()[:n_out], None if targets is None else targets.cpu().numpy()[:n_out]
 
@@ -228,7 +196,7 @@ def test_gather_is_the_cyclic_fill():
     rng = np.random.default_rng(9)
     n, k = 3000, 40
     cfg = np.stack([rng.uniform(0, 4, n), rng.uniform(0, 4, n), rng.uniform(-3, 3, n)], axis=1)
-    sim, dr = _synthetic_se2(cfg)
+    sim, dr, _ = DR.synthetic_se2(cfg)
     labels = np.concatenate([np.arange(k), rng.integers(0, k, n - k)]).astype(np.uint32)
     rng.shuffle(labels)
     ids = rng.permutation(n).astype(np.uint32)
@@ -251,23 +219,23 @@ def test_gather_is_the_cyclic_fill():
 
 def _one_edge(name, n, per_group, q):
     """One planner edge on the device and through the host; returns the second batch's records of both."""
-    w, sim, dr = _simulated(name, n)
+    w, sim, dr, _ = DR.simulated(name, n)
     stride = sim.config_stride
     # device edge: partition, cluster, groups, gather, simulate
     order = torch.empty(n, dtype=torch.int32, device="cuda")
-    n_free, _ = sim.end_states_partition(dr, n, order, stream=_stream())
+    n_free, _ = sim.end_states_partition(dr, n, order, stream=DR.stream())
     offsets = np.array([0, n_free, n], dtype=np.uint64)
-    mat = _gpu_matrix(sim, dr, _host_u32(order))
+    mat = DR.gpu_matrix(sim, dr, _host_u32(order))
     vals = mat[np.triu_indices(n, 1)]
     t = float(np.quantile(vals[np.isfinite(vals)], q, method="lower"))
     labels = torch.empty(n, dtype=torch.int32, device="cuda")
-    counts = sim.end_states_cluster(dr, offsets, labels, t, capi.LINKAGE_COMPLETE, order, stream=_stream())
+    counts = sim.end_states_cluster(dr, offsets, labels, t, capi.LINKAGE_COMPLETE, order, stream=DR.stream())
     k = int(counts.sum())
     off = torch.empty(k + 1, dtype=torch.int32, device="cuda")
     mem = torch.empty(n, dtype=torch.int32, device="cuda")
     reps = torch.empty(k, dtype=torch.int32, device="cuda")
     radius = torch.empty(k, dtype=torch.float64, device="cuda")
-    sizes = sim.end_states_groups(dr, n, labels, k, off, mem, reps, radius, order, stream=_stream())
+    sizes = sim.end_states_groups(dr, n, labels, k, off, mem, reps, radius, order, stream=DR.stream())
     by_size = np.argsort(-sizes.astype(np.int64), kind="stable")
     selected = np.concatenate([by_size[:4], by_size[-2:], by_size[:2]])  # the largest and the smallest groups, two repeats
     g_targets = np.where(np.arange(len(selected))[:, None] % 2 == 0, w.targets.reshape(-1, stride)[:1], w.starts.reshape(-1, stride)[:1])
@@ -275,9 +243,9 @@ def _one_edge(name, n, per_group, q):
     starts = torch.empty(n2, stride, dtype=torch.float64, device="cuda")
     targets = torch.empty(n2, stride, dtype=torch.float64, device="cuda")
     sim.end_states_gather_starts(dr, off, mem, k, selected, per_group, starts, torch.from_numpy(np.ascontiguousarray(g_targets)).cuda(),
-                                 targets, stream=_stream())
+                                 targets, stream=DR.stream())
     dr2 = torch.empty(n2 * sim.result_stride, dtype=torch.uint8, device="cuda")
-    sim.forward_simulate_device(starts, targets, n2, n2, dr2, True, capi.NOISE_PHILOX, first_particle_id=n, stream=_stream())
+    sim.forward_simulate_device(starts, targets, n2, n2, dr2, True, capi.NOISE_PHILOX, first_particle_id=n, stream=DR.stream())
     torch.cuda.synchronize()
     device_records = dr2.cpu().numpy().tobytes()
     # host edge: download the records and the labels, group and gather in numpy, simulate from host buffers
@@ -304,14 +272,14 @@ def test_one_planner_edge_on_the_device_equals_the_host_edge(name, n, q):
 def test_invalid_arguments_and_empty_calls():
     rng = np.random.default_rng(6)
     n = 12000
-    sim, dr = _synthetic_se2(rng.uniform(0, 1, (n, 3)))
+    sim, dr, _ = DR.synthetic_se2(rng.uniform(0, 1, (n, 3)))
     off = torch.empty(n + 1, dtype=torch.int32, device="cuda")
     mem = torch.empty(n, dtype=torch.int32, device="cuda")
     reps = torch.empty(n, dtype=torch.int32, device="cuda")
     radius = torch.empty(n, dtype=torch.float64, device="cuda")
 
     def refused(labels, k, m=None, **kw):
-        args = dict(d_results=dr, m=len(labels) if m is None else m, d_labels=_u32(labels) if len(labels) else None, n_clusters=k,
+        args = dict(d_results=dr, m=len(labels) if m is None else m, d_labels=DR.u32(labels) if len(labels) else None, n_clusters=k,
                     d_group_offsets=off, d_members=mem, d_representatives=reps, d_radius=radius)
         args.update(kw)
         with pytest.raises(capi.FksError) as e:
@@ -333,9 +301,9 @@ def test_invalid_arguments_and_empty_calls():
     assert sim.end_states_groups(None, 0, None, 0, None, None, None, None).tolist() == []
     assert sim.launch_count == before
     # the same launches for 1 group or 10 000
-    sim.end_states_groups(dr, 5, _u32(np.zeros(5)), 1, off, mem, reps, radius)
+    sim.end_states_groups(dr, 5, DR.u32(np.zeros(5)), 1, off, mem, reps, radius)
     one = sim.launch_count - before
-    sim.end_states_groups(dr, n, _u32(np.arange(n) % 10000), 10000, off, mem, reps, radius)
+    sim.end_states_groups(dr, n, DR.u32(np.arange(n) % 10000), 10000, off, mem, reps, radius)
     assert sim.launch_count - before == 2 * one
 
     labels = np.arange(n) % 10

@@ -7,32 +7,19 @@ import torch
 
 from fast_kinematic_simulator_b200 import capi, workloads as W
 
+import device_records as DR
 import nearest_reference as NR
 
 pytestmark = pytest.mark.gpu
 
 MAX_K = 64
-MIN_CHUNK = 2048  # fewest candidates per chunk of a split (fks_kernels.cu)
+MIN_CHUNK = 2048  # fewest candidates per chunk of a split (fks_consumers.cu)
 PAIRWISE_MAX = 16384  # records per pairwise call here: a 2 GiB matrix
 
 
-def _stream():
-    return torch.cuda.current_stream().cuda_stream
-
-
-def _u32(a):
-    return torch.from_numpy(np.ascontiguousarray(a, dtype=np.uint32).view(np.int32)).cuda()
-
-
 def _split_switch():
-    """Fewest queries that take the query-tiled path whatever m: more than 2 * 8 queries per SM (fks_kernels.cu)."""
+    """Fewest queries that take the query-tiled path whatever m: more than 2 * 8 queries per SM (fks_consumers.cu)."""
     return 16 * torch.cuda.get_device_properties(0).multi_processor_count + 1
-
-
-def _records(sim, cfg):
-    rec = np.zeros(len(cfg), dtype=sim.dtype)
-    rec["cfg"] = cfg
-    return torch.from_numpy(rec.view(np.uint8).copy()).cuda()
 
 
 def gpu_distances(sim, cand, queries, query_rows=None):
@@ -40,14 +27,14 @@ def gpu_distances(sim, cand, queries, query_rows=None):
     over subsets of the records: candidate chunks together with the chosen queries."""
     m, n_q = len(cand), len(queries)
     rows = np.arange(n_q) if query_rows is None else np.asarray(query_rows)
-    dr = _records(sim, np.concatenate([cand, queries]) if m else queries)
+    dr, _ = DR.records(sim, np.concatenate([cand, queries]) if m else queries)
     chunk = max(1, PAIRWISE_MAX - len(rows))
     out = np.empty((m, len(rows)))
     for c0 in range(0, m, chunk):
         c = min(chunk, m - c0)
         ids = np.concatenate([np.arange(c0, c0 + c), m + rows])
         mat = torch.empty(len(ids), len(ids), dtype=torch.float64, device="cuda")
-        sim.end_states_pairwise_distance(dr, len(ids), mat, _u32(ids), stream=_stream())
+        sim.end_states_pairwise_distance(dr, len(ids), mat, DR.u32(ids), stream=DR.stream())
         out[c0:c0 + c] = mat[:c, c:].cpu().numpy()
     torch.cuda.synchronize()
     return out
@@ -56,7 +43,7 @@ def gpu_distances(sim, cand, queries, query_rows=None):
 def run_nearest(sim, d_cand, m, d_q, n_q, k, stream=None):
     ids = torch.full((max(n_q * k, 1),), -7, dtype=torch.int32, device="cuda")
     dist = torch.full((max(n_q * k, 1),), -7.0, dtype=torch.float64, device="cuda")
-    sim.nearest_configurations(d_cand, m, d_q, n_q, k, ids, dist, stream=stream if stream is not None else _stream())
+    sim.nearest_configurations(d_cand, m, d_q, n_q, k, ids, dist, stream=stream if stream is not None else DR.stream())
     return ids, dist
 
 
