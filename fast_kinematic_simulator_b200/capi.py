@@ -58,6 +58,7 @@ EXPORTS = (
     "fks_multi_get_statistics",
     "fks_multi_reset_statistics",
     "fks_check_config_collision",
+    "fks_check_config_collision_device",
     "fks_sim_trace_stride",
     "fks_forward_simulate_traced",
     "fks_get_statistics",
@@ -132,6 +133,7 @@ lib.fks_forward_simulate_device.argtypes = [
     C.c_uint64, C.c_void_p, C.c_void_p,
 ]
 lib.fks_check_config_collision.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_double, C.c_void_p]
+lib.fks_check_config_collision_device.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_double, C.c_void_p, C.c_void_p]
 lib.fks_sim_trace_stride.argtypes = [C.c_void_p]
 lib.fks_sim_trace_stride.restype = C.c_size_t
 lib.fks_forward_simulate_traced.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, P(NoiseTape), C.c_uint64, C.c_void_p,

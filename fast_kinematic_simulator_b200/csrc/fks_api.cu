@@ -47,6 +47,21 @@ int upload(T** dst, const T* src, size_t n) {
     return FKS_OK;
 }
 
+// The launches of one simulator share its particle counter, statistics and scratch slots (the simulate kernel's contexts and
+// check_config_kernel's warps both use d_scratch), so they never overlap: the one kernel `enqueue` puts on `stream` waits for
+// the previous launch when that was on another stream, and the next launch waits for it.  `enqueue` returns FKS_OK or a code.
+template <typename Enqueue>
+int serialised_launch(fks_sim* s, cudaStream_t stream, Enqueue&& enqueue) {
+    if (s->has_last && stream != s->last_stream) FKS_CUDA(cudaStreamWaitEvent(stream, s->last_done, 0));
+    const int rc = enqueue();
+    if (rc != FKS_OK) return rc;
+    FKS_CUDA(cudaEventRecord(s->last_done, stream));
+    s->last_stream = stream;
+    s->has_last = true;
+    s->launches++;
+    return FKS_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -639,21 +654,46 @@ static int simulate_on_stream(fks_sim* s, const double* d_starts, const double* 
     const size_t dyn_smem = (size_t)a.sync_off + kSyncBytes;
     const size_t blocks_needed = (n + (size_t)wpb - 1) / (size_t)wpb;
     const int grid = (int)std::min<size_t>((size_t)s->grid_max, blocks_needed);
-    if (s->has_last && stream != s->last_stream) FKS_CUDA(cudaStreamWaitEvent(stream, s->last_done, 0));
-    FKS_CUDA(cudaMemsetAsync(s->d_counter, 0, 4 * sizeof(unsigned int), stream));
     const void* l2_base = s->env->l2_window_bytes ? s->env->d_sdf : nullptr;
     a.ctx_store = s->d_ctx_store;
     a.pool = std::max(wpb, std::min((s->pool_eighths * wpb + 7) / 8, s->pool));
-    if (s->timing) FKS_CUDA(cudaEventRecord(s->tev[0], stream));
-    const int rc = launch_simulate(s->robot->host.kind, a, grid, dyn_smem, stream, l2_base, s->env->l2_window_bytes);
-    if (rc != 0) return cuda_fail((cudaError_t)rc, "simulate kernel launch");
-    if (s->timing) FKS_CUDA(cudaEventRecord(s->tev[1], stream));
-    s->timed_kernels = s->timing ? 1 : 0;
-    FKS_CUDA(cudaEventRecord(s->last_done, stream));
-    s->last_stream = stream;
-    s->has_last = true;
-    s->launches++;
-    return FKS_OK;
+    return serialised_launch(s, stream, [&]() -> int {
+        FKS_CUDA(cudaMemsetAsync(s->d_counter, 0, 4 * sizeof(unsigned int), stream));
+        if (s->timing) FKS_CUDA(cudaEventRecord(s->tev[0], stream));
+        const int rc = launch_simulate(s->robot->host.kind, a, grid, dyn_smem, stream, l2_base, s->env->l2_window_bytes);
+        if (rc != 0) return cuda_fail((cudaError_t)rc, "simulate kernel launch");
+        if (s->timing) FKS_CUDA(cudaEventRecord(s->tev[1], stream));
+        s->timed_kernels = s->timing ? 1 : 0;
+        return FKS_OK;
+    });
+}
+
+// CheckConfigCollision of n configurations d_configs[n][cfg_stride] into d_out[0 .. n), one warp per configuration
+static int check_config_on_stream(fks_sim* s, const double* d_configs, size_t n, double inflation_ratio, uint8_t* d_out,
+                                  cudaStream_t stream) {
+    LaunchArgs a = s->plan;
+    a.env = s->env->dev;
+    a.sp = s->sp;
+    a.robot = s->robot->d_robot;
+    a.pxy = s->robot->d_pxy;
+    a.pzl = s->robot->d_pzl;
+    a.starts = d_configs;
+    a.scratch = s->d_scratch;
+    a.jscratch = s->d_jscratch;
+    a.ctx_store = s->d_ctx_store;
+    a.n_particles = n;
+    a.cfg_stride = s->robot->stride;
+    const size_t per_sm = (n + (size_t)s->num_sms - 1) / (size_t)s->num_sms;
+    const int wpb = (int)std::max<size_t>(1, std::min<size_t>((size_t)s->plan.warps_per_block, per_sm));
+    a.warps_per_block = wpb;
+    a.pool = wpb;  // (check_config keeps no context pool; scratch slots are per warp)
+    a.sync_off = a.warps_off + wpb * a.wl.total * 8;
+    const size_t dyn_smem = (size_t)a.sync_off + kSyncBytes;
+    const int grid = (int)std::min<size_t>((size_t)s->grid_max, (n + (size_t)wpb - 1) / (size_t)wpb);
+    return serialised_launch(s, stream, [&]() -> int {
+        const int rc = launch_check_config(s->robot->host.kind, a, grid, dyn_smem, stream, inflation_ratio, d_out);
+        return rc != 0 ? cuda_fail((cudaError_t)rc, "check_config kernel launch") : FKS_OK;
+    });
 }
 
 static int check_batch(const fks_sim* sim, const void* starts, const void* targets, size_t n, size_t n_targets, int noise_mode,
@@ -864,31 +904,22 @@ int fks_check_config_collision(fks_sim* s, const double* configs, size_t n, doub
     if ((rc = ensure(&s->d_starts, &s->cap_starts, n * stride)) != FKS_OK) return rc;
     if ((rc = ensure(&s->d_results, &s->cap_results, n)) != FKS_OK) return rc;
     FKS_CUDA(cudaMemcpyAsync(s->d_starts, configs, n * stride * 8, cudaMemcpyHostToDevice, s->stream));
-    LaunchArgs a = s->plan;
-    a.env = s->env->dev;
-    a.sp = s->sp;
-    a.robot = s->robot->d_robot;
-    a.pxy = s->robot->d_pxy;
-    a.pzl = s->robot->d_pzl;
-    a.starts = s->d_starts;
-    a.scratch = s->d_scratch;
-    a.jscratch = s->d_jscratch;
-    a.ctx_store = s->d_ctx_store;
-    a.n_particles = n;
-    a.cfg_stride = s->robot->stride;
-    const size_t per_sm = (n + (size_t)s->num_sms - 1) / (size_t)s->num_sms;
-    const int wpb = (int)std::max<size_t>(1, std::min<size_t>((size_t)s->plan.warps_per_block, per_sm));
-    a.warps_per_block = wpb;
-    a.pool = wpb;  // (check_config keeps no context pool; scratch slots are per warp)
-    a.sync_off = a.warps_off + wpb * a.wl.total * 8;
-    const size_t dyn_smem = (size_t)a.sync_off + kSyncBytes;
-    const int grid = (int)std::min<size_t>((size_t)s->grid_max, (n + (size_t)wpb - 1) / (size_t)wpb);
-    rc = launch_check_config(s->robot->host.kind, a, grid, dyn_smem, s->stream, inflation_ratio, (unsigned char*)s->d_results);
-    if (rc != 0) return cuda_fail((cudaError_t)rc, "check_config kernel launch");
-    s->launches++;
+    rc = check_config_on_stream(s, s->d_starts, n, inflation_ratio, (uint8_t*)s->d_results, s->stream);
+    if (rc != FKS_OK) return rc;
     FKS_CUDA(cudaMemcpyAsync(out, s->d_results, n, cudaMemcpyDeviceToHost, s->stream));
     FKS_CUDA(cudaStreamSynchronize(s->stream));
     return FKS_OK;
+}
+
+int fks_check_config_collision_device(fks_sim* s, const double* d_configs, size_t n, double inflation_ratio, uint8_t* d_out,
+                                      void* cuda_stream) {
+    if (!s) return fail(FKS_ERR_INVALID_ARGUMENT, "fks_check_config_collision_device: null simulator");
+    if (n == 0) return FKS_OK;
+    if (!d_configs || !d_out || std::isnan(inflation_ratio))
+        return fail(FKS_ERR_INVALID_ARGUMENT, "fks_check_config_collision_device: bad argument");
+    DeviceGuard guard(s->device);
+    if (!guard.ok) return fail(FKS_ERR_CUDA, "fks_check_config_collision_device: cudaSetDevice failed");
+    return check_config_on_stream(s, d_configs, n, inflation_ratio, d_out, (cudaStream_t)cuda_stream);
 }
 
 // waits for the simulator's own work only: its stream and the last launch made on a caller's stream

@@ -151,7 +151,7 @@ struct fks_sim {
     cudaEvent_t tev[2];
     int timing, timed_kernels;
     // launches of one simulator share its particle counter, scratch slots and statistics: a launch on another stream waits
-    // for the previous one (fks_forward_simulate_device takes the caller's stream)
+    // for the previous one (the _device calls take the caller's stream; serialised_launch in fks_api.cu)
     cudaEvent_t last_done;
     cudaStream_t last_stream;
     bool has_last;

@@ -399,6 +399,13 @@ class GpuParticleContactSimulator:
         check(lib.fks_check_config_collision(self._h, configs.ctypes.data, configs.shape[0], float(inflation_ratio), out.ctypes.data))
         return out.astype(bool)
 
+    def check_config_collision_device(self, d_configs, n, d_out, inflation_ratio=0.0, stream=0):
+        """check_config_collision on device buffers (fks_check_config_collision_device): d_out[i] (uint8) = 1 when
+        configuration i of d_configs ([n][config_stride] float64) collides, else 0.  Asynchronous on `stream`, ordered with
+        the simulator's batch calls."""
+        check(lib.fks_check_config_collision_device(self._h, _dev_ptr(d_configs), int(n), float(inflation_ratio), _dev_ptr(d_out),
+                                                     int(stream) if stream else None))
+
     def get_statistics(self):
         out = (C.c_uint64 * capi.NUM_STATS)()
         check(lib.fks_get_statistics(self._h, out))

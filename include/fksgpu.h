@@ -276,9 +276,10 @@ int fks_sim_synchronize(fks_sim* sim);
  * d_tape_draws / d_tape_offsets may be NULL unless noise_mode == FKS_NOISE_INJECTED.
  * Streams: a simulator owns ONE particle counter, context store and scratch, so its batch calls never overlap -- each launch
  * records an event and the next launch of the same simulator, on whatever stream (a caller's or the simulator's own, which
- * the host-buffer calls use), waits for it.  Calls on different streams are therefore safe and ordered by issue; for
- * batches that should run concurrently use one simulator per stream.  Like the reference (spcs.hpp:846-850) a simulator
- * serves one caller thread at a time. */
+ * the host-buffer calls use), waits for it.  The collision checks (fks_check_config_collision and its _device flavour) use
+ * the same scratch and are serialised with the batch calls in the same way.  Calls on different streams are therefore safe
+ * and ordered by issue; for batches that should run concurrently use one simulator per stream.  Like the reference
+ * (spcs.hpp:846-850) a simulator serves one caller thread at a time. */
 int fks_forward_simulate_device(fks_sim* sim, const double* d_starts, const double* d_targets,
                                 size_t n_particles, size_t n_targets, int allow_contacts,
                                 int noise_mode, const double* d_tape_draws,
@@ -326,6 +327,15 @@ int fks_forward_simulate_sequence_device(fks_sim* sim, const double* d_starts, c
  * (inflation_ratio + 1) * resolution).  HOST buffers: configs n * cfg_stride doubles, out_collides n bytes. */
 int fks_check_config_collision(fks_sim* sim, const double* configs, size_t n_configs, double inflation_ratio,
                                uint8_t* out_collides);
+
+/* Same with DEVICE buffers, asynchronous on `cuda_stream` (a cudaStream_t; NULL = default stream): d_configs
+ * [n_configs][cfg_stride] doubles (the layout of starts, targets and fks_nearest_configurations queries), d_out[i] = 1 when
+ * configuration i collides, 0 otherwise -- the bytes fks_check_config_collision returns for the same input, from the same
+ * launch.  Writes d_out[0 .. n_configs) and nothing else.  A null simulator, and with n_configs > 0 a null buffer or a NaN
+ * inflation_ratio, is FKS_ERR_INVALID_ARGUMENT; n_configs == 0 launches nothing.  Ordered with the simulator's batch calls
+ * as described at fks_forward_simulate_device. */
+int fks_check_config_collision_device(fks_sim* sim, const double* d_configs, size_t n_configs, double inflation_ratio,
+                                      uint8_t* d_out, void* cuda_stream);
 
 /* ForwardSimulateRobot with enable_tracing == true (spcs.hpp:824-829; ForwardSimulationStepTrace filled at :1583-1617,
  * :1703, :1714, :1778) for ONE particle -- SURVEY.md 8(f)-4.  The nested trace of the reference (controller step ->
